@@ -62,7 +62,16 @@ def parse():
     ap.add_argument("--ref-device", default="cpu", choices=["cpu", "cuda"],
                     help="--impl reference: where the reference's own code runs (cpu = the contract's reference arm; cuda = the "
                          "stock PyTorch path of the unmodified reference on this GPU, context only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what rank 0's last timed step returned as DIR/<name>.npy (float32 / "
+                         "float64; a training step adds the parameter gradients as grad.<parameter>); above 64 MB in all, "
+                         "the per-pair outputs are cut to a fixed seeded sample of pairs, listed in pair_index.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return a
 
 
 def workload_cfg(a, name=None, world=1):
@@ -288,8 +297,9 @@ def build_net(cfg, dev):
     return net
 
 
-def measure(cfg, rank, world, dev, local_rank, steps, warmup, profile=False, clocks=False, e2e=True):
-    """Time `steps` steps of one workload on this rank's GPU through the module API.  -> per-rank sums (ms) etc."""
+def measure(cfg, rank, world, dev, local_rank, steps, warmup, profile=False, clocks=False, e2e=True, dump=False):
+    """Time `steps` steps of one workload on this rank's GPU through the module API.  -> per-rank sums (ms) etc.
+    dump: res["outputs"] = (per-pair arrays, other arrays) of the last timed step, as host float32 / float64."""
     import torch
     import torch.distributed as dist
     import vcr_net_b200 as V
@@ -354,12 +364,25 @@ def measure(cfg, rank, world, dev, local_rank, steps, warmup, profile=False, clo
         for i in range(steps):
             flush.fill_(float(i))                     # L2 flush, outside the per-step event bracket
             ev[i][0].record(stream)
-            step(i)
+            out = step(i)
             ev[i][1].record(stream)
+            if i < steps - 1:
+                del out                               # only the last step's outputs outlive the step
         barrier()
         res["wall_s"] = time.perf_counter() - t_wall0
         res["launches"] = launches() - l0
         res["ms_total"] = sum(e0.elapsed_time(e1) for e0, e1 in ev)
+        if dump:                                      # before the e2e steps recompute the gradients
+            to_host = lambda t: t.detach().to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu().numpy()
+            names = (("src_embedding", "tgt_embedding", "loss", "mse_ab", "mae_ab") if train else
+                     ("srcK", "src_corrK", "R_ab", "t_ab", "R_ba", "t_ba"))
+            outs = {n: to_host(o) for n, o in zip(names, out)}
+            per_pair = {n: v for n, v in outs.items() if v.ndim and v.shape[0] == B}
+            other = {n: v for n, v in outs.items() if n not in per_pair}
+            if train:
+                other.update(("grad." + n, to_host(p.grad)) for n, p in net.named_parameters() if p.grad is not None)
+            res["outputs"] = (per_pair, other)
+        del out
         res["ms_e2e"], res["h2d"], res["d2h"] = float("nan"), 0, 0
         if e2e:
             # ---- end-to-end: pinned host -> device -> vcrnetIter -> host --------------------------------
@@ -412,6 +435,25 @@ def measure(cfg, rank, world, dev, local_rank, steps, warmup, profile=False, clo
     del net, devb, flush
     torch.cuda.empty_cache()
     return res
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(path, per_pair, other):
+    """--dump-outputs: write every array as path/<name>.npy.  When they would pass DUMP_BYTES, the arrays indexed by pair
+    keep the same seeded sample of pairs (pair_index.npy), so that two runs with the same arguments write the same files."""
+    os.makedirs(path, exist_ok=True)
+    header = 4096                                             # bound on one .npy header, with room to spare
+    pairs = next(iter(per_pair.values())).shape[0] if per_pair else 0
+    room = DUMP_BYTES - sum(v.nbytes for v in other.values()) - header * (len(per_pair) + len(other) + 1)
+    pair_bytes = sum(v.nbytes for v in per_pair.values()) // max(pairs, 1)
+    if pair_bytes * pairs > room:
+        keep = np.sort(np.random.RandomState(0).choice(pairs, max(room, 0) // (pair_bytes + 8), replace=False))
+        per_pair = {n: v[keep] for n, v in per_pair.items()}
+        other = dict(other, pair_index=keep.astype(np.float64))
+    for n, v in {**per_pair, **other}.items():
+        np.save(os.path.join(path, n + ".npy"), v)
 
 
 def reduce_max(world, dev, *vals):
@@ -555,7 +597,10 @@ def run_gpu_arm(a, cfg, rank, world, local_rank):
         (m,) = reduce_max(world, dev, r[key])
         return r["B"] * steps * world / (m / 1e3), m / steps
 
-    r = measure(cfg, rank, world, dev, local_rank, a.steps, a.warmup, profile=True, clocks=True)
+    r = measure(cfg, rank, world, dev, local_rank, a.steps, a.warmup, profile=True, clocks=True,
+                dump=bool(a.dump_outputs) and rank == 0)
+    if "outputs" in r:
+        dump_outputs(a.dump_outputs, *r.pop("outputs"))
     ms_total, ms_e2e = reduce_max(world, dev, r["ms_total"], r["ms_e2e"])
     launches = reduce_sum_int(world, dev, r["launches"])
 
