@@ -73,7 +73,8 @@ int vcr_graph_feature(const float* xt, int B, int D, int N, int k, const int* id
                       cudaStream_t stream);
 
 /* ---- FPS: util/util.py:107-140 farthest_point_sample (== util/fps.py:10-49) ---------------------
- * xyz [B,3,N] -> idx [B,npoint]; N <= 14000. */
+ * xyz [B,3,N] -> idx [B,npoint]; N <= 229 376 (one CTA per cloud up to 14 336 points, beyond that one thread-block
+ * cluster of 2, 4, 8 or 16 CTAs per cloud; -2 above 229 376 or when the device cannot co-schedule the cluster). */
 int vcr_fps(const float* xyz, int B, int N, int npoint, int32_t* idx32, int64_t* idx64, cudaStream_t stream);
 
 /* ---- generic fp32 GEMM with fused epilogue -------------------------------------------------------

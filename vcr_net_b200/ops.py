@@ -112,6 +112,10 @@ def graph_feature(xt: torch.Tensor, idx: torch.Tensor):
     return out
 
 
+# vcr_fps: one CTA per cloud up to 14 336 points, one cluster of up to 16 such CTAs beyond
+FPS_MAX_POINTS = 16 * 14336
+
+
 def fps(xyz: torch.Tensor, npoint: int, want64: bool = True):
     _chk(xyz, "xyz")
     xyz = xyz.contiguous()
@@ -120,8 +124,12 @@ def fps(xyz: torch.Tensor, npoint: int, want64: bool = True):
     dt = torch.int64 if want64 else torch.int32
     out = torch.empty((B, npoint), dtype=dt, device=xyz.device)
     L = lib()
-    L.check(L.vcr_fps(xyz.data_ptr(), B, N, npoint, None if want64 else out.data_ptr(),
-                      out.data_ptr() if want64 else None, _stream(xyz)), "vcr_fps")
+    rc = L.vcr_fps(xyz.data_ptr(), B, N, npoint, None if want64 else out.data_ptr(),
+                   out.data_ptr() if want64 else None, _stream(xyz))
+    if rc != 0 and N > FPS_MAX_POINTS:
+        raise RuntimeError(f"vcr_fps failed: {rc}: farthest-point sampling takes at most {FPS_MAX_POINTS} points "
+                           f"per cloud, got {N}")
+    L.check(rc, "vcr_fps")
     return out
 
 
