@@ -143,10 +143,13 @@ int vcr_edgeconv_dg(const float* PQ, int ldpq, const int* idx, int k, int N, lon
                     cudaStream_t stream);
 /* Tensor-core (tcgen05/TMEM) flavour of vcr_edgeconv_dg, same contract: the DG2 GEMM runs transposed
  * (D[out-channel][edge]) so max-over-k is an in-thread reduction.  mode: 0 = fp16 3-term split (fp32 parity),
- * 1 = fp16, 2 = bf16.  ldpq, ld1 multiples of 4, slope >= 0. */
+ * 1 = fp16, 2 = bf16.  ldpq, ld1 multiples of 4, slope >= 0.  z (optional, NULL to skip): the per-edge convDG2
+ * pre-activations W2 e1 + b2, [total_pts * 20][128] -- the values x2 is the activated max of, which the LPDNet backward
+ * routes g_x2 by. */
 int vcr_edgeconv_dg_tc(const float* PQ, int ldpq, const int* idx, int k, int N, long long total_pts,
                        const float* W2, const float* b2, float slope, int mode, float* x1, int ld1,
-                       float* x2, int ld2, void* op1, void* op2, int ldop, long long op_plane, cudaStream_t stream);
+                       float* x2, int ld2, void* op1, void* op2, int ldop, long long op_plane, float* z,
+                       cudaStream_t stream);
 /* convSN1 + max (:130-132): out = act(max_k P[idx] + Q), C in {128,256,384,512}. */
 int vcr_gather_max(const float* P, int ldp, const float* Q, int ldq, const int* idx, int k, int N,
                    long long total_pts, int C, float slope, float* out, int ldo, void* op, int ldop,
@@ -300,9 +303,15 @@ int vcr_edge_max(const float* E, int k, long long total_pts, int C, float* out, 
  * vcr_wgrad_f32: dW[N,K] += G[M,N]^T X[M,K], db[N] += column sums of G (db may be NULL); caller zero-initialises. */
 int vcr_wgrad_f32(const float* G, int ldg, const float* X, int ldx, long long M, int N, int K, float* dW,
                   int lddw, float* db, cudaStream_t stream);
-/* gz = gy * LeakyReLU'(z) from the saved post-activation y (F.leaky_relu backward). */
+/* gz = gy * LeakyReLU'(z) from the saved post-activation y (F.leaky_relu backward).  scale_bits (may be NULL): the
+ * output of vcr_absmax_bits for gy; gy is then also multiplied by 2^-floor(log2 max|gy|) (exponent clamped to
+ * [-126, 126]), which brings max|gy| into [1, 2) so that the "h3" data-gradient products see normal fp16 operands. */
 int vcr_act_bwd(const float* gy, int ldg, const float* y, int ldy, long long rows, int cols, float slope,
-                float* gz, int ldz, cudaStream_t stream);
+                const int* scale_bits, float* gz, int ldz, cudaStream_t stream);
+/* bits = max(bits, bit pattern of max|x[i]|) over n contiguous floats; the caller zero-initialises bits. */
+int vcr_absmax_bits(const float* x, long long n, int* bits, cudaStream_t stream);
+/* out[0] = 2^floor(log2 m) for m the float whose bit pattern is bits[0] (same clamp): the inverse of vcr_act_bwd's scale. */
+int vcr_pow2_inverse(const int* bits, float* out, cudaStream_t stream);
 /* backward of vcr_gather_max (convSN1 + max over k, :130-132): gQ written, gP accumulated (zero-initialised). */
 int vcr_gather_max_bwd(const float* P, int ldp, const float* Q, int ldq, const int* idx, int k, int N,
                        long long total_pts, int C, float slope, const float* gout, int ldgo, float* gP,

@@ -65,12 +65,14 @@ __device__ __forceinline__ uint32_t sw_off(int r, int c4, int tile_bytes) {
     return (uint32_t)(kb * tile_bytes + r * 128 + ((chunk ^ (r & 7)) << 4) + ((c4 & 1) << 3));
 }
 
-template <int NTERMS, int FMT>
+// ZOUT: also write the per-edge pre-activations z (a separate instantiation keeps the forward's machine code unchanged)
+template <int NTERMS, int FMT, bool ZOUT>
 __global__ void __launch_bounds__(NTHREADS, 1)
 edgeconv_dg_tc_kernel(const float* __restrict__ PQ, int ldpq, const int* __restrict__ idx, int N, long long total_pts,
                       const float* __restrict__ W2, const float* __restrict__ b2, float slope,
                       float* __restrict__ x1, int ld1, float* __restrict__ x2, int ld2,
-                      __half* __restrict__ op1, __half* __restrict__ op2, int ldop, long long op_plane) {
+                      __half* __restrict__ op1, __half* __restrict__ op2, int ldop, long long op_plane,
+                      float* __restrict__ z) {
     using C_ = ECfg<NTERMS>;
     constexpr int PL = C_::PL;
     constexpr int obf = FMT;      // 1: bf16 operands
@@ -244,6 +246,10 @@ edgeconv_dg_tc_kernel(const float* __restrict__ PQ, int ldpq, const int* __restr
                     for (int i = 1; i < KN; ++i) m = fmaxf(m, v[g * KN + i]);
                     const long long pt = tile * PTS_TILE + sub * PTS_SUB + g;
                     if (pt < total_pts) {
+                        if (ZOUT) {              // per-edge pre-activations; max_k z == m + bias (rounding is monotone)
+#pragma unroll
+                            for (int i = 0; i < KN; ++i) z[(pt * KN + i) * C + o] = v[g * KN + i] + bias;
+                        }
                         const float val = leaky(m + bias, slope);
                         x2[pt * ld2 + o] = val;
                         if (op2 != nullptr) {
@@ -264,16 +270,17 @@ edgeconv_dg_tc_kernel(const float* __restrict__ PQ, int ldpq, const int* __restr
 template <int NTERMS, int FMT>
 int launch_dg_tc(const float* PQ, int ldpq, const int* idx, int N, long long total_pts, const float* W2, const float* b2,
                  float slope, float* x1, int ld1, float* x2, int ld2, __half* op1, __half* op2, int ldop, long long op_plane,
-                 cudaStream_t stream) {
+                 float* z, cudaStream_t stream) {
     using C_ = ECfg<NTERMS>;
-    auto kern = edgeconv_dg_tc_kernel<NTERMS, FMT>;
+    auto kern = z != nullptr ? edgeconv_dg_tc_kernel<NTERMS, FMT, true> : edgeconv_dg_tc_kernel<NTERMS, FMT, false>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C_::SMEM) != cudaSuccess) return VCR_ERR_LAUNCH;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const long long ntiles = (total_pts + PTS_TILE - 1) / PTS_TILE;
     const int grid = (int)(ntiles < sms ? ntiles : sms);
-    kern<<<grid, NTHREADS, C_::SMEM, stream>>>(PQ, ldpq, idx, N, total_pts, W2, b2, slope, x1, ld1, x2, ld2, op1, op2, ldop, op_plane);
+    kern<<<grid, NTHREADS, C_::SMEM, stream>>>(PQ, ldpq, idx, N, total_pts, W2, b2, slope, x1, ld1, x2, ld2, op1, op2, ldop, op_plane,
+                                               z);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
 }
@@ -282,9 +289,10 @@ int launch_dg_tc(const float* PQ, int ldpq, const int* idx, int N, long long tot
 
 // Tensor-core flavour of vcr_edgeconv_dg (same contract).  mode: 0 = fp16 3-term split ("h3", fp32 parity),
 // 1 = fp16, 2 = bf16 single pass.  k must be 20; ldpq, ld1 multiples of 4; PQ, x1 16-byte aligned.
+// z (optional): the convDG2 pre-activations of every edge, [total_pts * 20][128], the values x2 is the max of.
 VCR_API int vcr_edgeconv_dg_tc(const float* PQ, int ldpq, const int* idx, int k, int N, long long total_pts,
                                const float* W2, const float* b2, float slope, int mode, float* x1, int ld1,
-                               float* x2, int ld2, void* op1, void* op2, int ldop, long long op_plane,
+                               float* x2, int ld2, void* op1, void* op2, int ldop, long long op_plane, float* z,
                                cudaStream_t stream) {
     VCR_REQUIRE(PQ && idx && W2 && b2 && x1 && x2 && N > 0 && total_pts > 0);
     if (k != KN || mode < 0 || mode > 2 || slope < 0.f) return VCR_ERR_UNSUPPORTED;
@@ -296,7 +304,7 @@ VCR_API int vcr_edgeconv_dg_tc(const float* PQ, int ldpq, const int* idx, int k,
     if (op1 && ((ldop & 3) || (op_plane & 3) || (reinterpret_cast<uintptr_t>(op1) & 7))) return VCR_ERR_INVALID;
     __half* o1 = reinterpret_cast<__half*>(op1);
     __half* o2 = reinterpret_cast<__half*>(op2);
-    if (mode == 0) return launch_dg_tc<3, 0>(PQ, ldpq, idx, N, total_pts, W2, b2, slope, x1, ld1, x2, ld2, o1, o2, ldop, op_plane, stream);
-    if (mode == 1) return launch_dg_tc<1, 0>(PQ, ldpq, idx, N, total_pts, W2, b2, slope, x1, ld1, x2, ld2, o1, o2, ldop, op_plane, stream);
-    return launch_dg_tc<1, 1>(PQ, ldpq, idx, N, total_pts, W2, b2, slope, x1, ld1, x2, ld2, o1, o2, ldop, op_plane, stream);
+    if (mode == 0) return launch_dg_tc<3, 0>(PQ, ldpq, idx, N, total_pts, W2, b2, slope, x1, ld1, x2, ld2, o1, o2, ldop, op_plane, z, stream);
+    if (mode == 1) return launch_dg_tc<1, 0>(PQ, ldpq, idx, N, total_pts, W2, b2, slope, x1, ld1, x2, ld2, o1, o2, ldop, op_plane, z, stream);
+    return launch_dg_tc<1, 1>(PQ, ldpq, idx, N, total_pts, W2, b2, slope, x1, ld1, x2, ld2, o1, o2, ldop, op_plane, z, stream);
 }

@@ -5,7 +5,8 @@
 // pass mirrors that factoring, all in fp32:
 //   vcr_wgrad_f32          dW[n,k] += sum_m G[m,n] X[m,k], db[n] += sum_m G[m,n]   (weight / bias gradients of
 //                          every 1x1 conv: a tall-skinny A^T B product, split over M across CTAs)
-//   vcr_act_bwd            gz = gy * LeakyReLU'(z), from the saved post-activation output (y > 0 <=> z > 0)
+//   vcr_act_bwd            gz = gy * LeakyReLU'(z), from the saved post-activation output (y > 0 <=> z > 0), optionally
+//                          times the power of two vcr_absmax_bits picked for gy (see LPDNetTrainFn.backward)
 //   vcr_gather_max_bwd     backward of x3 = act(max_k P3[nbr] + Q3)  (convSN1 + max, :130-132)
 //   vcr_edge_gather_act    e1 = act(P1[nbr] + Q1), materialised [T*k, C]   (convDG1 output, :123)
 //   vcr_edge_max_bwd       route g_x2 to the arg-max edge of z2 = convDG2(e1) per (point, channel)   (:125-126)
@@ -70,13 +71,35 @@ wgrad_kernel(const float* __restrict__ G, int ldg, const float* __restrict__ X, 
     }
 }
 
+// 2^-floor(log2 m) (inverse = false) or 2^floor(log2 m) (inverse = true) for the bit pattern of m = max|g| >= 0, with
+// floor(log2 m) clamped to [-126, 126] so that both are normal floats (m = 0 gives 2^126 / 2^-126)
+__device__ __forceinline__ float pow2_scale(int mbits, bool inverse) {
+    const int e = min(max((mbits >> 23) & 255, 1), 253);
+    return __int_as_float((inverse ? e : 254 - e) << 23);
+}
+
+__global__ void absmax_kernel(const float* __restrict__ x, long long n, int* __restrict__ mbits) {
+    float m = 0.f;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        m = fmaxf(m, fabsf(x[i]));
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if ((threadIdx.x & 31) == 0) atomicMax(mbits, __float_as_int(m));     // non-negative floats order like their bits
+}
+
 __global__ void act_bwd_kernel(const float* __restrict__ gy, int ldg, const float* __restrict__ y, int ldy,
-                               long long rows, int cols, float slope, float* __restrict__ gz, int ldz) {
+                               long long rows, int cols, float slope, const int* __restrict__ mbits,
+                               float* __restrict__ gz, int ldz) {
     const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= rows * cols) return;
     const long long r = e / cols;
     const int c = (int)(e - r * cols);
-    gz[r * ldz + c] = gy[r * ldg + c] * (y[r * ldy + c] > 0.f ? 1.f : slope);
+    const float g = mbits ? gy[r * ldg + c] * pow2_scale(*mbits, false) : gy[r * ldg + c];
+    gz[r * ldz + c] = g * (y[r * ldy + c] > 0.f ? 1.f : slope);
+}
+
+__global__ void pow2_inverse_kernel(const int* __restrict__ mbits, float* __restrict__ out) {
+    *out = pow2_scale(*mbits, true);
 }
 
 // x3[pt,c] = act(max_k P[nbr_k,c] + Q[pt,c]):  gQ[pt,c] = g * act'(s),  gP[argmax nbr, c] += the same
@@ -191,9 +214,25 @@ VCR_API int vcr_wgrad_f32(const float* G, int ldg, const float* X, int ldx, long
 }
 
 VCR_API int vcr_act_bwd(const float* gy, int ldg, const float* y, int ldy, long long rows, int cols, float slope,
-                        float* gz, int ldz, cudaStream_t stream) {
+                        const int* scale_bits, float* gz, int ldz, cudaStream_t stream) {
     VCR_REQUIRE(gy && y && gz && rows > 0 && cols > 0);
-    act_bwd_kernel<<<blocks_for(rows * cols, 256), 256, 0, stream>>>(gy, ldg, y, ldy, rows, cols, slope, gz, ldz);
+    act_bwd_kernel<<<blocks_for(rows * cols, 256), 256, 0, stream>>>(gy, ldg, y, ldy, rows, cols, slope, scale_bits, gz,
+                                                                    ldz);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
+VCR_API int vcr_absmax_bits(const float* x, long long n, int* bits, cudaStream_t stream) {
+    VCR_REQUIRE(x && bits && n > 0);
+    const long long want = (n + 255) / 256;
+    absmax_kernel<<<(unsigned)(want < 4 * 148 ? want : 4 * 148), 256, 0, stream>>>(x, n, bits);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
+VCR_API int vcr_pow2_inverse(const int* bits, float* out, cudaStream_t stream) {
+    VCR_REQUIRE(bits && out);
+    pow2_inverse_kernel<<<1, 1, 0, stream>>>(bits, out);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
 }

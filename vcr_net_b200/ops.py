@@ -366,21 +366,26 @@ def edgeconv_dg(pq: torch.Tensor, idx: torch.Tensor, w2: torch.Tensor, b2: torch
 
 
 def edgeconv_dg_tc(pq: torch.Tensor, idx: torch.Tensor, w2: torch.Tensor, b2: torch.Tensor, slope: float,
-                   x1: torch.Tensor, x2: torch.Tensor, mode: str, op1: "Operand | None" = None, op2: "Operand | None" = None):
+                   x1: torch.Tensor, x2: torch.Tensor, mode: str, op1: "Operand | None" = None, op2: "Operand | None" = None,
+                   z: torch.Tensor | None = None):
     """edgeconv_dg on tcgen05 tensor cores (csrc/edgeconv_tc.cu); mode in TC_MODES.
-    op1 / op2: optional "h3" Operand views (same buffer) that also receive x1 / x2 in operand format."""
+    op1 / op2: optional "h3" Operand views (same buffer) that also receive x1 / x2 in operand format.
+    z: optional contiguous [B*N*20, 128] that receives the per-edge convDG2 pre-activations x2 is the max of."""
     B, N, _ = pq.shape
     _, _, ldpq = _rows(pq)
     _, _, ld1 = _rows(x1)
     _, _, ld2 = _rows(x2)
     if op1 is not None:
         assert op1.mode == "h3" and op2.mode == "h3" and op1.ld == op2.ld and op1.plane_stride == op2.plane_stride
+    if z is not None:
+        _chk(z, "z")
+        assert z.is_contiguous() and tuple(z.shape) == (B * N * idx.shape[2], 128)
     L = lib()
     L.check(L.vcr_edgeconv_dg_tc(pq.data_ptr(), ldpq, idx.data_ptr(), idx.shape[2], N, B * N, w2.data_ptr(),
                                  b2.data_ptr(), float(slope), TC_MODES[mode], x1.data_ptr(), ld1, x2.data_ptr(), ld2,
                                  op1.ptr if op1 is not None else None, op2.ptr if op2 is not None else None,
                                  op1.ld if op1 is not None else 0, op1.plane_stride if op1 is not None else 0,
-                                 _stream(pq)), "vcr_edgeconv_dg_tc")
+                                 z.data_ptr() if z is not None else None, _stream(pq)), "vcr_edgeconv_dg_tc")
 
 
 def gather_max(p: torch.Tensor, q: torch.Tensor, idx: torch.Tensor, slope: float, out: torch.Tensor,
@@ -445,17 +450,40 @@ def wgrad(g: torch.Tensor, x: torch.Tensor, want_bias: bool = True):
     return dW, db
 
 
-def act_bwd(gy: torch.Tensor, y: torch.Tensor, slope: float):
-    """gz = gy * LeakyReLU'(z), y = the saved post-activation output (row views)."""
+def act_bwd(gy: torch.Tensor, y: torch.Tensor, slope: float, scale_bits: torch.Tensor | None = None):
+    """gz = gy * LeakyReLU'(z), y = the saved post-activation output (row views).
+    scale_bits: absmax_bits(gy); gz is then also scaled by 2^-floor(log2 max|gy|)."""
     _chk(gy, "gy"); _chk(y, "y")
     M, N, ldg = _rows(gy)
     M2, N2, ldy = _rows(y)
     assert (M, N) == (M2, N2)
+    if scale_bits is not None:
+        _chk(scale_bits, "scale_bits", torch.int32)
     gz = torch.empty(gy.shape, dtype=_F32, device=gy.device)
     L = lib()
-    L.check(L.vcr_act_bwd(gy.data_ptr(), ldg, y.data_ptr(), ldy, M, N, float(slope), gz.data_ptr(), N, _stream(gy)),
+    L.check(L.vcr_act_bwd(gy.data_ptr(), ldg, y.data_ptr(), ldy, M, N, float(slope),
+                          scale_bits.data_ptr() if scale_bits is not None else None, gz.data_ptr(), N, _stream(gy)),
             "vcr_act_bwd")
     return gz
+
+
+def absmax_bits(x: torch.Tensor):
+    """x contiguous fp32 -> int32 [1]: the bit pattern of max|x| (on the device, no host synchronisation)."""
+    _chk(x, "x")
+    assert x.is_contiguous()
+    bits = torch.zeros(1, dtype=torch.int32, device=x.device)
+    L = lib()
+    L.check(L.vcr_absmax_bits(x.data_ptr(), x.numel(), bits.data_ptr(), _stream(x)), "vcr_absmax_bits")
+    return bits
+
+
+def pow2_inverse(bits: torch.Tensor):
+    """absmax_bits output -> fp32 [1]: the inverse of the scale act_bwd applies for it."""
+    _chk(bits, "bits", torch.int32)
+    out = torch.empty(1, dtype=_F32, device=bits.device)
+    L = lib()
+    L.check(L.vcr_pow2_inverse(bits.data_ptr(), out.data_ptr(), _stream(bits)), "vcr_pow2_inverse")
+    return out
 
 
 def gather_max_bwd(p: torch.Tensor, q: torch.Tensor, idx: torch.Tensor, slope: float, gout: torch.Tensor,
