@@ -202,7 +202,9 @@ int vcr_softmax_colsum(const float* S, int ld, int B, long long rows_per_batch, 
 int vcr_colsum_softmax(const float* S, int ld, int B, long long rows_per_batch, int n, const float* rmax,
                        const float* rsum, float* out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 int vcr_rowsum(const float* P, int ld, long long rows, int n, float* out, cudaStream_t stream);
-/* top-K (value desc, ties -> lower index): sorted indices and/or a uint8 membership mask (:41-47). */
+/* top-K (value desc, ties -> lower index, -0 == +0): sorted indices and/or a uint8 membership mask (:41-47).
+ * n <= 262 144: one CTA per row up to 16 384, beyond that one thread-block cluster of 2, 4, 8 or 16 CTAs per row (16 384
+ * keys each); -2 above 262 144 or when the device cannot co-schedule the cluster.  No workspace, no host sync. */
 int vcr_topk_select(const float* vals, int B, int n, int K, int* idx_out, uint8_t* mask_out, cudaStream_t stream);
 
 /* ---- VcpTopK head: model/vcrnet_model.py:162-347 ---------------------------------------------------
@@ -224,6 +226,14 @@ int vcr_softcorr_tc(const void* S, int lds, long long s_plane, const void* T, in
 int vcr_softcorr_best_tc(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
                          const float* xx, const float* yy, int B, int Ns, int Nt, int D,
                          int* best_idx, float* best_val, cudaStream_t stream);
+/* selectCom's statistics (as vcr_select_stats) straight from the operands, on tensor cores, with no [Ns,Nt] buffer:
+ * S / T, xx / yy as vcr_softcorr_best_tc takes them -> row_stat [B,Ns], col_stat [B,Nt].  Four launches of the fused
+ * kernel (row max / sum over targets, the same over sources, then the two weighted sums), each row owned by one thread
+ * pair: deterministic.  workspace: 2*(B*Ns + B*Nt) floats (the per-row and per-column max and 1/sum). */
+size_t vcr_select_stats_tc_workspace_bytes(int B, int Ns, int Nt);
+int vcr_select_stats_tc(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
+                        const float* xx, const float* yy, int B, int Ns, int Nt, int D, float* row_stat, float* col_stat,
+                        void* workspace, size_t workspace_bytes, cudaStream_t stream);
 /* row sums of the softmax taken over sources (dim=1) (:243-244); workspace from the size query. */
 size_t vcr_rowsum_colsoftmax_workspace_bytes(int B, int Nt);
 int vcr_rowsum_colsoftmax(const float* pd, int ld, int B, int Ns, int Nt, float* out, void* workspace,

@@ -104,17 +104,8 @@ fps_kernel(const float* __restrict__ xyz, int N, int npoint, int32_t* __restrict
 }
 
 // ---------------------------------------------------------------- cluster variant ------------------------
-__device__ __forceinline__ int cluster_nctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
-    return (int)r;
-}
-// address of the same shared-memory object in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t cluster_addr(const void* p, int rank) {
-    uint32_t a;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(tc::smem_u32(p)), "r"(rank));
-    return a;
-}
+using tc::cluster_nctarank;
+using tc::cluster_addr;
 __device__ __forceinline__ float4 ld_cluster_f4(uint32_t a) {
     float4 v;
     asm volatile("ld.shared::cluster.v4.f32 {%0, %1, %2, %3}, [%4];"

@@ -10,6 +10,9 @@
 // row into pd with the reference's operation order, keeps a running (max, sum, sum * xyz) per row (online softmax)
 // and writes corr[B,3,Ns] at the end of the item.  The logits cancel catastrophically (|f|^2 ~ 500 against gaps
 // < 1, SURVEY.md section 7), so this kernel exists in the 3-term mode only, in every precision mode.
+// The same main loop gives selectCom's two statistics (vcr_select_stats_tc): MODE 3 keeps only the row's running
+// (max, sum) and writes (max, 1/sum); MODE 4 sums exp(pd_ij - M_j) * invL_j with per-column (M, 1/L) staged in shared
+// memory.  SWAP runs a launch with the targets as rows: pd keeps the reference order with the source norm first.
 #include "tc_common.cuh"
 
 namespace {
@@ -35,9 +38,15 @@ struct SoftcorrParams {
     float* corr;          // [B,3,Ns]           (mode 0)
     int* best_idx;        // [B,Ns] argmax_j     (mode 2: hard correspondences, model/vcrnet_model.py:295-299)
     float* best_val;      // [B,Ns] max_j P_ij   (mode 2)
+    float* row_m;         // [B,Ns] max_j pd_ij          (mode 3)
+    float* row_il;        // [B,Ns] 1 / sum_j exp(pd_ij - max)   (mode 3)
+    const float* col_m;   // [B,Nt] per-column max        (mode 4)
+    const float* col_il;  // [B,Nt] per-column 1 / sum    (mode 4)
+    float* row_stat;      // [B,Ns] sum_j exp(pd_ij - col_m_j) * col_il_j   (mode 4)
 };
 
-template <int MODE>
+// SWAP: the rows (A, xx) are targets and the columns (B, yy) sources.
+template <int MODE, bool SWAP = false>
 __global__ void __launch_bounds__(NTHREADS, 1)
 softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const SoftcorrParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -116,8 +125,13 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                             const uint32_t acc = (kb | kk) != 0;
                             const uint64_t adv = (uint64_t)(kk * 2);  // 16 elements = 32 B along K
                             tc::umma_f16(d0, a_hi + adv, b_hi + adv, idesc, acc);
-                            tc::umma_f16(d1, a_hi + adv, b_lo + adv, idesc, acc);
-                            tc::umma_f16(d1, a_lo + adv, b_hi + adv, idesc, 1);
+                            if (SWAP) {                               // per element: s_hi t_lo, then s_lo t_hi, as unswapped
+                                tc::umma_f16(d1, a_lo + adv, b_hi + adv, idesc, acc);
+                                tc::umma_f16(d1, a_hi + adv, b_lo + adv, idesc, 1);
+                            } else {
+                                tc::umma_f16(d1, a_hi + adv, b_lo + adv, idesc, acc);
+                                tc::umma_f16(d1, a_lo + adv, b_hi + adv, idesc, 1);
+                            }
                         }
                         tc::umma_commit(&empty[s]);
                         if (++s == NSTAGES) { s = 0; ph ^= 1; }
@@ -159,6 +173,10 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                         cols[128 + q * 32 + lane] = ok ? tb[p.Nt + cj] : 0.f;
                         cols[192 + q * 32 + lane] = ok ? tb[2 * p.Nt + cj] : 0.f;
                     }
+                    if (MODE == 4) {
+                        cols[64 + q * 32 + lane] = ok ? p.col_m[(size_t)b * p.Nt + cj] : 0.f;
+                        cols[128 + q * 32 + lane] = ok ? p.col_il[(size_t)b * p.Nt + cj] : 0.f;
+                    }
                 }
                 __syncwarp();
                 tc::mbar_wait(&tfull[a], aph);
@@ -178,13 +196,19 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                         for (int j = 0; j < 32; ++j) {
                             const float dot = fmaf(__uint_as_float(r1[j]), 1.f / 2048.f, __uint_as_float(r0[j]));
                             // reference op order (:341-342): (-xx - (-2 dot)) - yy
-                            pd[j] = __fsub_rn(__fsub_rn(nx, -2.f * dot), cols[cc * 32 + j]);
+                            if (SWAP) pd[j] = __fsub_rn(__fsub_rn(-cols[cc * 32 + j], -2.f * dot), -nx);
+                            else pd[j] = __fsub_rn(__fsub_rn(nx, -2.f * dot), cols[cc * 32 + j]);
                         }
                     }
                     if (col0 + 32 > p.Nt) {
 #pragma unroll
                         for (int j = 0; j < 32; ++j)
                             if (col0 + j >= p.Nt) pd[j] = -INFINITY;
+                    }
+                    if (MODE == 4) {                           // columns past Nt: exp(-inf) * 0
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) s = fmaf(__expf(pd[j] - cols[64 + cc * 32 + j]), cols[128 + cc * 32 + j], s);
+                        continue;
                     }
                     float cm = pd[0];
                     int cj = 0;
@@ -234,12 +258,17 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                         cb[row] = (cx * f0 + x5[2] * f1) / st;
                         cb[p.Ns + row] = (cy * f0 + x5[3] * f1) / st;
                         cb[2 * p.Ns + row] = (cz * f0 + x5[4] * f1) / st;
-                    } else {
+                    } else if (MODE == 2) {
                         // equal maxima in the two halves: the lower index wins (the halves interleave 64-column blocks)
                         const int mj1 = __float_as_int(x5[2]);
                         const int best = (m1 > m || (m1 == m && mj1 < mj)) ? mj1 : mj;
                         p.best_idx[(size_t)b * p.Ns + row] = best;
                         p.best_val[(size_t)b * p.Ns + row] = 1.0f / st;     // exp(0) / sum: the maximum probability
+                    } else if (MODE == 3) {
+                        p.row_m[(size_t)b * p.Ns + row] = mt;
+                        p.row_il[(size_t)b * p.Ns + row] = 1.0f / st;
+                    } else {
+                        p.row_stat[(size_t)b * p.Ns + row] = s + x5[1];           // no running max: plain sum
                     }
                 }
             }
@@ -253,6 +282,21 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 
 }  // namespace
 
+template <int MODE, bool SWAP>
+static int softcorr_run(const CUtensorMap& tmA, const CUtensorMap& tmB, const SoftcorrParams& p, cudaStream_t stream) {
+    auto kern = softcorr_tc_kernel<MODE, SWAP>;
+    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess)
+        return VCR_ERR_LAUNCH;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const long long items = (long long)p.B * vcr_cdiv(p.Ns, BM);
+    const int grid = (int)(items < sms ? items : sms);
+    kern<<<grid, NTHREADS, SMEM_BYTES, stream>>>(tmA, tmB, p);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
 // S / T: operand-format ("h3": 2 planes, fp16 hi and lo * 2^11) embeddings [2][B*Ns][lds] / [2][B*Nt][ldt];
 // xx / yy: their fp32 squared row norms (vcr_sqnorm_rows); tgt [B,3,Nt]; corr [B,3,Ns].
 // Replaces the matmul + softmax + matmul of model/vcrnet_model.py:337-345 without materialising the score matrix.
@@ -265,20 +309,10 @@ static int softcorr_launch(int mode, const void* S, int lds, long long s_plane, 
     if (rc != VCR_OK) return rc;
     rc = vcr_make_operand_tmap(&tmB, T, D, (long long)B * Nt, ldt, t_plane, 2, BN);
     if (rc != VCR_OK) return rc;
-    SoftcorrParams p;
+    SoftcorrParams p = {};
     p.B = B; p.Ns = Ns; p.Nt = Nt; p.D = D; p.xx = xx; p.yy = yy; p.tgt = tgt; p.corr = corr;
     p.best_idx = best_idx; p.best_val = best_val;
-    auto kern = mode == 0 ? softcorr_tc_kernel<0> : softcorr_tc_kernel<2>;
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess)
-        return VCR_ERR_LAUNCH;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const long long items = (long long)B * vcr_cdiv(Ns, BM);
-    const int grid = (int)(items < sms ? items : sms);
-    kern<<<grid, NTHREADS, SMEM_BYTES, stream>>>(tmA, tmB, p);
-    VCR_CHECK_LAUNCH();
-    return VCR_OK;
+    return mode == 0 ? softcorr_run<0, false>(tmA, tmB, p, stream) : softcorr_run<2, false>(tmA, tmB, p, stream);
 }
 
 VCR_API int vcr_softcorr_tc(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
@@ -295,4 +329,41 @@ VCR_API int vcr_softcorr_best_tc(const void* S, int lds, long long s_plane, cons
                                  int* best_idx, float* best_val, cudaStream_t stream) {
     VCR_REQUIRE(S && T && xx && yy && best_idx && best_val && B > 0 && Ns > 0 && Nt > 0 && D > 0);
     return softcorr_launch(2, S, lds, s_plane, T, ldt, t_plane, xx, yy, nullptr, B, Ns, Nt, D, nullptr, best_idx, best_val, stream);
+}
+
+VCR_API size_t vcr_select_stats_tc_workspace_bytes(int B, int Ns, int Nt) {
+    return (size_t)2 * ((size_t)B * Ns + (size_t)B * Nt) * sizeof(float);
+}
+
+// selectCom's two statistics (model/vcrnet_model.py:213-222, 243-244) from the operands, without the [Ns, Nt] matrix:
+//   row_stat[i] = sum_j exp(pd_ij - Mc_j) / Lc_j      col_stat[j] = sum_i exp(pd_ij - Mr_i) / Lr_i
+// Four launches of the fused kernel, each owning its rows: (a) sources x targets -> (Mr, 1/Lr); (b) targets x sources ->
+// (Mc, 1/Lc); (c) sources x targets -> row_stat; (d) targets x sources -> col_stat.  Every sum runs inside one thread (two
+// column halves added once) in tile order, so the result is deterministic.  workspace: Mr | 1/Lr | Mc | 1/Lc.
+VCR_API int vcr_select_stats_tc(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
+                                const float* xx, const float* yy, int B, int Ns, int Nt, int D, float* row_stat,
+                                float* col_stat, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+    VCR_REQUIRE(S && T && xx && yy && row_stat && col_stat && B > 0 && Ns > 0 && Nt > 0 && D > 0);
+    if (!workspace || workspace_bytes < vcr_select_stats_tc_workspace_bytes(B, Ns, Nt)) return VCR_ERR_WORKSPACE;
+    if ((long long)B * (Ns > Nt ? Ns : Nt) > 0x7fffffffLL) return VCR_ERR_UNSUPPORTED;
+    CUtensorMap tmS, tmT;                                  // BM == BN: one map per operand serves both roles
+    int rc = vcr_make_operand_tmap(&tmS, S, D, (long long)B * Ns, lds, s_plane, 2, BM);
+    if (rc != VCR_OK) return rc;
+    rc = vcr_make_operand_tmap(&tmT, T, D, (long long)B * Nt, ldt, t_plane, 2, BN);
+    if (rc != VCR_OK) return rc;
+    float* mr = reinterpret_cast<float*>(workspace);
+    float* ilr = mr + (size_t)B * Ns;
+    float* mc = ilr + (size_t)B * Ns;
+    float* ilc = mc + (size_t)B * Nt;
+    SoftcorrParams ps = {}, pt = {};                       // rows = sources / rows = targets
+    ps.B = B; ps.Ns = Ns; ps.Nt = Nt; ps.D = D; ps.xx = xx; ps.yy = yy;
+    pt.B = B; pt.Ns = Nt; pt.Nt = Ns; pt.D = D; pt.xx = yy; pt.yy = xx;
+    ps.row_m = mr; ps.row_il = ilr;
+    pt.row_m = mc; pt.row_il = ilc;
+    if ((rc = softcorr_run<3, false>(tmS, tmT, ps, stream)) != VCR_OK) return rc;
+    if ((rc = softcorr_run<3, true>(tmT, tmS, pt, stream)) != VCR_OK) return rc;
+    ps.col_m = mc; ps.col_il = ilc; ps.row_stat = row_stat;
+    pt.col_m = mr; pt.col_il = ilr; pt.row_stat = col_stat;
+    if ((rc = softcorr_run<4, false>(tmS, tmT, ps, stream)) != VCR_OK) return rc;
+    return softcorr_run<4, true>(tmT, tmS, pt, stream);
 }

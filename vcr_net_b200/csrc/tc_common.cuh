@@ -216,6 +216,17 @@ __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
     asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
+__device__ __forceinline__ int cluster_nctarank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
+    return (int)r;
+}
+// address of the same shared-memory object in CTA `rank` of the cluster
+__device__ __forceinline__ uint32_t cluster_addr(const void* p, int rank) {
+    uint32_t a;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(smem_u32(p)), "r"(rank));
+    return a;
+}
 __device__ __forceinline__ void tma_load_3d_2sm(void* smem_dst, const CUtensorMap* m, uint64_t* leader_bar, int c0, int c1, int c2) {
     asm volatile(
         "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"

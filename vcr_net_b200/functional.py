@@ -947,19 +947,13 @@ class Selected:
         self.op, self.sq = op, sq
 
 
-def vcp_select(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2, pre=None, want_tokens=True):
-    """selectCom (model/vcrnet_model.py:190-262) without the unused *_remain host round trips.
+# vcp_select materialises the [B, Ns, Nt] fp32 score products up to this many points per cloud (in every precision
+# mode); past it the tensor-core modes take the statistics from select_stats_tc and fp32 keeps materialising.
+SELECT_STATS_MATERIALISED_MAX = 16384
 
-    The two selection statistics come from one fused two-read pass over the score products (vcr_select_stats).  With
-    ``pre`` (operand copies + squared norms of both embeddings) and ``want_tokens=False`` the selected embeddings are
-    returned as ``Selected`` operand rows for vcp_copair instead of fp32 tokens (src_tok / tgt_tok may then be None)."""
-    if pre is not None and config.precision == "fp32":
-        pre = None
-    ref = pre[0].sq if pre is not None else src_tok
-    B, Ns = ref.shape[0], ref.shape[1]
-    Nt = pre[1].sq.shape[1] if pre is not None else tgt_tok.shape[1]
-    srcK = int(Ns * 0.84 * overlap2)
-    tgtK = int(Nt * 0.84 * overlap2)
+
+def _select_stats_materialised(src_tok, tgt_tok, pre, B, Ns, Nt):
+    """selectCom's (row_stat, col_stat) over the score products dot [B, Ns, ld] written to HBM."""
     if pre is None:
         src_tok, tgt_tok = src_tok.contiguous(), tgt_tok.contiguous()
         dot, ld = pair_dots(src_tok, tgt_tok)
@@ -978,6 +972,28 @@ def vcp_select(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2, pre=None, want_toke
         pd = ops.negdist_(dot, ld, Ns, Nt, xx, yy)
         row_stat = ops.rowsum_colsoftmax(pd, ld, Ns, Nt)
         col_stat = ops.colsum(ops.softmax_rows_(pd.view(B * Ns, ld)[:, :Nt]), B)
+    return row_stat, col_stat
+
+
+def vcp_select(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2, pre=None, want_tokens=True):
+    """selectCom (model/vcrnet_model.py:190-262) without the unused *_remain host round trips.
+
+    The two selection statistics come from one fused two-read pass over the score products (vcr_select_stats), or, in
+    the tensor-core modes past 16 384 points, from the operands without the score products (vcr_select_stats_tc).  With
+    ``pre`` (operand copies + squared norms of both embeddings) and ``want_tokens=False`` the selected embeddings are
+    returned as ``Selected`` operand rows for vcp_copair instead of fp32 tokens (src_tok / tgt_tok may then be None)."""
+    if pre is not None and config.precision == "fp32":
+        pre = None
+    ref = pre[0].sq if pre is not None else src_tok
+    B, Ns = ref.shape[0], ref.shape[1]
+    Nt = pre[1].sq.shape[1] if pre is not None else tgt_tok.shape[1]
+    srcK = int(Ns * 0.84 * overlap2)
+    tgtK = int(Nt * 0.84 * overlap2)
+    if pre is not None and max(Ns, Nt) > SELECT_STATS_MATERIALISED_MAX:
+        # past 16 384 points the [Ns, Nt] score matrix is 1 GB per pair and up: statistics from the operands instead
+        row_stat, col_stat = ops.select_stats_tc(pre[0].op, pre[1].op, pre[0].sq, pre[1].sq, B, Ns, Nt, pre[0].op.cols)
+    else:
+        row_stat, col_stat = _select_stats_materialised(src_tok, tgt_tok, pre, B, Ns, Nt)
     both = row_stat._base
     if srcK == tgtK and both is not None and both is col_stat._base and tuple(both.shape) == (2, B, Ns):
         idx = ops.topk_select(both.view(2 * B, Ns), srcK)[0]           # both rankings (:222, :244) in one launch

@@ -594,6 +594,10 @@ def colsum(P: torch.Tensor, B: int, out=None):
     return out
 
 
+# vcr_topk_select: one CTA per row up to 16 384 values, one cluster of up to 16 such CTAs beyond
+TOPK_MAX_N = 16 * 16384
+
+
 def topk_select(vals: torch.Tensor, K: int, want_idx=True, want_mask=False):
     _chk(vals, "vals")
     vals = vals.contiguous()
@@ -601,8 +605,12 @@ def topk_select(vals: torch.Tensor, K: int, want_idx=True, want_mask=False):
     idx = torch.empty((B, K), dtype=torch.int32, device=vals.device) if want_idx else None
     mask = torch.empty((B, n), dtype=torch.uint8, device=vals.device) if want_mask else None
     L = lib()
-    L.check(L.vcr_topk_select(vals.data_ptr(), B, n, K, idx.data_ptr() if want_idx else None,
-                              mask.data_ptr() if want_mask else None, _stream(vals)), "vcr_topk_select")
+    rc = L.vcr_topk_select(vals.data_ptr(), B, n, K, idx.data_ptr() if want_idx else None,
+                           mask.data_ptr() if want_mask else None, _stream(vals))
+    if rc != 0 and n > TOPK_MAX_N:
+        raise RuntimeError(f"vcr_topk_select failed: {rc}: top-K selection takes at most {TOPK_MAX_N} values per row, "
+                           f"got {n}")
+    L.check(rc, "vcr_topk_select")
     return idx, mask
 
 
@@ -742,6 +750,26 @@ def select_stats(dot: torch.Tensor, ld: int, Ns: int, Nt: int, xx: torch.Tensor,
     ws = torch.empty(wsb // 4, dtype=_F32, device=dev)
     L.check(L.vcr_select_stats(dot.data_ptr(), ld, B, Ns, Nt, xx.data_ptr(), yy.data_ptr(), row_stat.data_ptr(),
                                col_stat.data_ptr(), ws.data_ptr(), wsb, _stream(dot)), "vcr_select_stats")
+    return row_stat, col_stat
+
+
+def select_stats_tc(s_op: "Operand", t_op: "Operand", xx, yy, B: int, Ns: int, Nt: int, D: int):
+    """selectCom's two statistics on tensor cores from "h3" operands (csrc/softcorr_tc.cu), no [Ns,Nt] matrix in HBM:
+    (row_stat [B,Ns], col_stat [B,Nt]), laid out as select_stats lays them out."""
+    assert s_op.mode == "h3" and t_op.mode == "h3" and s_op.rows == B * Ns and t_op.rows == B * Nt
+    dev = xx.device
+    if Ns == Nt:                              # one [2, B, N] buffer: the caller can rank both statistics in one launch
+        both = torch.empty((2, B, Ns), dtype=_F32, device=dev)
+        row_stat, col_stat = both[0], both[1]
+    else:
+        row_stat = torch.empty((B, Ns), dtype=_F32, device=dev)
+        col_stat = torch.empty((B, Nt), dtype=_F32, device=dev)
+    L = lib()
+    wsb = L.vcr_select_stats_tc_workspace_bytes(B, Ns, Nt)
+    ws = torch.empty(wsb // 4, dtype=_F32, device=dev)
+    L.check(L.vcr_select_stats_tc(s_op.ptr, s_op.ld, s_op.plane_stride, t_op.ptr, t_op.ld, t_op.plane_stride,
+                                  xx.data_ptr(), yy.data_ptr(), B, Ns, Nt, D, row_stat.data_ptr(), col_stat.data_ptr(),
+                                  ws.data_ptr(), wsb, _stream(xx)), "vcr_select_stats_tc")
     return row_stat, col_stat
 
 
