@@ -278,11 +278,22 @@ int vcr_add(const float* a, const float* b, float* out, long long n, cudaStream_
  *   src[p,:,n] = base[p, idx_src[p,n]], tgt[p,:,n] = R_p base[p, idx_tgt[p,n]] + t_p in float64 (:289-291), outputs as
  *   fp64 [P,3,N] (input of the crop) and / or fp32.  pose [P,12] fp64 = row-major R then t.
  * vcr_crop_nearest: util/data.py:320-329: the `keep` points nearest to the last point, nearest first -> fp32 [P,3,keep].
+ *   pc64 fp64 [P,3,N]; squared distances in fp64, ties -> lower index.  One CTA per cloud ranks by counting in shared
+ *   memory: N <= 25 600 (-2 above).
+ * vcr_crop_nearest_sort: the same crop for any N (P >= 1, 1 <= keep <= N, P*N <= 2^31 - 1, else -2): a stable LSD radix sort
+ *   of the distances' fp64 bit patterns (8 passes of 8-bit digits, segmented per cloud) in `workspace` of at least
+ *   vcr_crop_nearest_workspace_bytes(P, N) bytes (-4 if smaller), then a gather of the first `keep`.  Where both apply
+ *   and no distance is NaN, the output equals vcr_crop_nearest's bit for bit; NaN distances go last in index order (as in
+ *   numpy's stable argsort), and all `keep` columns are written for any input.
+ *   No host sync, no allocation: the call can be captured in a CUDA graph.
  * vcr_eval_metrics: model/vcrnet_model.py:583-630 per-batch metrics accumulated into device double acc[8] =
  *   {pose loss, cycle loss, mse_ab, mae_ab, mse_ba, mae_ba, examples, -}, each weighted by the batch size. */
 int vcr_make_pairs(const float* base, int P, int Nb, const int* idx_src, const int* idx_tgt, const double* pose,
                    int N, double* src64, double* tgt64, float* src, float* tgt, cudaStream_t stream);
 int vcr_crop_nearest(const double* pc64, int P, int N, int keep, float* out, cudaStream_t stream);
+size_t vcr_crop_nearest_workspace_bytes(int P, int N);
+int vcr_crop_nearest_sort(const double* pc64, int P, int N, int keep, float* out, void* workspace, size_t workspace_bytes,
+                          cudaStream_t stream);
 int vcr_eval_metrics(const float* src, const float* tgt, int N, const float* srcK, const float* corrK, int M,
                      const float* R_gt, const float* t_gt, const float* R_ab, const float* t_ab,
                      const float* R_ba, const float* t_ba, int B, double* acc, cudaStream_t stream);

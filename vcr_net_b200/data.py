@@ -13,6 +13,7 @@ import math
 import numpy as np
 import torch
 
+from . import ops
 from ._lib import lib
 
 
@@ -82,10 +83,8 @@ class PairGenerator:
             t64 = torch.empty((P, 3, N), dtype=torch.float64, device=dev)
             L.check(L.vcr_make_pairs(base.data_ptr(), P, Nb, d_is.data_ptr(), d_it.data_ptr(), d_pose.data_ptr(), N,
                                      s64.data_ptr(), t64.data_ptr(), None, None, st), "vcr_make_pairs")
-            src = torch.empty((P, 3, keep), dtype=torch.float32, device=dev)
-            tgt = torch.empty((P, 3, keep), dtype=torch.float32, device=dev)
-            L.check(L.vcr_crop_nearest(s64.data_ptr(), P, N, keep, src.data_ptr(), st), "vcr_crop_nearest")
-            L.check(L.vcr_crop_nearest(t64.data_ptr(), P, N, keep, tgt.data_ptr(), st), "vcr_crop_nearest")
+            src = ops.crop_nearest(s64, keep)
+            tgt = ops.crop_nearest(t64, keep)
         else:
             src = torch.empty((P, 3, N), dtype=torch.float32, device=dev)
             tgt = torch.empty((P, 3, N), dtype=torch.float32, device=dev)

@@ -134,6 +134,49 @@ def fps(xyz: torch.Tensor, npoint: int, want64: bool = True):
 
 
 # --------------------------------------------------------------------------------------------------
+# nearest-to-anchor crop of the data step
+# --------------------------------------------------------------------------------------------------
+
+# vcr_crop_nearest: one CTA per cloud (its fp64 distances in shared memory) up to 25 600 points; vcr_crop_nearest_sort:
+# a segmented radix sort in a workspace, any cloud size while the batch holds at most 2^31 - 1 points
+CROP_ONE_CTA_MAX_POINTS = 25600
+CROP_MAX_TOTAL_POINTS = 2**31 - 1
+
+
+def crop_nearest(pc64: torch.Tensor, keep: int):
+    """pc64 fp64 [P,3,N] -> fp32 [P,3,keep]: the keep points nearest to point N-1, nearest first, ties to the lower index
+    (util/data.py:320-329).  Up to 25 600 points the one-CTA rank-count kernel, above that the radix sort."""
+    _chk(pc64, "pc64", torch.float64)
+    P, C, N = pc64.shape
+    assert C == 3
+    if N > CROP_ONE_CTA_MAX_POINTS:
+        return crop_nearest_sort(pc64, keep)
+    pc64 = pc64.contiguous()
+    out = torch.empty((P, 3, keep), dtype=_F32, device=pc64.device)
+    L = lib()
+    L.check(L.vcr_crop_nearest(pc64.data_ptr(), P, N, keep, out.data_ptr(), _stream(pc64)), "vcr_crop_nearest")
+    return out
+
+
+def crop_nearest_sort(pc64: torch.Tensor, keep: int):
+    """crop_nearest by the segmented radix sort (vcr_crop_nearest_sort) at any N; P * N <= 2^31 - 1."""
+    _chk(pc64, "pc64", torch.float64)
+    P, C, N = pc64.shape
+    assert C == 3
+    if P * N > CROP_MAX_TOTAL_POINTS:
+        raise RuntimeError(f"vcr_crop_nearest_sort: the crop takes at most {CROP_MAX_TOTAL_POINTS} points per call "
+                           f"(clouds x points), got {P} x {N}")
+    pc64 = pc64.contiguous()
+    out = torch.empty((P, 3, keep), dtype=_F32, device=pc64.device)
+    L = lib()
+    wsb = L.vcr_crop_nearest_workspace_bytes(P, N)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=pc64.device)
+    L.check(L.vcr_crop_nearest_sort(pc64.data_ptr(), P, N, keep, out.data_ptr(), ws.data_ptr(), wsb, _stream(pc64)),
+            "vcr_crop_nearest_sort")
+    return out
+
+
+# --------------------------------------------------------------------------------------------------
 # GEMM
 # --------------------------------------------------------------------------------------------------
 
