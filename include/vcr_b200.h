@@ -66,6 +66,17 @@ int vcr_set_knn_tc_tpq(int on);
 size_t vcr_knn_tc_workspace_bytes(int B, int N);
 int vcr_knn_topk_tc(const float* x, const void* xop, int ld, long long plane_stride, int B, int D, int N, int k,
                     int32_t* idx32, int64_t* idx64, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+/* Ragged batches of both: item b holds n[b] real points (int32, device; clamped to [k+1, N]) in its N rows, the rest is
+ * padding of any value.  Candidates j >= n[b] are never ranked, the tensor-core certificate's max |x|^2 is taken over the
+ * real points, and the indices of a real query equal those of vcr_knn_topk / vcr_knn_topk_tc on the item alone.  A padded
+ * query (n[b] <= q < N) gets its own index q in all k slots, so EdgeConv / gather-max over the graph stay in bounds.  The
+ * lengths are read on the device only (no host sync): a captured graph can be replayed with new lengths.  Same workspace
+ * sizes and the same vcr_set_knn3_direct / vcr_set_knn_tc_tpq routes. */
+int vcr_knn_topk_ragged(const float* x, const int* n, int B, int D, int N, int k, int token_major, int32_t* idx32,
+                        int64_t* idx64, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+int vcr_knn_topk_tc_ragged(const float* x, const void* xop, int ld, long long plane_stride, const int* n, int B, int D,
+                           int N, int k, int32_t* idx32, int64_t* idx64, void* workspace, size_t workspace_bytes,
+                           cudaStream_t stream);
 
 /* ---- get_graph_feature: util/util.py:176-199 ---------------------------------------------------
  * xt token-major [B,N,D]; idx [B,N,k]; out [B,2D,N,k] contiguous = concat(x[idx], x centre). */
@@ -117,6 +128,16 @@ int vcr_flash_attn_tc(const void* Q, int ldq, long long q_plane, const void* K, 
                       const void* VT, int ldv, long long v_plane, int B, int H, int Nq, int Nk, int dk,
                       int mode, float scale, const uint8_t* keep, void* O, int ldo, long long o_plane,
                       float* lse, cudaStream_t stream);
+/* Ragged batch: item b has nq[b] queries and nk[b] keys (int32, device; clamped to [1, Nq] / [1, Nk]) in its Nq / Nk
+ * rows.  Key tiles past nk[b] are not loaded, keys past nk[b] in the last tile get -inf whatever their score (the tail
+ * treatment of a call with Nk = nk[b]), and a 128-query tile wholly past nq[b] is written as zeros after one key tile.
+ * Output rows of real queries equal vcr_flash_attn_tc on the item alone bit for bit, provided the padded V columns of the
+ * item's last key tile are finite (their probabilities are exactly 0).  Runs organisation 3 whatever vcr_set_flash_warps
+ * says (2 gives the same bits); no key mask, no lse. */
+int vcr_flash_attn_tc_ragged(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                             const void* VT, int ldv, long long v_plane, const int* nq, const int* nk, int B, int H,
+                             int Nq, int Nk, int dk, int mode, float scale, void* O, int ldo, long long o_plane,
+                             cudaStream_t stream);
 /* Organisation of vcr_flash_attn_tc: 3 (default) = Q and P in tensor memory (tcgen05.mma with the A operand in TMEM; P is
  * written over the S tile it came from), 8 softmax warps; 2 = every operand in shared memory, 8 warps on every key tile
  * (same bits as 3); 4 = 16 warps; 1 = two groups of 4 warps alternating key tiles.  Process-wide tuning knob; returns the
@@ -221,6 +242,13 @@ int vcr_negdist(float* dot, int ld, int B, int Ns, int Nt, const float* xx, cons
 int vcr_softcorr_tc(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
                     const float* xx, const float* yy, const float* tgt, int B, int Ns, int Nt, int D,
                     float* corr, cudaStream_t stream);
+/* Ragged batch: pair b has ns[b] sources and nt[b] targets (int32, device; clamped to [1, Ns] / [1, Nt]) in its Ns / Nt
+ * rows.  128-source tiles past ns[b] and target tiles past nt[b] are skipped, targets past nt[b] in the last tile get the
+ * tail treatment of a call with Nt = nt[b], the online softmax visits the tiles in the same order, and corr columns >= ns[b]
+ * are written as 0: columns < ns[b] equal vcr_softcorr_tc on the pair alone, bit for bit. */
+int vcr_softcorr_tc_ragged(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
+                           const float* xx, const float* yy, const float* tgt, const int* ns, const int* nt, int B,
+                           int Ns, int Nt, int D, float* corr, cudaStream_t stream);
 /* getCopair (:264-332) through the same fused kernel: best_idx[B,Ns] = argmax_j pd_ij (ties -> lower j),
  * best_val[B,Ns] = max_j softmax_j(pd_ij) -- the hard correspondences of the partial path. */
 int vcr_softcorr_best_tc(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
@@ -261,6 +289,13 @@ int vcr_copair_gather(const float* src, const float* tgt, int B, int Ns, int Nt,
  * src, corr [B,3,M] -> R_ab [B,3,3], t_ab [B,3]; optional R_ba = R^T, t_ba = -R^T t, H (covariance). */
 int vcr_svd_head(const float* src, const float* corr, int B, int M, float* R_ab, float* t_ab,
                  float* R_ba, float* t_ba, float* H_out, cudaStream_t stream);
+/* Ragged batch: pair b has m[b] points (int32, device; clamped to [1, M]) in its M columns; the fp64 means and covariance
+ * run over exactly those points in the order of a call on the pair alone, so the outputs equal it bit for bit. */
+int vcr_svd_head_ragged(const float* src, const float* corr, const int* m, int B, int M, float* R_ab, float* t_ab,
+                        float* R_ba, float* t_ba, float* H_out, cudaStream_t stream);
+/* out [B,C,N] = x with columns n >= len[b] (len clamped to [lo, N]) set to 0: the padding of a ragged batch made finite and
+ * independent of what the caller left there.  out may be x. */
+int vcr_zero_padding(const float* x, const int* len, int B, int C, int N, int lo, float* out, cudaStream_t stream);
 int vcr_rigid_apply(const float* pc, const float* R, const float* t, int B, int N, float* out, cudaStream_t stream);
 int vcr_pose_compose(const float* R_i, const float* t_i, float* R_f, float* t_f, int B, cudaStream_t stream);
 int vcr_pose_inverse(const float* R, const float* t, float* R_inv, float* t_inv, int B, cudaStream_t stream);

@@ -35,6 +35,8 @@ struct AttnParams {
     int B, H, Nq, Nk;
     float scale_log2;             // softmax scale * log2(e)
     const uint8_t* keep;          // [B, Nk] or null
+    const int* nq_len;            // ragged batch (flash_attn_ts_kernel only): queries of item b, or null
+    const int* nk_len;            // keys of item b, or null (a uniform batch)
     __half* O; int ldo; long long o_plane;
     float* lse;                   // [B, H, Nq] log2-domain log-sum-exp, or null
     int out_bf16;
@@ -72,6 +74,14 @@ __device__ __forceinline__ float ex2_approx(float x) {
 // 640 threads).  The softmax is a chain of dependent phases (TMEM load, max, exchange, exp2, split, store) per tile, and
 // with two warps per scheduler the chain's latency, not its ~380 instructions, set the tile period (ncu: tensor pipe
 // 50 % active, stalls on scoreboards and the pair barrier); four warps per scheduler with half the chain each hide it.
+// Key tiles item (b, query tile qt) walks: all of them in a uniform batch; in a ragged batch those up to item b's key count,
+// and a single tile for a query tile wholly past the item's queries (its output rows are written as zeros).
+__device__ __forceinline__ int attn_item_kv_tiles(const AttnParams& p, int b, int qt) {
+    if (p.nk_len == nullptr) return (p.Nk + BKV - 1) / BKV;
+    if (qt * BQ >= vcr_item_len(p.nq_len, b, p.Nq, 1)) return 1;
+    return (vcr_item_len(p.nk_len, b, p.Nk, 1) + BKV - 1) / BKV;
+}
+
 __device__ __forceinline__ int ordered_key(float f) { const int b = __float_as_int(f); return b >= 0 ? b : b ^ 0x7fffffff; }
 __device__ __forceinline__ float ordered_val(int k) { return __int_as_float(k >= 0 ? k : k ^ 0x7fffffff); }
 constexpr int kNegInfKey = (int)0x807fffffu;         // ordered_key(-inf)
@@ -732,7 +742,6 @@ flash_attn_ts_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int nqt = (p.Nq + BQ - 1) / BQ;
-    const int nkv = (p.Nk + BKV - 1) / BKV;
     const long long items = (long long)p.B * p.H * nqt;
 
     if (warp == 0 && lane == 0) { tc::tma_prefetch_desc(&tmQ); tc::tma_prefetch_desc(&tmK); tc::tma_prefetch_desc(&tmV); }
@@ -769,6 +778,7 @@ flash_attn_ts_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
                     for (int pl = 0; pl < PL; ++pl)
                         tc::tma_load_3d(smem + (kb * PL + pl) * C_::Q_TILE, &tmQ, q_full, hh * DK + kb * 64,
                                         b * p.Nq + qt * BQ, pl);
+                const int nkv = attn_item_kv_tiles(p, b, qt);
                 for (int j = 0; j < nkv; ++j, ++g) {
                     const int s = g & 1;
                     uint8_t* st = smem + C_::OFF_KV + s * C_::KV_STAGE;
@@ -838,6 +848,7 @@ flash_attn_ts_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
                 ++g_qk;
             };
             for (long long it = blockIdx.x; it < items; it += gridDim.x, ++w) {
+                const int nkv = attn_item_kv_tiles(p, (int)(it / nqt) / p.H, (int)(it % nqt));
                 tc::mbar_wait(qt_full, w & 1);
                 tc::tc_fence_after();
                 issue_qk();
@@ -908,16 +919,19 @@ flash_attn_ts_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
             const int bh = (int)(it / nqt);
             const int hh = bh % p.H, b = bh / p.H;
             const uint8_t* keep = p.keep ? p.keep + (size_t)b * p.Nk : nullptr;
+            const int nkv = attn_item_kv_tiles(p, b, qt);
+            const int nk_b = vcr_item_len(p.nk_len, b, p.Nk, 1);
+            const bool q_live = qt * BQ < vcr_item_len(p.nq_len, b, p.Nq, 1);
             float m_used = -INFINITY, l = 0.f;
             for (int j = 0; j < nkv; ++j, ++g) {
                 const int sb = g & 1;
-                // additive score bias of key (this warp's column `lane`): 0 = kept, -1e9 (log2 domain) = masked, -inf = past Nk;
-                // requested before the wait on S, broadcast column by column with shuffles below
-                const bool biased = keep != nullptr || j * BKV + BKV > p.Nk;      // warp-uniform
+                // additive score bias of key (this warp's column `lane`): 0 = kept, -1e9 (log2 domain) = masked, -inf = past
+                // the item's keys; requested before the wait on S, broadcast column by column with shuffles below
+                const bool biased = keep != nullptr || j * BKV + BKV > nk_b;      // warp-uniform
                 float bias_l = 0.f;
                 if (biased) {
                     const int key = j * BKV + hf * CW + lane;
-                    if (key >= p.Nk) bias_l = -INFINITY;
+                    if (key >= nk_b) bias_l = -INFINITY;
                     else if (keep != nullptr && __ldg(keep + key) == 0) bias_l = -1e9f * kLog2e;
                 }
                 tc::mbar_wait(&s_full[sb], (g >> 1) & 1);
@@ -934,7 +948,11 @@ flash_attn_ts_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
                 float sc = p.scale_log2;
                 if (biased) {                                     // one shuffle + one fma per score (the bias is the same for every row)
 #pragma unroll
-                    for (int i = 0; i < CW; ++i) s[i] = fmaf(s[i], sc, __shfl_sync(0xffffffffu, bias_l, i));
+                    for (int i = 0; i < CW; ++i) {
+                        const float bi = __shfl_sync(0xffffffffu, bias_l, i);
+                        // a key past the item is -inf whatever its score (the padding of a ragged batch may hold anything)
+                        s[i] = bi == -INFINITY ? -INFINITY : fmaf(s[i], sc, bi);
+                    }
                     sc = 1.f;
                 }
                 float mt;
@@ -1027,6 +1045,10 @@ flash_attn_ts_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
 #pragma unroll
                     for (int i = 0; i < 32; ++i) v[c + i] = __uint_as_float(r0[i]) * inv_l;
                 }
+            }
+            if (!q_live) {                                        // query tile past the item's queries: rows written as 0
+#pragma unroll
+                for (int i = 0; i < OW; ++i) v[i] = 0.f;
             }
             tc::tc_fence_before();
             tc::mbar_arrive(o_empty);
@@ -1127,7 +1149,7 @@ VCR_API int vcr_flash_attn_tc(const void* Q, int ldq, long long q_plane, const v
     if (rc != VCR_OK) return rc;
     AttnParams p;
     p.B = B; p.H = H; p.Nq = Nq; p.Nk = Nk;
-    p.scale_log2 = scale * kLog2e; p.keep = keep;
+    p.scale_log2 = scale * kLog2e; p.keep = keep; p.nq_len = nullptr; p.nk_len = nullptr;
     p.O = reinterpret_cast<__half*>(O); p.ldo = ldo; p.o_plane = o_plane; p.lse = lse; p.out_bf16 = mode == 2;
     const int org = g_vcr_flash_warps.load(std::memory_order_relaxed);
     if (org == 3) {
@@ -1148,4 +1170,33 @@ VCR_API int vcr_flash_attn_tc(const void* Q, int ldq, long long q_plane, const v
     if (mode == 0) return launch_attn<3, 0, 2>(tq, tk, tv, p, stream);
     if (mode == 1) return launch_attn<1, 0, 2>(tq, tk, tv, p, stream);
     return launch_attn<1, 1, 2>(tq, tk, tv, p, stream);
+}
+
+// Ragged batch: item b has nq[b] queries and nk[b] keys (each clamped to [1, Nq] / [1, Nk]) in its Nq / Nk rows.  Key tiles
+// past nk[b] are not loaded, the last one is masked as the tail of a call with Nk = nk[b], and a query tile wholly past
+// nq[b] is written as zeros after one key tile.  Rows of a real query equal vcr_flash_attn_tc on the item alone, bit for
+// bit, provided the padded V columns of the last key tile are finite (their probability is exactly 0).  Always the default
+// organisation (Q and P in tensor memory); no key mask, no lse.
+VCR_API int vcr_flash_attn_tc_ragged(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                                     const void* VT, int ldv, long long v_plane, const int* nq, const int* nk, int B, int H,
+                                     int Nq, int Nk, int dk, int mode, float scale, void* O, int ldo, long long o_plane,
+                                     cudaStream_t stream) {
+    VCR_REQUIRE(Q && K && VT && O && nq && nk && B > 0 && H > 0 && Nq > 0 && Nk > 0);
+    if (dk != DK || mode < 0 || mode > 2) return VCR_ERR_UNSUPPORTED;
+    if ((ldo & 7) || (o_plane & 7)) return VCR_ERR_INVALID;
+    const int planes = mode == 0 ? 2 : 1;
+    CUtensorMap tq, tk, tv;
+    int rc = vcr_make_operand_tmap(&tq, Q, H * DK, (long long)B * Nq, ldq, q_plane, planes, BQ);
+    if (rc != VCR_OK) return rc;
+    rc = vcr_make_operand_tmap(&tk, K, H * DK, (long long)B * Nk, ldk, k_plane, planes, BKV);
+    if (rc != VCR_OK) return rc;
+    rc = vcr_make_operand_tmap(&tv, VT, Nk, (long long)B * H * DK, ldv, v_plane, planes, DK);
+    if (rc != VCR_OK) return rc;
+    AttnParams p;
+    p.B = B; p.H = H; p.Nq = Nq; p.Nk = Nk;
+    p.scale_log2 = scale * kLog2e; p.keep = nullptr; p.nq_len = nq; p.nk_len = nk;
+    p.O = reinterpret_cast<__half*>(O); p.ldo = ldo; p.o_plane = o_plane; p.lse = nullptr; p.out_bf16 = mode == 2;
+    if (mode == 0) return launch_attn_ts<3, 0>(tq, tk, tv, p, stream);
+    if (mode == 1) return launch_attn_ts<1, 0>(tq, tk, tv, p, stream);
+    return launch_attn_ts<1, 1>(tq, tk, tv, p, stream);
 }

@@ -31,6 +31,12 @@ static inline int vcr_cdiv(long long a, long long b) { return (int)((a + b - 1) 
 
 __device__ __forceinline__ float leaky(float v, float slope) { return v >= 0.f ? v : v * slope; }
 
+// Length of item b of a ragged batch (the *_ragged entry points): len[b] clamped to [lo, n_max], so that an out-of-range
+// length stays in bounds; n_max when len is null (a uniform batch).
+__device__ __forceinline__ int vcr_item_len(const int* len, int b, int n_max, int lo) {
+    return len != nullptr ? min(max(__ldg(len + b), lo), n_max) : n_max;
+}
+
 __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));

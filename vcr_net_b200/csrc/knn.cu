@@ -251,12 +251,30 @@ struct Smem {
     static constexpr size_t total = region0 + (size_t)TC * sizeof(float) + (size_t)TQ * TC * sizeof(float);
 };
 
+// Ragged batches (nlen != null): item b holds nlen[b] real points in its N rows.  Candidates past it are never ranked, and
+// a padded query (nlen[b] <= q < N) gets its own index in all k slots, so consumers of the graph stay inside the cloud.
+__device__ __forceinline__ void knn_write_self(int32_t* idx32, int64_t* idx64, int b, int N, int k, int q0, int nq, int tid,
+                                               int nthreads) {
+    for (int e = tid; e < nq * k; e += nthreads) {
+        const int q = q0 + e / k;
+        const size_t o = ((size_t)b * N + q) * k + e % k;
+        if (idx32) idx32[o] = q;
+        if (idx64) idx64[o] = (int64_t)q;
+    }
+}
+
 template <int DCH, bool TOKEN_MAJOR>
 __global__ void __launch_bounds__(NT, 2)
 knn_select_kernel(const float* __restrict__ x, const float* __restrict__ xx, int D, int N, int k,
-                  int32_t* __restrict__ idx32, int64_t* __restrict__ idx64, const int* __restrict__ redo) {
+                  int32_t* __restrict__ idx32, int64_t* __restrict__ idx64, const int* __restrict__ redo,
+                  const int* __restrict__ nlen) {
     // redo != null: this launch only repairs the 32-query groups the tensor-core kernel could not certify
     if (redo != nullptr && redo[blockIdx.y * gridDim.x + blockIdx.x] == 0) return;
+    const int Nb = vcr_item_len(nlen, blockIdx.y, N, k + 1);
+    if ((int)blockIdx.x * TQ >= Nb) {                     // every query of the CTA is padding
+        knn_write_self(idx32, idx64, blockIdx.y, N, k, blockIdx.x * TQ, min(TQ, N - (int)blockIdx.x * TQ), threadIdx.x, NT);
+        return;
+    }
     using S = Smem<DCH>;
     constexpr int DCP = S::DCP;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -277,7 +295,7 @@ knn_select_kernel(const float* __restrict__ x, const float* __restrict__ xx, int
 #pragma unroll
     for (int w = 0; w < QW; ++w) run[w].hi = run[w].lo = 0u;
 
-    for (int j0 = 0; j0 < N; j0 += TC) {
+    for (int j0 = 0; j0 < Nb; j0 += TC) {
         float acc[8][8];
 #pragma unroll
         for (int qi = 0; qi < 8; ++qi)
@@ -321,7 +339,7 @@ knn_select_kernel(const float* __restrict__ x, const float* __restrict__ xx, int
 
             const float* qrow = Qb + (qg * 8) * DCP;
             const float* crow = Cb + (cg * 256 + lane) * DCP;
-            if (j0 + cg * 256 < N) {               // else this warp's 256 candidates are all past N (e.g. N = 768): warp-uniform
+            if (j0 + cg * 256 < Nb) {              // else this warp's 256 candidates are all past N (e.g. N = 768): warp-uniform
 #pragma unroll 1   // (a fully unrolled body makes ptxas rotate the 64 accumulators: +20% MOVs and spills at 128 regs)
             for (int d4 = 0; d4 < DCH / 4; ++d4) {
 #pragma unroll
@@ -360,7 +378,7 @@ knn_select_kernel(const float* __restrict__ x, const float* __restrict__ xx, int
         for (int ci = 0; ci < 8; ++ci) {
             const int c = cg * 256 + ci * 32 + lane;
             const float nxc = -xxc[c];
-            const bool cvalid = j0 + c < N;
+            const bool cvalid = j0 + c < Nb;
 #pragma unroll
             for (int qi = 0; qi < 8; ++qi) {
                 const float pd = __fsub_rn(__fsub_rn(nxc, -2.f * acc[qi][ci]), xxq[qi]);
@@ -378,7 +396,7 @@ knn_select_kernel(const float* __restrict__ x, const float* __restrict__ xx, int
     for (int w = 0; w < QW; ++w) {
         const int q = q0 + warp * QW + w;
         if (q < N && lane >= 1 && lane <= k) {
-            const int j = (int)(~run[w].lo);
+            const int j = q < Nb ? (int)(~run[w].lo) : q;
             const size_t o = ((size_t)b * N + q) * k + lane - 1;
             if (idx32) idx32[o] = j;
             if (idx64) idx64[o] = (int64_t)j;
@@ -388,13 +406,13 @@ knn_select_kernel(const float* __restrict__ x, const float* __restrict__ xx, int
 
 template <int DCH, bool TM>
 int launch_knn(const float* x, const float* xx, int B, int D, int N, int k, int32_t* i32, int64_t* i64,
-               cudaStream_t st, const int* redo = nullptr) {
+               cudaStream_t st, const int* redo = nullptr, const int* nlen = nullptr) {
     auto kern = knn_select_kernel<DCH, TM>;
     const size_t smem = Smem<DCH>::total;
     // set on every launch: the attribute is per device, and one process may drive several (nn.DataParallel)
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return VCR_ERR_LAUNCH;
     dim3 grid(vcr_cdiv(N, TQ), B);
-    kern<<<grid, NT, smem, st>>>(x, xx, D, N, k, i32, i64, redo);
+    kern<<<grid, NT, smem, st>>>(x, xx, D, N, k, i32, i64, redo, nlen);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
 }
@@ -455,18 +473,23 @@ constexpr int TQ3 = QW3 * (NT / 32);     // queries per CTA
 template <bool TOKEN_MAJOR>
 __global__ void __launch_bounds__(NT, 4)
 knn3_kernel(const float* __restrict__ x, const float* __restrict__ xx, int N, int k,
-            int32_t* __restrict__ idx32, int64_t* __restrict__ idx64) {
+            int32_t* __restrict__ idx32, int64_t* __restrict__ idx64, const int* __restrict__ nlen) {
     __shared__ float cs[4][TC];                       // x | y | z | xx of the chunk's candidates
     __shared__ uint2 surv[NT / 32][TC];               // per-warp survivor buffers
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.y, q0 = blockIdx.x * TQ3;
     const float* xb = x + (size_t)b * 3 * N;
     const float* xxb = xx + (size_t)b * N;
+    const int Nb = vcr_item_len(nlen, b, N, k + 1);
+    if (q0 >= Nb) {                                   // every query of the CTA is padding
+        knn_write_self(idx32, idx64, b, N, k, q0, min(TQ3, N - q0), tid, NT);
+        return;
+    }
 
     float qx[QW3], qy[QW3], qz[QW3], xxq[QW3];
 #pragma unroll
     for (int w = 0; w < QW3; ++w) {
-        const int q = min(q0 + warp * QW3 + w, N - 1);  // queries past N are computed and not written
+        const int q = min(q0 + warp * QW3 + w, Nb - 1); // queries past the cloud are computed and not written
         qx[w] = TOKEN_MAJOR ? xb[(size_t)q * 3 + 0] : xb[q];
         qy[w] = TOKEN_MAJOR ? xb[(size_t)q * 3 + 1] : xb[(size_t)N + q];
         qz[w] = TOKEN_MAJOR ? xb[(size_t)q * 3 + 2] : xb[2 * (size_t)N + q];
@@ -477,7 +500,7 @@ knn3_kernel(const float* __restrict__ x, const float* __restrict__ xx, int N, in
     for (int w = 0; w < QW3; ++w) run[w].hi = run[w].lo = 0u;
     uint2* buf = surv[warp];
 
-    for (int j0 = 0; j0 < N; j0 += TC) {
+    for (int j0 = 0; j0 < Nb; j0 += TC) {
         __syncthreads();                               // the previous chunk's rows are no longer read
         for (int c = tid; c < TC; c += NT) {
             const int g = j0 + c;
@@ -492,7 +515,7 @@ knn3_kernel(const float* __restrict__ x, const float* __restrict__ xx, int N, in
             const int c = r * 32 + lane;
             const float acc = fmaf(qz[w], cs[2][c], fmaf(qy[w], cs[1][c], fmaf(qx[w], cs[0][c], 0.f)));
             const float v = __fsub_rn(__fsub_rn(-cs[3][c], -2.f * acc), xxq[w]);
-            return j0 + c < N ? v : -INFINITY;
+            return j0 + c < Nb ? v : -INFINITY;
         };
         float tau[QW3];
         if (j0 == 0) {
@@ -526,7 +549,7 @@ knn3_kernel(const float* __restrict__ x, const float* __restrict__ xx, int N, in
     for (int w = 0; w < QW3; ++w) {
         const int q = q0 + warp * QW3 + w;
         if (q < N && lane >= 1 && lane <= k) {
-            const int j = (int)(~run[w].lo);
+            const int j = q < Nb ? (int)(~run[w].lo) : q;
             const size_t o = ((size_t)b * N + q) * k + lane - 1;
             if (idx32) idx32[o] = j;
             if (idx64) idx64[o] = (int64_t)j;
@@ -569,6 +592,7 @@ struct KnnTcParams {
     const uint32_t* xxmax;   // [B] bit pattern of max_j xx_j
     int* redo;               // [B * ceil(N/32)] flags for the exact kernel (one per CTA)
     int* nflag;              // [1] number of uncertified queries (telemetry)
+    const int* nlen;         // [B] points per item of a ragged batch, or null
     int D, N, k, ksel, KB;
     int32_t* idx32;
     int64_t* idx64;
@@ -583,7 +607,7 @@ __host__ __device__ constexpr size_t knn_tc_smem_bytes(int KB) {
 }
 
 __global__ void knn_sqnorm_max_kernel(const float* __restrict__ x, int D, int N, float* __restrict__ xx,
-                                      uint32_t* __restrict__ xxmax) {
+                                      uint32_t* __restrict__ xxmax, const int* __restrict__ nlen, int k) {
     const int b = blockIdx.y;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t bits = 0u;
@@ -592,7 +616,8 @@ __global__ void knn_sqnorm_max_kernel(const float* __restrict__ x, int D, int N,
         float acc = 0.f;
         for (int d = 0; d < D; ++d) acc = fmaf(r[d], r[d], acc);      // canonical chain (oracle/canon.c)
         xx[(size_t)b * N + i] = acc;
-        bits = __float_as_uint(acc);                                   // acc >= 0 (or NaN, which sorts above +inf)
+        // acc >= 0 (or NaN, which sorts above +inf); the maximum is taken over the real points only
+        if (i < vcr_item_len(nlen, b, N, k + 1)) bits = __float_as_uint(acc);
     }
     bits = __reduce_max_sync(0xffffffffu, bits);
     if ((threadIdx.x & 31) == 0 && bits) atomicMax(xxmax + b, bits);
@@ -620,7 +645,12 @@ knn_tc_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ C
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int b = blockIdx.y, q0 = blockIdx.x * TQ;
     const float* xxb = p.xx + (size_t)b * N;
-    const int nch = (N + TC - 1) / TC;
+    const int Nb = vcr_item_len(p.nlen, b, N, k + 1);
+    if (q0 >= Nb) {                                   // every query of the CTA is padding
+        knn_write_self(p.idx32, p.idx64, b, N, k, q0, min(TQ, N - q0), tid, T2NT);
+        return;
+    }
+    const int nch = (Nb + TC - 1) / TC;
 
     if (warp == NT / 32 && lane == 0) {
         tc::tma_prefetch_desc(&tmC); tc::tma_prefetch_desc(&tmQ);
@@ -659,7 +689,7 @@ knn_tc_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ C
                 if (c > 0) { tc::mbar_wait(stage_free, (c - 1) & 1); tc::tc_fence_after(); }
                 for (int t = 0; t < T2TILES; ++t, ++g) {
                     const int cand0 = c * TC + t * T2M;
-                    if (cand0 < N) {
+                    if (cand0 < Nb) {
                         tc::mbar_expect_tx(c_full, cbytes);
                         for (int kb = 0; kb < KB; ++kb)
                             for (int pl = 0; pl < 2; ++pl)
@@ -709,9 +739,9 @@ knn_tc_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ C
                 const int cl = t * T2M + qq * 32 + lane;                 // candidate of this thread within the chunk
                 const int j = j0 + cl;
                 float* dcol = dist + cl;
-                if (j0 + t * T2M < N) {                                  // warp-uniform: the tile holds data
+                if (j0 + t * T2M < Nb) {                                 // warp-uniform: the tile holds data
                     const uint32_t ta = tmem_base + ((uint32_t)(qq * 32) << 16) + t * TQ;
-                    const bool cvalid = j < N;
+                    const bool cvalid = j < Nb;
                     const float nxc = cvalid ? -xxb[j] : 0.f;
 #pragma unroll
                     for (int h = 0; h < 2; ++h) {
@@ -746,10 +776,14 @@ knn_tc_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ C
         for (int qi = 0; qi < QW; ++qi) {
             const int q = q0 + warp * QW + qi;
             if (q >= N) continue;                                        // warp-uniform
+            if (q >= Nb) {                                               // padded query: its own index
+                if (lane < k) knn_write_self(p.idx32, p.idx64, b, N, k, q, 1, lane, k);
+                continue;
+            }
             const Key a = run[qi];
             const uint32_t thr_hi = __shfl_sync(0xffffffffu, a.hi, ksel);
             const int j = (int)(~a.lo);
-            const bool valid = j >= 0 && j < N;
+            const bool valid = j >= 0 && j < Nb;
             const float xxq = xxq_s[warp * QW + qi];
             Key e[1];
             e[0].hi = 0u; e[0].lo = 0u;
@@ -817,9 +851,8 @@ VCR_API int vcr_set_knn_tc_tpq(int on) {
     return g_vcr_knn_tc_tpq.exchange(on < 0 ? 0 : (on > 2 ? 2 : on));
 }
 
-VCR_API int vcr_knn_topk(const float* x, int B, int D, int N, int k, int token_major, int32_t* idx32,
+static int knn_topk_impl(const float* x, const int* nlen, int B, int D, int N, int k, int token_major, int32_t* idx32,
                          int64_t* idx64, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
-    VCR_REQUIRE(x && (idx32 || idx64) && B > 0 && N > 0 && k >= 1);
     if (N < k + 1) return VCR_ERR_INVALID;
     if (!workspace || workspace_bytes < vcr_knn_workspace_bytes(B, N)) return VCR_ERR_WORKSPACE;
     float* xx = reinterpret_cast<float*>(workspace);
@@ -831,16 +864,30 @@ VCR_API int vcr_knn_topk(const float* x, int B, int D, int N, int k, int token_m
     const int route3 = g_vcr_knn3_direct.load(std::memory_order_relaxed);
     if (D == 3 && route3 != 0) {
         dim3 grid(vcr_cdiv(N, TQ3), B);
-        if (token_major) knn3_kernel<true><<<grid, NT, 0, stream>>>(x, xx, N, k, idx32, idx64);
-        else knn3_kernel<false><<<grid, NT, 0, stream>>>(x, xx, N, k, idx32, idx64);
+        if (token_major) knn3_kernel<true><<<grid, NT, 0, stream>>>(x, xx, N, k, idx32, idx64, nlen);
+        else knn3_kernel<false><<<grid, NT, 0, stream>>>(x, xx, N, k, idx32, idx64, nlen);
         VCR_CHECK_LAUNCH();
         return VCR_OK;
     }
     if (D <= 4)
-        return token_major ? launch_knn<4, true>(x, xx, B, D, N, k, idx32, idx64, stream)
-                           : launch_knn<4, false>(x, xx, B, D, N, k, idx32, idx64, stream);
-    return token_major ? launch_knn<16, true>(x, xx, B, D, N, k, idx32, idx64, stream)
-                       : launch_knn<16, false>(x, xx, B, D, N, k, idx32, idx64, stream);
+        return token_major ? launch_knn<4, true>(x, xx, B, D, N, k, idx32, idx64, stream, nullptr, nlen)
+                           : launch_knn<4, false>(x, xx, B, D, N, k, idx32, idx64, stream, nullptr, nlen);
+    return token_major ? launch_knn<16, true>(x, xx, B, D, N, k, idx32, idx64, stream, nullptr, nlen)
+                       : launch_knn<16, false>(x, xx, B, D, N, k, idx32, idx64, stream, nullptr, nlen);
+}
+
+VCR_API int vcr_knn_topk(const float* x, int B, int D, int N, int k, int token_major, int32_t* idx32,
+                         int64_t* idx64, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+    VCR_REQUIRE(x && (idx32 || idx64) && B > 0 && N > 0 && k >= 1);
+    return knn_topk_impl(x, nullptr, B, D, N, k, token_major, idx32, idx64, workspace, workspace_bytes, stream);
+}
+
+// Ragged batch: item b has n[b] real points (clamped to [k+1, N]) in its N rows.  Indices of real queries equal
+// vcr_knn_topk's on the item alone; padded queries get their own index in all k slots.
+VCR_API int vcr_knn_topk_ragged(const float* x, const int* n, int B, int D, int N, int k, int token_major, int32_t* idx32,
+                                int64_t* idx64, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+    VCR_REQUIRE(x && n && (idx32 || idx64) && B > 0 && N > 0 && k >= 1);
+    return knn_topk_impl(x, n, B, D, N, k, token_major, idx32, idx64, workspace, workspace_bytes, stream);
 }
 
 // ---- tensor-core prefilter + exact re-rank (16 <= D <= 128, token-major) --------------------------------------
@@ -849,13 +896,9 @@ VCR_API size_t vcr_knn_tc_workspace_bytes(int B, int N) {
     return ((size_t)B * N + (size_t)B + (size_t)B * ((N + 31) / 32) + 1) * 4;
 }
 
-// x: fp32 [B,N,D] token-major; xop: its operand-format copy [2 planes][B*N][ld] (fp16 hi, lo*2^11; vcr_to_operand).
-// Writes exactly what vcr_knn_topk writes (bit-identical indices) -- see the kernel comment for the certificate.
-// After the call, the last word of the workspace holds the number of queries that went through the exact kernel.
-VCR_API int vcr_knn_topk_tc(const float* x, const void* xop, int ld, long long plane_stride, int B, int D, int N, int k,
-                            int32_t* idx32, int64_t* idx64, void* workspace, size_t workspace_bytes,
+static int knn_topk_tc_impl(const float* x, const void* xop, int ld, long long plane_stride, const int* nlen, int B, int D,
+                            int N, int k, int32_t* idx32, int64_t* idx64, void* workspace, size_t workspace_bytes,
                             cudaStream_t stream) {
-    VCR_REQUIRE(x && xop && (idx32 || idx64) && B > 0 && N > 0 && k >= 1);
     if (N < k + 1) return VCR_ERR_INVALID;
     if (D < 16 || D > 128 || k > 30 || (long long)B * N > 0x7fffffffLL || B > 65535) return VCR_ERR_UNSUPPORTED;
     if (!workspace || workspace_bytes < vcr_knn_tc_workspace_bytes(B, N)) return VCR_ERR_WORKSPACE;
@@ -866,7 +909,7 @@ VCR_API int vcr_knn_topk_tc(const float* x, const void* xop, int ld, long long p
     int* nflag = redo + (size_t)B * nq32;
     if (cudaMemsetAsync(xxmax, 0, ((size_t)B + (size_t)B * nq32 + 1) * 4, stream) != cudaSuccess) return VCR_ERR_LAUNCH;
     dim3 g(vcr_cdiv(N, 256), B);
-    knn_sqnorm_max_kernel<<<g, 256, 0, stream>>>(x, D, N, xx, xxmax);
+    knn_sqnorm_max_kernel<<<g, 256, 0, stream>>>(x, D, N, xx, xxmax, nlen, k);
     VCR_CHECK_LAUNCH();
     CUtensorMap tmC, tmQ;
     const int tpq = g_vcr_knn_tc_tpq.load(std::memory_order_relaxed);
@@ -876,7 +919,7 @@ VCR_API int vcr_knn_topk_tc(const float* x, const void* xop, int ld, long long p
         rc = vcr_make_operand_tmap(&tmQ, xop, D, (long long)B * N, ld, plane_stride, 2, TQ2);
         if (rc != VCR_OK) return rc;
         KnnTcParams p;
-        p.x = x; p.xx = xx; p.xxmax = xxmax; p.redo = redo; p.nflag = nflag;
+        p.x = x; p.xx = xx; p.xxmax = xxmax; p.redo = redo; p.nflag = nflag; p.nlen = nlen;
         p.D = D; p.N = N; p.k = k; p.ksel = k + 8 < 31 ? k + 8 : 31; p.KB = (D + 63) / 64;
         p.idx32 = idx32; p.idx64 = idx64;
         const size_t smem = knn_tc2_smem_bytes(p.KB);
@@ -884,14 +927,14 @@ VCR_API int vcr_knn_topk_tc(const float* x, const void* xop, int ld, long long p
             return VCR_ERR_LAUNCH;
         knn_tc2_kernel<<<dim3(vcr_cdiv(N, TQ2), B), T2_THREADS, smem, stream>>>(tmC, tmQ, p);
         VCR_CHECK_LAUNCH();
-        return launch_knn<16, true>(x, xx, B, D, N, k, idx32, idx64, stream, redo);   // repairs flagged groups only
+        return launch_knn<16, true>(x, xx, B, D, N, k, idx32, idx64, stream, redo, nlen);   // repairs flagged groups only
     }
     int rc = vcr_make_operand_tmap(&tmC, xop, D, (long long)B * N, ld, plane_stride, 2, T2M);
     if (rc != VCR_OK) return rc;
     rc = vcr_make_operand_tmap(&tmQ, xop, D, (long long)B * N, ld, plane_stride, 2, TQ);
     if (rc != VCR_OK) return rc;
     KnnTcParams p;
-    p.x = x; p.xx = xx; p.xxmax = xxmax; p.redo = redo; p.nflag = nflag;
+    p.x = x; p.xx = xx; p.xxmax = xxmax; p.redo = redo; p.nflag = nflag; p.nlen = nlen;
     p.D = D; p.N = N; p.k = k; p.ksel = k + 8 < 31 ? k + 8 : 31; p.KB = (D + 63) / 64;
     p.idx32 = idx32; p.idx64 = idx64;
     const size_t smem = knn_tc_smem_bytes(p.KB);
@@ -899,5 +942,23 @@ VCR_API int vcr_knn_topk_tc(const float* x, const void* xop, int ld, long long p
         return VCR_ERR_LAUNCH;
     knn_tc_kernel<<<dim3(nq32, B), T2NT, smem, stream>>>(tmC, tmQ, p);
     VCR_CHECK_LAUNCH();
-    return launch_knn<16, true>(x, xx, B, D, N, k, idx32, idx64, stream, redo);       // repairs flagged groups only
+    return launch_knn<16, true>(x, xx, B, D, N, k, idx32, idx64, stream, redo, nlen);       // repairs flagged groups only
+}
+
+// x: fp32 [B,N,D] token-major; xop: its operand-format copy [2 planes][B*N][ld] (fp16 hi, lo*2^11; vcr_to_operand).
+// Writes exactly what vcr_knn_topk writes (bit-identical indices) -- see the kernel comment for the certificate.
+// After the call, the last word of the workspace holds the number of queries that went through the exact kernel.
+VCR_API int vcr_knn_topk_tc(const float* x, const void* xop, int ld, long long plane_stride, int B, int D, int N, int k,
+                            int32_t* idx32, int64_t* idx64, void* workspace, size_t workspace_bytes,
+                            cudaStream_t stream) {
+    VCR_REQUIRE(x && xop && (idx32 || idx64) && B > 0 && N > 0 && k >= 1);
+    return knn_topk_tc_impl(x, xop, ld, plane_stride, nullptr, B, D, N, k, idx32, idx64, workspace, workspace_bytes, stream);
+}
+
+// Ragged batch, as vcr_knn_topk_ragged: the maximum squared norm of the certificate is taken over item b's n[b] points.
+VCR_API int vcr_knn_topk_tc_ragged(const float* x, const void* xop, int ld, long long plane_stride, const int* n, int B,
+                                   int D, int N, int k, int32_t* idx32, int64_t* idx64, void* workspace,
+                                   size_t workspace_bytes, cudaStream_t stream) {
+    VCR_REQUIRE(x && xop && n && (idx32 || idx64) && B > 0 && N > 0 && k >= 1);
+    return knn_topk_tc_impl(x, xop, ld, plane_stride, n, B, D, N, k, idx32, idx64, workspace, workspace_bytes, stream);
 }

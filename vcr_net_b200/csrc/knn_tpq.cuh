@@ -157,7 +157,12 @@ knn_tc2_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int b = blockIdx.y, q0 = blockIdx.x * TQ2;
     const float* xxb = p.xx + (size_t)b * N;
-    const int ntiles = (N + TC2 - 1) / TC2;
+    const int Nb = vcr_item_len(p.nlen, b, N, k + 1);      // ragged batch: candidates and queries past Nb are padding
+    if (q0 >= Nb) {
+        knn_write_self(p.idx32, p.idx64, b, N, k, q0, min(TQ2, N - q0), tid, T2_THREADS);
+        return;
+    }
+    const int ntiles = (Nb + TC2 - 1) / TC2;
 
     if (warp == 4 && lane == 0) {
         tc::tma_prefetch_desc(&tmC); tc::tma_prefetch_desc(&tmQ);
@@ -233,7 +238,7 @@ knn_tc2_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ 
     } else {
         // ============================== consumers: thread = query ==============================
         const int q = q0 + tid;
-        const bool qok = q < N;
+        const bool qok = q < Nb;
         const float xxq = qok ? xxb[q] : 0.f;
         const uint32_t lane_adr = (uint32_t)(warp * 32) << 16;
         KP run[TPQ_L];
@@ -263,7 +268,7 @@ knn_tc2_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ 
                 const float nxc = -__ldg(xxb + min(j, N - 1));                  // warp-uniform address: one broadcast load
                 const float pd = __fsub_rn(__fsub_rn(nxc, -2.f * dot), xxq);
                 const uint32_t key = okey(pd);
-                if (qok && j < N && key > tau) {
+                if (qok && j < Nb && key > tau) {
                     buf.k[cnt * TQ2 + tid] = key;
                     buf.p[cnt * TQ2 + tid] = ~(uint32_t)j;
                     ++cnt;
@@ -288,7 +293,7 @@ knn_tc2_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ 
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 const int j = (int)(~run[g + u].p);
-                valid[u] = qok && g + u <= ksel && run[g + u].k != 0u && j >= 0 && j < N;
+                valid[u] = qok && g + u <= ksel && run[g + u].k != 0u && j >= 0 && j < Nb;
                 xj[u] = p.x + ((size_t)b * N + (valid[u] ? j : 0)) * D;
             }
             if (g <= ksel) {                                                     // warp-uniform
@@ -334,6 +339,8 @@ knn_tc2_kernel(const __grid_constant__ CUtensorMap tmC, const __grid_constant__ 
                     if (p.idx64) p.idx64[o + i - 1] = (int64_t)jn;
                 }
             }
+        } else if (!qok && q < N) {
+            knn_write_self(p.idx32, p.idx64, b, N, k, q, 1, 0, 1);     // padded query of a ragged batch
         }
         const uint32_t bad = __ballot_sync(0xffffffffu, !safe);
         if (bad != 0u && lane == 0) {

@@ -43,7 +43,17 @@ struct SoftcorrParams {
     const float* col_m;   // [B,Nt] per-column max        (mode 4)
     const float* col_il;  // [B,Nt] per-column 1 / sum    (mode 4)
     float* row_stat;      // [B,Ns] sum_j exp(pd_ij - col_m_j) * col_il_j   (mode 4)
+    const int* ns_len;    // ragged batch (mode 0): rows of item b, or null
+    const int* nt_len;    // columns of item b, or null (a uniform batch)
 };
+
+// Target tiles of work item (b, row tile m_blk): all of them in a uniform batch; in a ragged batch those up to item b's
+// column count, none for a row tile wholly past the item's rows (its corr columns are written as zeros).
+__device__ __forceinline__ int softcorr_item_tiles(const SoftcorrParams& p, int b, int m_blk) {
+    if (p.nt_len == nullptr) return (p.Nt + BN - 1) / BN;
+    if (m_blk * BM >= vcr_item_len(p.ns_len, b, p.Ns, 1)) return 0;
+    return (vcr_item_len(p.nt_len, b, p.Nt, 1) + BN - 1) / BN;
+}
 
 // SWAP: the rows (A, xx) are targets and the columns (B, yy) sources.
 template <int MODE, bool SWAP = false>
@@ -59,7 +69,7 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int tiles_m = (p.Ns + BM - 1) / BM, tiles_n = (p.Nt + BN - 1) / BN;
+    const int tiles_m = (p.Ns + BM - 1) / BM;
     const int items = p.B * tiles_m;
     const int nkb = (p.D + BK - 1) / BK;
 
@@ -82,6 +92,7 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
             for (int it = blockIdx.x; it < items; it += gridDim.x) {
                 const int b = it / tiles_m, m_blk = it - b * tiles_m;
                 const int a_row = b * p.Ns + m_blk * BM;
+                const int tiles_n = softcorr_item_tiles(p, b, m_blk);
                 for (int n_blk = 0; n_blk < tiles_n; ++n_blk) {
                     const int b_row = b * p.Nt + n_blk * BN;
                     for (int kb = 0; kb < nkb; ++kb) {
@@ -105,6 +116,7 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
             int s = 0; uint32_t ph = 0;
             int tl = 0;                                               // running tile counter of this CTA
             for (int it = blockIdx.x; it < items; it += gridDim.x) {
+                const int tiles_n = softcorr_item_tiles(p, it / tiles_m, it % tiles_m);
                 for (int n_blk = 0; n_blk < tiles_n; ++n_blk, ++tl) {
                     const int a = tl & 1;
                     const uint32_t aph = (tl >> 1) & 1;
@@ -151,7 +163,16 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         for (int it = blockIdx.x; it < items; it += gridDim.x) {
             const int b = it / tiles_m, m_blk = it - b * tiles_m;
             const int row = m_blk * BM + rloc;
-            const bool row_ok = row < p.Ns;
+            const int tiles_n = softcorr_item_tiles(p, b, m_blk);
+            const int ns_b = vcr_item_len(p.ns_len, b, p.Ns, 1), nt_b = vcr_item_len(p.nt_len, b, p.Nt, 1);
+            const bool row_ok = row < ns_b;
+            if (MODE == 0 && !row_ok) {                        // ragged batch: rows past the item's sources get corr = 0
+                if (chalf == 0 && row < p.Ns) {
+                    float* cb = p.corr + (size_t)b * 3 * p.Ns;
+                    cb[row] = 0.f; cb[p.Ns + row] = 0.f; cb[2 * p.Ns + row] = 0.f;
+                }
+                if (tiles_n == 0) continue;                    // item without target tiles: nothing else to do (uniform per item)
+            }
             const float nx = row_ok ? -p.xx[(size_t)b * p.Ns + row] : 0.f;
             const float* yb = p.yy + (size_t)b * p.Nt;
             const float* tb = MODE == 0 ? p.tgt + (size_t)b * 3 * p.Nt : nullptr;
@@ -166,7 +187,7 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 #pragma unroll
                 for (int q = 0; q < 2; ++q) {
                     const int cj = col_h + q * 32 + lane;
-                    const bool ok = cj < p.Nt;
+                    const bool ok = cj < nt_b;
                     cols[q * 32 + lane] = ok ? yb[cj] : 0.f;
                     if (MODE == 0) {
                         cols[64 + q * 32 + lane] = ok ? tb[cj] : 0.f;
@@ -185,7 +206,7 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 #pragma unroll 1
                 for (int cc = 0; cc < 2; ++cc) {
                     const int col0 = col_h + cc * 32;
-                    if (col0 >= p.Nt) break;                   // warp-uniform
+                    if (col0 >= nt_b) break;                   // warp-uniform
                     float pd[32];
                     {
                         uint32_t r0[32], r1[32];
@@ -200,10 +221,10 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                             else pd[j] = __fsub_rn(__fsub_rn(nx, -2.f * dot), cols[cc * 32 + j]);
                         }
                     }
-                    if (col0 + 32 > p.Nt) {
+                    if (col0 + 32 > nt_b) {
 #pragma unroll
                         for (int j = 0; j < 32; ++j)
-                            if (col0 + j >= p.Nt) pd[j] = -INFINITY;
+                            if (col0 + j >= nt_b) pd[j] = -INFINITY;
                     }
                     if (MODE == 4) {                           // columns past Nt: exp(-inf) * 0
 #pragma unroll
@@ -366,4 +387,23 @@ VCR_API int vcr_select_stats_tc(const void* S, int lds, long long s_plane, const
     pt.col_m = mr; pt.col_il = ilr; pt.row_stat = col_stat;
     if ((rc = softcorr_run<4, false>(tmS, tmT, ps, stream)) != VCR_OK) return rc;
     return softcorr_run<4, true>(tmT, tmS, pt, stream);
+}
+
+// Ragged batch: item b has ns[b] sources and nt[b] targets (each clamped to [1, Ns] / [1, Nt]) in its Ns / Nt rows.  Row
+// tiles past ns[b] and target tiles past nt[b] are skipped, the last target tile is masked as the tail of a call with
+// Nt = nt[b], and corr columns >= ns[b] are written as 0.  Columns < ns[b] equal vcr_softcorr_tc on the pair alone.
+VCR_API int vcr_softcorr_tc_ragged(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
+                                   const float* xx, const float* yy, const float* tgt, const int* ns, const int* nt, int B,
+                                   int Ns, int Nt, int D, float* corr, cudaStream_t stream) {
+    VCR_REQUIRE(S && T && xx && yy && tgt && ns && nt && corr && B > 0 && Ns > 0 && Nt > 0 && D > 0);
+    if ((long long)B * (Ns > Nt ? Ns : Nt) > 0x7fffffffLL) return VCR_ERR_UNSUPPORTED;
+    CUtensorMap tmA, tmB;
+    int rc = vcr_make_operand_tmap(&tmA, S, D, (long long)B * Ns, lds, s_plane, 2, BM);
+    if (rc != VCR_OK) return rc;
+    rc = vcr_make_operand_tmap(&tmB, T, D, (long long)B * Nt, ldt, t_plane, 2, BN);
+    if (rc != VCR_OK) return rc;
+    SoftcorrParams p = {};
+    p.B = B; p.Ns = Ns; p.Nt = Nt; p.D = D; p.xx = xx; p.yy = yy; p.tgt = tgt; p.corr = corr;
+    p.ns_len = ns; p.nt_len = nt;
+    return softcorr_run<0, false>(tmA, tmB, p, stream);
 }

@@ -113,16 +113,18 @@ __host__ __device__ __forceinline__ double det3(const M3& A) {
 __global__ void svd_head_kernel(const float* __restrict__ src, const float* __restrict__ corr, int B, int M,
                                 float* __restrict__ R_ab, float* __restrict__ t_ab,
                                 float* __restrict__ R_ba, float* __restrict__ t_ba,
-                                float* __restrict__ H_out) {
+                                float* __restrict__ H_out, const int* __restrict__ mlen) {
     const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (b >= B) return;
     const float* s = src + (size_t)b * 3 * M;
     const float* c = corr + (size_t)b * 3 * M;
+    const int ld = M;                                  // row stride of the pair's three coordinate rows
+    M = vcr_item_len(mlen, b, ld, 1);                  // points of the pair: all of them, or its length in a ragged batch
     double ms[3] = {0, 0, 0}, mc[3] = {0, 0, 0};
     for (int n = lane; n < M; n += 32) {
 #pragma unroll
-        for (int a = 0; a < 3; ++a) { ms[a] += s[a * M + n]; mc[a] += c[a * M + n]; }
+        for (int a = 0; a < 3; ++a) { ms[a] += s[a * ld + n]; mc[a] += c[a * ld + n]; }
     }
     float fs[3], fc[3];
 #pragma unroll
@@ -134,7 +136,7 @@ __global__ void svd_head_kernel(const float* __restrict__ src, const float* __re
     for (int n = lane; n < M; n += 32) {
         float sv[3], cv[3];
 #pragma unroll
-        for (int a = 0; a < 3; ++a) { sv[a] = s[a * M + n] - fs[a]; cv[a] = c[a * M + n] - fc[a]; }
+        for (int a = 0; a < 3; ++a) { sv[a] = s[a * ld + n] - fs[a]; cv[a] = c[a * ld + n] - fc[a]; }
 #pragma unroll
         for (int i = 0; i < 3; ++i)
 #pragma unroll
@@ -260,7 +262,38 @@ VCR_API int vcr_svd_head(const float* src, const float* corr, int B, int M, floa
                          float* R_ba, float* t_ba, float* H_out, cudaStream_t stream) {
     VCR_REQUIRE(src && corr && R_ab && t_ab && B > 0 && M > 0);
     const int wpb = 4;
-    svd_head_kernel<<<vcr_cdiv(B, wpb), wpb * 32, 0, stream>>>(src, corr, B, M, R_ab, t_ab, R_ba, t_ba, H_out);
+    svd_head_kernel<<<vcr_cdiv(B, wpb), wpb * 32, 0, stream>>>(src, corr, B, M, R_ab, t_ab, R_ba, t_ba, H_out, nullptr);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
+// Ragged batch: pair b has m[b] points (clamped to [1, M]) in its M columns; the result equals vcr_svd_head on the pair's
+// first m[b] columns alone (the fp64 sums run over the same points in the same order).
+VCR_API int vcr_svd_head_ragged(const float* src, const float* corr, const int* m, int B, int M, float* R_ab, float* t_ab,
+                                float* R_ba, float* t_ba, float* H_out, cudaStream_t stream) {
+    VCR_REQUIRE(src && corr && m && R_ab && t_ab && B > 0 && M > 0);
+    const int wpb = 4;
+    svd_head_kernel<<<vcr_cdiv(B, wpb), wpb * 32, 0, stream>>>(src, corr, B, M, R_ab, t_ab, R_ba, t_ba, H_out, m);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
+__global__ void zero_padding_kernel(const float* x, const int* __restrict__ len, int C, int N, int lo,
+                                    float* out) {
+    const int n = blockIdx.x * blockDim.x + threadIdx.x;
+    const int b = blockIdx.y;
+    if (n >= N) return;
+    const bool real = n < vcr_item_len(len, b, N, lo);
+    for (int c = 0; c < C; ++c) {
+        const size_t o = ((size_t)b * C + c) * N + n;
+        out[o] = real ? x[o] : 0.f;
+    }
+}
+
+// out[b,c,n] = x[b,c,n] for n < len[b] (clamped to [lo, N]), 0 past it: a ragged batch [B,C,N] with its padding zeroed.
+VCR_API int vcr_zero_padding(const float* x, const int* len, int B, int C, int N, int lo, float* out, cudaStream_t stream) {
+    VCR_REQUIRE(x && len && out && B > 0 && C > 0 && N > 0 && B <= 65535 && lo >= 1);
+    zero_padding_kernel<<<dim3(vcr_cdiv(N, 256), B), 256, 0, stream>>>(x, len, C, N, lo, out);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
 }

@@ -81,11 +81,16 @@ def lpdnet_weights(m):
     return packed(m, "lpdnet", params, build)
 
 
-def lpdnet_tokens(m, xyz: torch.Tensor, idx_feat=None, idx_xyz=None, stages=None, out=None):
+def lpdnet_tokens(m, xyz: torch.Tensor, idx_feat=None, idx_xyz=None, stages=None, out=None, lengths=None):
     """xyz [B,3,N] -> embedding tokens [B,N,emb_dims]  (model/lpdnet_model.py:103-137, incl. the optional t3d / tfea
     TranformNets, eval mode).
 
-    idx_feat / idx_xyz (int32 [B,N,20]) inject neighbour sets, as get_graph_feature(x, idx=...) allows."""
+    idx_feat / idx_xyz (int32 [B,N,20]) inject neighbour sets, as get_graph_feature(x, idx=...) allows.
+    lengths (int32 [B] on the device): a ragged batch, cloud b is xyz[b, :, :lengths[b]].  Both kNN graphs then stay inside
+    each cloud (a padded point is its own neighbour), and every other layer is per point, so the rows of a cloud equal those
+    of the cloud embedded alone.  Not with the TranformNets, which pool over the whole cloud."""
+    if lengths is not None and (m.t3d or m.tfea):
+        raise NotImplementedError("ragged batches: LPDNet with t3d / tfea (a TranformNet pools over the padded cloud)")
     W = lpdnet_weights(m)
     slope = float(m.negative_slope)
     k = m.k
@@ -110,6 +115,9 @@ def lpdnet_tokens(m, xyz: torch.Tensor, idx_feat=None, idx_xyz=None, stages=None
             ops.bgemm(h2, 64, N * 64, 0, trans_feat, 64, 64 * 64, 0, 1, h2t, 64, N * 64, 0, N, 64, 64, B, 1)
             h2 = h2t
         h2_op = ops.to_operand(h2.view(B * N, 64), "h3") if tc else None     # shared by the kNN prefilter and the DG1 GEMM
+    if idx_feat is None and lengths is not None:
+        idx_feat = (ops.knn_topk_tc_ragged(h2, h2_op, lengths, k) if config.use_knn_tc(N) and ops.knn_tc_supported(64, k)
+                    else ops.knn_topk_ragged(h2, lengths, k, token_major=True))
     if idx_feat is None:                                                     # :122 (feature-space kNN)
         if config.use_knn_tc(N) and ops.knn_tc_supported(64, k):
             idx_feat = ops.knn_topk_tc(h2, h2_op, k)
@@ -133,7 +141,8 @@ def lpdnet_tokens(m, xyz: torch.Tensor, idx_feat=None, idx_xyz=None, stages=None
                            config.precision, op1=cat_op.cols_view(0, 128) if cat_op is not None else None,
                            op2=cat_op.cols_view(128, 128) if cat_op is not None else None)
     if idx_xyz is None:
-        idx_xyz = ops.knn_topk(xyz, k, token_major=False)                    # :129 (3-d kNN)
+        idx_xyz = (ops.knn_topk(xyz, k, token_major=False) if lengths is None      # :129 (3-d kNN)
+                   else ops.knn_topk_ragged(xyz, lengths, k, token_major=False))
     if tc:
         pq3 = torch.empty((B, N, 512), dtype=_F32, device=xyz.device)
         x2_op = cat_op.cols_view(128, 128) if cat_op is not None else ops.to_operand(cat[:, :, 128:256], "h3")
@@ -571,12 +580,18 @@ def mha_project_kv(m, xkv_op, B, Nk, mode, dev, k_out=None, vt_out=None):
     return k_v, vt
 
 
-def mha_attention(m, q_v, k_v, vt, B, Nq, Nk, mode, dev, max_ws_bytes=3 << 30):
+def mha_attention(m, q_v, k_v, vt, B, Nq, Nk, mode, dev, max_ws_bytes=3 << 30, lens=None):
     """softmax(QK^T/sqrt(d_k)) V (+ the partial-overlap key selection, model/transformer.py:29-55) with the heads merged:
-    -> operand-format [B*Nq, D].  q_v / k_v / vt: operand-format projections of B batch items."""
+    -> operand-format [B*Nq, D].  q_v / k_v / vt: operand-format projections of B batch items.
+    lens: (query lengths, key lengths) int32 [B] of a ragged batch -- the flash kernel attends to each item's own keys."""
     D, h, dk = m.h * m.d_k, m.h, m.d_k
     scale = 1.0 / math.sqrt(dk)
     att = ops.Operand.empty(B * Nq, D, mode, dev)
+    if lens is not None:
+        if m.is_src or dk != 128 or not config.flash_attention or m.__dict__.get("record_attn", False):
+            raise NotImplementedError("ragged batches: attention needs the flash kernel (d_k = 128, VCR_FLASH on), "
+                                      "no partial-overlap key selection and no record_attn")
+        return ops.flash_attn_tc_ragged(q_v, k_v, vt, att, B, h, Nq, Nk, dk, scale, lens[0], lens[1])
     keep = None
     if m.is_src:
         # partial overlap (:35-53): column sums of the unmasked probabilities pick the surviving keys.
@@ -625,8 +640,8 @@ def mha_output(m, att, B, Nq, residual, mode, out=None):
     return out
 
 
-def mha_attend(m, q_v, k_v, vt, B, Nq, Nk, residual, mode, out=None, max_ws_bytes=3 << 30):
-    att = mha_attention(m, q_v, k_v, vt, B, Nq, Nk, mode, residual.device, max_ws_bytes=max_ws_bytes)
+def mha_attend(m, q_v, k_v, vt, B, Nq, Nk, residual, mode, out=None, max_ws_bytes=3 << 30, lens=None):
+    att = mha_attention(m, q_v, k_v, vt, B, Nq, Nk, mode, residual.device, max_ws_bytes=max_ws_bytes, lens=lens)
     return mha_output(m, att, B, Nq, residual, mode, out=out)
 
 
@@ -668,7 +683,7 @@ def attn_probs_head_sum(q_v, k_v, B, h, Nq, Nk, dk, scale, keep):
     return S[..., :Nk].sum(dim=1)
 
 
-def mha_tc(m, xq_op, xkv_op, B, Nq, Nk, residual, mode, max_ws_bytes=3 << 30, out=None):
+def mha_tc(m, xq_op, xkv_op, B, Nq, Nk, residual, mode, max_ws_bytes=3 << 30, out=None, lens=None):
     """MultiHeadedAttention.forward (model/transformer.py:202-224) on tensor cores.
 
     xq_op / xkv_op: operand-format LayerNorm outputs [B*N, D] (xkv_op None => self-attention).
@@ -680,7 +695,7 @@ def mha_tc(m, xq_op, xkv_op, B, Nq, Nk, residual, mode, max_ws_bytes=3 << 30, ou
     else:
         q_v = mha_project_q(m, xq_op, B * Nq, mode, dev)
         k_v, vt = mha_project_kv(m, xkv_op, B, Nk, mode, dev)
-    return mha_attend(m, q_v, k_v, vt, B, Nq, Nk, residual, mode, out=out, max_ws_bytes=max_ws_bytes)
+    return mha_attend(m, q_v, k_v, vt, B, Nq, Nk, residual, mode, out=out, max_ws_bytes=max_ws_bytes, lens=lens)
 
 
 def ffn_tc(m, n_op, rows, residual, mode):
@@ -707,15 +722,19 @@ class HeadPre:
         self.op, self.sq = op, sq
 
 
-def encoder_decoder_tc(model, src, tgt, final_residual, mode, swap_mem=False, want_head=False, want_out=True):
+def encoder_decoder_tc(model, src, tgt, final_residual, mode, swap_mem=False, want_head=False, want_out=True, lens=None):
     """swap_mem: decoder batch item b attends to the encoder output of item (b + B/2) mod B -- the two directions of
     Transformer.forward run as one batch [src; tgt] without building the swapped copy [tgt; src]: only the encoder's
-    final LayerNorm writes its two halves exchanged."""
+    final LayerNorm writes its two halves exchanged.
+    lens: (src lengths, tgt lengths) int32 [B] of a ragged batch (not with swap_mem): every attention sees only the item's
+    own tokens; the other sublayers are per token."""
+    ls, lt = lens if lens is not None else (None, None)
+    l_ss, l_tt, l_ts = ((ls, ls), (lt, lt), (lt, ls)) if lens is not None else (None, None, None)
     B, Ns, D = src.shape
     Nt = tgt.shape[1]
     x = src
     for layer in model.encoder.layers:
-        x = mha_tc(layer.self_attn, _ln_op(layer.sublayer[0].norm, x, mode), None, B, Ns, Ns, x, mode)
+        x = mha_tc(layer.self_attn, _ln_op(layer.sublayer[0].norm, x, mode), None, B, Ns, Ns, x, mode, lens=l_ss)
         x = ffn_tc(layer.feed_forward, _ln_op(layer.sublayer[1].norm, x, mode), B * Ns, x, mode)
     if swap_mem:
         half, nrm = B // 2, model.encoder.norm
@@ -726,8 +745,8 @@ def encoder_decoder_tc(model, src, tgt, final_residual, mode, swap_mem=False, wa
         mem = _ln_op(model.encoder.norm, x, mode)
     y = tgt
     for layer in model.decoder.layers:
-        y = mha_tc(layer.self_attn, _ln_op(layer.sublayer[0].norm, y, mode), None, B, Nt, Nt, y, mode)
-        y = mha_tc(layer.src_attn, _ln_op(layer.sublayer[1].norm, y, mode), mem, B, Nt, Ns, y, mode)
+        y = mha_tc(layer.self_attn, _ln_op(layer.sublayer[0].norm, y, mode), None, B, Nt, Nt, y, mode, lens=l_tt)
+        y = mha_tc(layer.src_attn, _ln_op(layer.sublayer[1].norm, y, mode), mem, B, Nt, Ns, y, mode, lens=l_ts)
         y = ffn_tc(layer.feed_forward, _ln_op(layer.sublayer[2].norm, y, mode), B * Nt, y, mode)
     if want_head:
         nrm = model.decoder.norm
@@ -898,9 +917,10 @@ def pair_dots(src_tok, tgt_tok, alpha=1.0, pre=None):
     return dot, ld
 
 
-def vcp_whole(src_tok, tgt_tok, tgt_xyz, pre=None):
+def vcp_whole(src_tok, tgt_tok, tgt_xyz, pre=None, lengths=None):
     """getCopairALL (model/vcrnet_model.py:334-347): src_corr [B,3,N].  pre: (HeadPre src, HeadPre tgt) from the final
-    LayerNorm of the Transformer (operand copies + squared norms already in HBM)."""
+    LayerNorm of the Transformer (operand copies + squared norms already in HBM).
+    lengths: (src lengths, tgt lengths) int32 [B] of a ragged batch; src_corr is then 0 past each pair's sources."""
     if pre is not None and config.precision == "fp32":
         pre = None
     if pre is not None:
@@ -909,6 +929,13 @@ def vcp_whole(src_tok, tgt_tok, tgt_xyz, pre=None):
         B, Ns, D = src_tok.shape
         Nt = tgt_tok.shape[1]
     xx, yy = (pre[0].sq, pre[1].sq) if pre is not None else (ops.sqnorm_rows(src_tok), ops.sqnorm_rows(tgt_tok))
+    if lengths is not None:
+        if config.precision == "fp32" or not config.fused_softcorr:
+            raise NotImplementedError("ragged batches: the VCP head needs the fused tensor-core kernel (not fp32 mode, "
+                                      "VCR_FUSED_SOFTCORR on)")
+        s_op = pre[0].op if pre is not None else ops.to_operand(src_tok.reshape(B * Ns, D), "h3")
+        t_op = pre[1].op if pre is not None else ops.to_operand(tgt_tok.reshape(B * Nt, D), "h3")
+        return ops.softcorr_tc_ragged(s_op, t_op, xx, yy, tgt_xyz, B, Ns, Nt, D, lengths[0], lengths[1])
     if config.precision != "fp32" and config.fused_softcorr:
         # one kernel: 3-term tcgen05 products + online softmax + weighted sum of the target points in the epilogue
         s_op = pre[0].op if pre is not None else ops.to_operand(src_tok.reshape(B * Ns, D), "h3")

@@ -40,6 +40,96 @@ def vcrnetIter(net, src, tgt, iter=1):
     return _vcrnet_iter_eager(net, src, tgt, iter)
 
 
+def vcrnetIterRagged(net, src, tgt, src_len, tgt_len, iter=1):
+    """vcrnetIter over a ragged batch: pairs of different sizes in one call.
+
+    src [B,3,Ns_max], tgt [B,3,Nt_max] fp32 CUDA, padded; src_len / tgt_len int32 [B] on the same device: pair b is
+    (src[b, :, :src_len[b]], tgt[b, :, :tgt_len[b]]) -- vcr_net_b200.ragged.pad_clouds builds such a batch and checks the
+    lengths (21 <= len <= N_max).  Padded columns may hold any finite values; nothing depends on them.
+    Returns (srcK, src_corrK, R_ab, t_ab, R_ba, t_ba) as vcrnetIter does; restricted to a pair's lengths, each output equals
+    vcrnetIter(net, src_b, tgt_b, iter) on the pair alone bit for bit.  Padded columns of srcK and src_corrK are 0.
+
+    The lengths are read on the device only: no host sync and no length-dependent allocation, so the call can be captured
+    in a CUDA graph once per (B, Ns_max, Nt_max) and replayed with new clouds and lengths written into the same tensors.
+    Supported: eval-mode VCRNet on one device, whole-to-whole (partial=False), LPDNet embedding without t3d / tfea,
+    Transformer or Identity pointer, topK head, the tensor-core precision modes; anything else raises
+    NotImplementedError.  The network's cycle estimate (R_ba, t_ba of VCRNet.forward) is never computed: vcrnetIter
+    returns the inverse of the composed pose instead, so ``cycle`` does not change the outputs."""
+    from .. import config
+    _check_ragged_support(net)
+    if config.precision == "fp32":
+        raise NotImplementedError("vcrnetIterRagged: precision 'fp32' (the tensor-core modes h3 / fp16 / bf16 are supported)")
+    B = src.shape[0]
+    for name, x in (("src", src), ("tgt", tgt)):
+        ops._chk(x, name)
+        if x.dim() != 3 or x.shape[0] != B or x.shape[1] != 3:
+            raise ValueError(f"vcrnetIterRagged: `{name}` must be [B,3,N], got {tuple(x.shape)}")
+    for name, n in (("src_len", src_len), ("tgt_len", tgt_len)):
+        ops._lengths(n, B, name)
+        if n.device != src.device:
+            raise ValueError(f"vcrnetIterRagged: `{name}` must be on {src.device}")
+    k = net.emb_nn.k
+    with torch.no_grad():
+        # the padding is replaced by zeros once: every padded row the network computes is then finite (flash attention
+        # multiplies padded V columns by probabilities of exactly 0), whatever the caller left there
+        transformed_src = ops.zero_padding(src, src_len, k + 1)
+        tgt_z = ops.zero_padding(tgt, tgt_len, k + 1)
+        R_f = t_f = None
+        srcK = src_corrK = None
+        for _ in range(iter):
+            srcK = transformed_src
+            src_corrK, R, t = _forward_ragged(net, transformed_src, tgt_z, src_len, tgt_len)
+            transformed_src = ops.rigid_apply(transformed_src, R, t)
+            if R_f is None:
+                R_f, t_f = R, t
+            else:
+                ops.pose_compose_(R, t, R_f, t_f)
+        R_ba, t_ba = ops.pose_inverse(R_f, t_f)
+        return ops.zero_padding(srcK, src_len, k + 1), src_corrK, R_f, t_f, R_ba, t_ba
+
+
+def _check_ragged_support(net):
+    if isinstance(net, nn.DataParallel):
+        raise NotImplementedError("vcrnetIterRagged: nn.DataParallel (pass the module on one device)")
+    if not isinstance(net, VCRNet):
+        raise NotImplementedError(f"vcrnetIterRagged: {type(net).__name__} (a VCRNet is required)")
+    if net.training:
+        raise NotImplementedError("vcrnetIterRagged: training mode (call .eval())")
+    if not isinstance(net.emb_nn, LPDNet):
+        raise NotImplementedError(f"vcrnetIterRagged: emb_nn {type(net.emb_nn).__name__} (only lpdnet)")
+    if net.emb_nn.t3d or net.emb_nn.tfea:
+        raise NotImplementedError("vcrnetIterRagged: LPDNet with t3d / tfea")
+    if not isinstance(net.pointer, (Transformer, Identity)):
+        raise NotImplementedError(f"vcrnetIterRagged: pointer {type(net.pointer).__name__} (transformer or identity)")
+    if not isinstance(net.head, VcpTopK):
+        raise NotImplementedError(f"vcrnetIterRagged: vcp_nn {type(net.head).__name__} (only topK)")
+    if net.head.partial:
+        raise NotImplementedError("vcrnetIterRagged: partial=True (only whole-to-whole registration)")
+
+
+def _forward_ragged(net, src, tgt, src_len, tgt_len):
+    """VCRNet.forward's (src_corrK, R_ab, t_ab) for a ragged batch (model/vcrnet_model.py:495-516, whole-to-whole)."""
+    from .. import config
+    src_tok = Fn.lpdnet_tokens(net.emb_nn, src, lengths=src_len)
+    tgt_tok = Fn.lpdnet_tokens(net.emb_nn, tgt, lengths=tgt_len)
+    pre = None
+    if isinstance(net.pointer, Identity):
+        src_tok, tgt_tok = src_tok * 2.0, tgt_tok * 2.0                                   # :502-505 with Identity
+    else:
+        # Transformer.forward (model/transformer.py:264-272) + emb: tgt_p = model(src, tgt), src_p = model(tgt, src), each
+        # attention restricted to the pair's own tokens; the final LayerNorm writes what the head reads
+        model, mode = net.pointer.model, config.precision
+        _, op_t, sq_t = Fn.encoder_decoder_tc(model, src_tok, tgt_tok, tgt_tok, mode, want_head=True, want_out=False,
+                                              lens=(src_len, tgt_len))
+        _, op_s, sq_s = Fn.encoder_decoder_tc(model, tgt_tok, src_tok, src_tok, mode, want_head=True, want_out=False,
+                                              lens=(tgt_len, src_len))
+        pre = (Fn.HeadPre(op_s, sq_s), Fn.HeadPre(op_t, sq_t))
+        src_tok = tgt_tok = None
+    corr = Fn.vcp_whole(src_tok, tgt_tok, tgt, pre=pre, lengths=(src_len, tgt_len))            # :507
+    R, t, _, _ = ops.svd_head_ragged(src, corr, src_len)                                       # :509-516
+    return corr, R, t
+
+
 class _IterLoop(nn.Module):
     """The refinement loop as a module, so that nn.DataParallel replicates / scatters once per vcrnetIter call."""
 

@@ -95,6 +95,61 @@ def knn_topk_tc(x: torch.Tensor, xop, k: int, want64: bool = False, want_flagged
     return out if len(out) > 1 else out[0]
 
 
+def _lengths(n: torch.Tensor, B: int, name: str):
+    """Per-item lengths of a ragged batch: int32 [B] on the device (read there only; the kernels clamp them)."""
+    _chk(n, name, torch.int32)
+    if tuple(n.shape) != (B,):
+        raise RuntimeError(f"vcr_net_b200: `{name}` must have shape ({B},), got {tuple(n.shape)}")
+    return n.contiguous()
+
+
+def knn_topk_ragged(x: torch.Tensor, n: torch.Tensor, k: int, token_major: bool = False):
+    """knn_topk of a ragged batch: item b holds n[b] points of x's N; padded queries get their own index in all k slots."""
+    _chk(x, "x")
+    x = x.contiguous()
+    B, N, D = x.shape if token_major else (x.shape[0], x.shape[2], x.shape[1])
+    n = _lengths(n, B, "n")
+    L = lib()
+    idx32 = torch.empty((B, N, k), dtype=torch.int32, device=x.device)
+    ws_bytes = L.vcr_knn_workspace_bytes(B, N)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+    L.check(L.vcr_knn_topk_ragged(x.data_ptr(), n.data_ptr(), B, D, N, k, int(token_major), idx32.data_ptr(), None,
+                                  ws.data_ptr(), ws_bytes, _stream(x)), "vcr_knn_topk_ragged")
+    return idx32
+
+
+def knn_topk_tc_ragged(x: torch.Tensor, xop, n: torch.Tensor, k: int):
+    """knn_topk_tc of a ragged batch (token-major x [B,N,D], its "h3" Operand or None), as knn_topk_ragged."""
+    _chk(x, "x")
+    x = x.contiguous()
+    B, N, D = x.shape
+    n = _lengths(n, B, "n")
+    if xop is None:
+        xop = to_operand(x.view(B * N, D), "h3")
+    assert xop.mode == "h3" and xop.rows == B * N and xop.cols == D
+    L = lib()
+    idx32 = torch.empty((B, N, k), dtype=torch.int32, device=x.device)
+    ws_bytes = L.vcr_knn_tc_workspace_bytes(B, N)
+    ws = torch.empty(ws_bytes // 4, dtype=torch.int32, device=x.device)
+    L.check(L.vcr_knn_topk_tc_ragged(x.data_ptr(), xop.ptr, xop.ld, xop.plane_stride, n.data_ptr(), B, D, N, k,
+                                     idx32.data_ptr(), None, ws.data_ptr(), ws_bytes, _stream(x)),
+            "vcr_knn_topk_tc_ragged")
+    return idx32
+
+
+def zero_padding(x: torch.Tensor, n: torch.Tensor, lo: int = 1):
+    """[B,C,N] ragged batch -> a copy with the columns past n[b] (clamped to [lo, N]) set to 0."""
+    _chk(x, "x")
+    x = x.contiguous()
+    B, C, N = x.shape
+    n = _lengths(n, B, "n")
+    out = torch.empty_like(x)
+    L = lib()
+    L.check(L.vcr_zero_padding(x.data_ptr(), n.data_ptr(), B, C, N, int(lo), out.data_ptr(), _stream(x)),
+            "vcr_zero_padding")
+    return out
+
+
 def knn_tc_supported(D: int, k: int) -> bool:
     return 16 <= D <= 128 and D % 4 == 0 and 1 <= k <= 30
 
@@ -311,6 +366,17 @@ def flash_attn_tc(q: Operand, k: Operand, vt: Operand, out: Operand, B, H, Nq, N
                                 vt.plane_stride, B, H, Nq, Nk, dk, TC_MODES[q.mode], float(scale),
                                 keep.data_ptr() if keep is not None else None, out.ptr, out.ld, out.plane_stride,
                                 lse.data_ptr() if lse is not None else None, _stream(q.buf)), "vcr_flash_attn_tc")
+    return out
+
+
+def flash_attn_tc_ragged(q: Operand, k: Operand, vt: Operand, out: Operand, B, H, Nq, Nk, dk, scale, nq, nk):
+    """flash_attn_tc of a ragged batch: item b has nq[b] queries and nk[b] keys (int32 [B] device tensors)."""
+    L = lib()
+    nq, nk = _lengths(nq, B, "nq"), _lengths(nk, B, "nk")
+    L.check(L.vcr_flash_attn_tc_ragged(q.ptr, q.ld, q.plane_stride, k.ptr, k.ld, k.plane_stride, vt.ptr, vt.ld,
+                                       vt.plane_stride, nq.data_ptr(), nk.data_ptr(), B, H, Nq, Nk, dk, TC_MODES[q.mode],
+                                       float(scale), out.ptr, out.ld, out.plane_stride, _stream(q.buf)),
+            "vcr_flash_attn_tc_ragged")
     return out
 
 
@@ -748,6 +814,21 @@ def softcorr_tc(s_op: "Operand", t_op: "Operand", xx, yy, tgt_xyz: torch.Tensor,
     return corr
 
 
+def softcorr_tc_ragged(s_op: "Operand", t_op: "Operand", xx, yy, tgt_xyz: torch.Tensor, B: int, Ns: int, Nt: int, D: int,
+                       ns: torch.Tensor, nt: torch.Tensor):
+    """softcorr_tc of a ragged batch: pair b has ns[b] sources and nt[b] targets; corr columns >= ns[b] are 0."""
+    assert s_op.mode == "h3" and t_op.mode == "h3" and s_op.rows == B * Ns and t_op.rows == B * Nt
+    tgt_xyz = tgt_xyz.contiguous()
+    _chk(tgt_xyz, "tgt")
+    ns, nt = _lengths(ns, B, "ns"), _lengths(nt, B, "nt")
+    corr = torch.empty((B, 3, Ns), dtype=_F32, device=tgt_xyz.device)
+    L = lib()
+    L.check(L.vcr_softcorr_tc_ragged(s_op.ptr, s_op.ld, s_op.plane_stride, t_op.ptr, t_op.ld, t_op.plane_stride,
+                                     xx.data_ptr(), yy.data_ptr(), tgt_xyz.data_ptr(), ns.data_ptr(), nt.data_ptr(),
+                                     B, Ns, Nt, D, corr.data_ptr(), _stream(tgt_xyz)), "vcr_softcorr_tc_ragged")
+    return corr
+
+
 def softcorr_best_tc(s_op: "Operand", t_op: "Operand", xx, yy, B: int, Ns: int, Nt: int, D: int):
     """Fused getCopair statistics on tensor cores: (argmax_j pd_ij int32 [B,Ns], max_j softmax_j(pd_ij) [B,Ns])."""
     assert s_op.mode == "h3" and t_op.mode == "h3" and s_op.rows == B * Ns and t_op.rows == B * Nt
@@ -886,6 +967,21 @@ def svd_head(src: torch.Tensor, corr: torch.Tensor, want_H=False):
     L.check(L.vcr_svd_head(src.data_ptr(), corr.data_ptr(), B, M, R.data_ptr(), t.data_ptr(), Rb.data_ptr(),
                            tb.data_ptr(), H.data_ptr() if want_H else None, _stream(src)), "vcr_svd_head")
     return (R, t, Rb, tb, H) if want_H else (R, t, Rb, tb)
+
+
+def svd_head_ragged(src: torch.Tensor, corr: torch.Tensor, m: torch.Tensor):
+    """svd_head of a ragged batch: pair b uses its first m[b] columns.  -> (R_ab, t_ab, R_ba, t_ba)."""
+    _chk(src, "src"); _chk(corr, "src_corr")
+    src, corr = src.contiguous(), corr.contiguous()
+    B, _, M = src.shape
+    m = _lengths(m, B, "m")
+    dev = src.device
+    R, Rb = torch.empty((B, 3, 3), dtype=_F32, device=dev), torch.empty((B, 3, 3), dtype=_F32, device=dev)
+    t, tb = torch.empty((B, 3), dtype=_F32, device=dev), torch.empty((B, 3), dtype=_F32, device=dev)
+    L = lib()
+    L.check(L.vcr_svd_head_ragged(src.data_ptr(), corr.data_ptr(), m.data_ptr(), B, M, R.data_ptr(), t.data_ptr(),
+                                  Rb.data_ptr(), tb.data_ptr(), None, _stream(src)), "vcr_svd_head_ragged")
+    return R, t, Rb, tb
 
 
 def rigid_apply(pc: torch.Tensor, R: torch.Tensor, t: torch.Tensor):
