@@ -138,6 +138,13 @@ int vcr_flash_attn_tc_ragged(const void* Q, int ldq, long long q_plane, const vo
                              const void* VT, int ldv, long long v_plane, const int* nq, const int* nk, int B, int H,
                              int Nq, int Nk, int dk, int mode, float scale, void* O, int ldo, long long o_plane,
                              cudaStream_t stream);
+/* vcr_flash_attn_tc_ragged with the partial-overlap key mask keep [B, Nk] (uint8, row stride Nk): a key of item b with
+ * keep == 0 gets -1e9 (:51-52), a key past nk[b] gets -inf whatever keep holds.  Rows of real queries equal
+ * vcr_flash_attn_tc with keep = the item's first nk[b] mask bytes on the item alone, bit for bit (same finiteness condition). */
+int vcr_flash_attn_tc_ragged_keep(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                                  const void* VT, int ldv, long long v_plane, const int* nq, const int* nk,
+                                  const uint8_t* keep, int B, int H, int Nq, int Nk, int dk, int mode, float scale, void* O,
+                                  int ldo, long long o_plane, cudaStream_t stream);
 /* Organisation of vcr_flash_attn_tc: 3 (default) = Q and P in tensor memory (tcgen05.mma with the A operand in TMEM; P is
  * written over the S tile it came from), 8 softmax warps; 2 = every operand in shared memory, 8 warps on every key tile
  * (same bits as 3); 4 = 16 warps; 1 = two groups of 4 warps alternating key tiles.  Process-wide tuning knob; returns the
@@ -198,6 +205,15 @@ int vcr_softmax_rows(float* S, int ld, long long rows, int n, const uint8_t* kee
 size_t vcr_colsum_workspace_bytes(int B, int n);
 int vcr_colsum(const float* P, int ld, int B, long long rows_per_batch, int n, float* out, void* workspace,
                size_t workspace_bytes, cudaStream_t stream);
+/* The materialised selectCom passes of a ragged batch (vcr_select_stats_ragged computes the other pairs): pd [B][Ns][ld]
+ * from vcr_negdist over the padded block, pair b's ns[b] x nt[b] corner in use (int32, device; clamped to [0, Ns] /
+ * [0, Nt]).  Only the pairs with nt[b] > 1024 -- those a pair alone routes to the materialised passes -- are touched, each
+ * equal to its entry point on the pair alone over the pair's rows / columns, bit for bit.
+ * vcr_softmax_rows_ragged: the pair's rows over its columns, in place.  vcr_colsum_ragged: out [B, Nt] column sums of the
+ * pair's rows, columns past nt[b] written as 0 (workspace as vcr_colsum).  vcr_rowsum_colsoftmax_ragged: below. */
+int vcr_softmax_rows_ragged(float* S, int ld, const int* ns, const int* nt, int B, int Ns, int Nt, cudaStream_t stream);
+int vcr_colsum_ragged(const float* P, int ld, const int* ns, const int* nt, int B, int Ns, int Nt, float* out,
+                      void* workspace, size_t workspace_bytes, cudaStream_t stream);
 /* operand-format producers for vcr_gemm_tc: LayerNorm output / softmax probabilities written directly as
  * 16-bit hi(/lo) planes; row log-sum-exp statistics and the column sums of softmax(S) without
  * materialising the probabilities (partial-overlap key selection, model/transformer.py:39). */
@@ -216,10 +232,25 @@ size_t vcr_attn_colsum_workspace_bytes(int B, int H, int Nq, int Nk);
 int vcr_attn_colsum_tc(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
                        int B, int H, int Nq, int Nk, int dk, float scale, float* out, void* workspace,
                        size_t workspace_bytes, cudaStream_t stream);
+/* Ragged batch: item b has nq[b] queries and nk[b] keys (int32, device; clamped to [0, Nq] / [0, Nk]) in its Nq / Nk rows.
+ * Keys past nk[b] are -inf in the row maxima and sums and their tiles are not loaded, query tiles past nq[b] are skipped,
+ * and item b's partials are added in the order of the item alone ((hh * nqt_b + qt) * 4 + quarter, nqt_b = ceil(nq_b/128)).
+ * out [B, Nk]: columns < nk[b] equal vcr_attn_colsum_tc on the item alone, bit for bit; the rest are 0.  Workspace as
+ * vcr_attn_colsum_tc. */
+int vcr_attn_colsum_tc_ragged(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                              const int* nq, const int* nk, int B, int H, int Nq, int Nk, int dk, float scale, float* out,
+                              void* workspace, size_t workspace_bytes, cudaStream_t stream);
 /* fused, single-read form of vcr_row_lse + vcr_colsum_softmax (unmasked): out[B,n] = column sums of softmax rows */
 size_t vcr_softmax_colsum_workspace_bytes(int B, long long rows_per_batch, int ld, int n);
 int vcr_softmax_colsum(const float* S, int ld, int B, long long rows_per_batch, int n, float* out,
                        void* workspace, size_t workspace_bytes, cudaStream_t stream);
+/* The same over a ragged batch of scaled scores S [B][H][Nq][ld] (fp32, ld >= Nk, ld % 4 == 0, 16-byte aligned): item b has
+ * nq[b] queries and nk[b] keys (int32, device; clamped to [0, Nq] / [0, Nk]).  Its compact rows hh * nq_b + q are slabbed by
+ * the rows-per-CTA of its own ld_b = ceil(nk_b / 4) * 4, as vcr_softmax_colsum slabs the item alone, so out [B, Nk] columns
+ * < nk[b] equal vcr_softmax_colsum on S_b [H * nq_b, ld_b] bit for bit; the rest are 0. */
+size_t vcr_softmax_colsum_ragged_workspace_bytes(int B, int H, int Nq, int Nk);
+int vcr_softmax_colsum_ragged(const float* S, int ld, const int* nq, const int* nk, int B, int H, int Nq, int Nk,
+                              float* out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 int vcr_colsum_softmax(const float* S, int ld, int B, long long rows_per_batch, int n, const float* rmax,
                        const float* rsum, float* out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 int vcr_rowsum(const float* P, int ld, long long rows, int n, float* out, cudaStream_t stream);
@@ -227,6 +258,11 @@ int vcr_rowsum(const float* P, int ld, long long rows, int n, float* out, cudaSt
  * n <= 262 144: one CTA per row up to 16 384, beyond that one thread-block cluster of 2, 4, 8 or 16 CTAs per row (16 384
  * keys each); -2 above 262 144 or when the device cannot co-schedule the cluster.  No workspace, no host sync. */
 int vcr_topk_select(const float* vals, int B, int n, int K, int* idx_out, uint8_t* mask_out, cudaStream_t stream);
+/* Ragged rows: row b of vals [B, n] holds n_len[b] values (clamped to [0, n]) and selects k_len[b] of them (clamped to
+ * [0, min(K, n_len[b])]); both int32 on the device.  idx_out [B, K]: the indices vcr_topk_select gives on the row alone,
+ * then 0; mask_out [B, n]: 1 on the selected keys, 0 elsewhere (past n_len[b] too).  n <= 16 384 (-2 above). */
+int vcr_topk_select_ragged(const float* vals, const int* n_len, const int* k_len, int B, int n, int K, int* idx_out,
+                           uint8_t* mask_out, cudaStream_t stream);
 
 /* ---- VcpTopK head: model/vcrnet_model.py:162-347 ---------------------------------------------------
  * Row pass over dot[B,Ns,ld] = s_i.t_j: pd = (-xx_i + 2 dot) - yy_j, softmax over j, then
@@ -254,6 +290,11 @@ int vcr_softcorr_tc_ragged(const void* S, int lds, long long s_plane, const void
 int vcr_softcorr_best_tc(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
                          const float* xx, const float* yy, int B, int Ns, int Nt, int D,
                          int* best_idx, float* best_val, cudaStream_t stream);
+/* Ragged batch, with the tile walk of vcr_softcorr_tc_ragged: rows < ns[b] equal vcr_softcorr_best_tc on the pair alone,
+ * bit for bit; rows past ns[b] get best_idx = 0 and best_val = 0. */
+int vcr_softcorr_best_tc_ragged(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
+                                const float* xx, const float* yy, const int* ns, const int* nt, int B, int Ns, int Nt,
+                                int D, int* best_idx, float* best_val, cudaStream_t stream);
 /* selectCom's statistics (as vcr_select_stats) straight from the operands, on tensor cores, with no [Ns,Nt] buffer:
  * S / T, xx / yy as vcr_softcorr_best_tc takes them -> row_stat [B,Ns], col_stat [B,Nt].  Four launches of the fused
  * kernel (row max / sum over targets, the same over sources, then the two weighted sums), each row owned by one thread
@@ -266,12 +307,25 @@ int vcr_select_stats_tc(const void* S, int lds, long long s_plane, const void* T
 size_t vcr_rowsum_colsoftmax_workspace_bytes(int B, int Nt);
 int vcr_rowsum_colsoftmax(const float* pd, int ld, int B, int Ns, int Nt, float* out, void* workspace,
                           size_t workspace_bytes, cudaStream_t stream);
+/* Ragged batch (see vcr_softmax_rows_ragged): out [B, Ns], rows past ns[b] written as 0; workspace as
+ * vcr_rowsum_colsoftmax. */
+int vcr_rowsum_colsoftmax_ragged(const float* pd, int ld, const int* ns, const int* nt, int B, int Ns, int Nt, float* out,
+                                 void* workspace, size_t workspace_bytes, cudaStream_t stream);
 /* selectCom (model/vcrnet_model.py:213-222, 243-244) selection statistics in two reads of the score products:
  * pd_ij = (-xx_i - (-2 dot_ij)) - yy_j is formed on the fly (dot [B,Ns,ld] is left untouched); row_stat [B,Ns] = row sums of
  * the column softmax, col_stat [B,Nt] = column sums of the row softmax.  Deterministic (fixed slab order). */
 size_t vcr_select_stats_workspace_bytes(int B, int Ns, int Nt);
 int vcr_select_stats(const float* dot, int ld, int B, int Ns, int Nt, const float* xx, const float* yy,
                      float* row_stat, float* col_stat, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+/* Ragged batch: pair b has ns[b] sources and nt[b] targets (int32, device; clamped to [0, Ns] / [0, Nt]) in dot [B][Ns][ld],
+ * xx [B, Ns], yy [B, Nt].  Only the pairs with nt[b] <= 1024 -- those a pair alone sends to vcr_select_stats -- are computed:
+ * row_stat rows < ns[b] and col_stat columns < nt[b] equal vcr_select_stats on the pair alone, bit for bit, and the rest of
+ * their rows are 0.  The other pairs are left to the materialised passes (vcr_negdist in place, then
+ * vcr_rowsum_colsoftmax_ragged, vcr_softmax_rows_ragged, vcr_colsum_ragged), which must run after this call.  Any Nt;
+ * workspace: vcr_select_stats_workspace_bytes(B, Ns, Nt). */
+int vcr_select_stats_ragged(const float* dot, int ld, const int* ns, const int* nt, int B, int Ns, int Nt, const float* xx,
+                            const float* yy, float* row_stat, float* col_stat, void* workspace, size_t workspace_bytes,
+                            cudaStream_t stream);
 /* Rows idx[b,:] of an operand-format buffer ([2 planes][B*Nin][ld_in], 16-bit) and of its squared row norms: what getCopair
  * (model/vcrnet_model.py:264-332) needs of the points selectCom kept, without going back through fp32. */
 int vcr_gather_operand_rows(const void* in, int ld_in, long long plane_in, int B, int Nin, const int* idx, int K,

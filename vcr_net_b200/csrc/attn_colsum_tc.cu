@@ -41,10 +41,29 @@ struct ColsumParams {
     int B, H, Nq, Nk;
     float scale_log2;
     float* part;          // [B][H * nqt * 4][Nk]
+    const int* nq_len;    // ragged batch: queries / keys of item b (clamped to [0, Nq] / [0, Nk]); null in a uniform batch
+    const int* nk_len;
 };
+
+// Ragged batch: the items a CTA walks are those whose query tile holds a query of its batch item; every role walks the same
+// list.  Item b's partial slabs are laid out as the item alone lays them out, (hh * nqt_b + qt) * 4 + ew with
+// nqt_b = ceil(nq_b / 128), so colsum_reduce_kernel adds them in the pair-alone order.
+struct ItemLens {
+    int nq, nk, nqt, nkt;
+};
+template <bool RAGGED>
+__device__ __forceinline__ ItemLens colsum_item(const ColsumParams& p, int b) {
+    ItemLens r;
+    r.nq = RAGGED ? min(max(__ldg(p.nq_len + b), 0), p.Nq) : p.Nq;
+    r.nk = RAGGED ? min(max(__ldg(p.nk_len + b), 0), p.Nk) : p.Nk;
+    r.nqt = (r.nq + BQ - 1) / BQ;
+    r.nkt = (r.nk + BKV - 1) / BKV;
+    return r;
+}
 
 __device__ __forceinline__ float ex2_approx(float x) { return tc::ex2_mufu(x); }
 
+template <bool RAGGED>
 __global__ void __launch_bounds__(128 + NSTAT, 1)
 attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK, const ColsumParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -57,8 +76,15 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int nqt = (p.Nq + BQ - 1) / BQ;
-    const int nkt = (p.Nk + BKV - 1) / BKV;
+    const int nkt_u = (p.Nk + BKV - 1) / BKV;                // a uniform batch: every item's key tiles
     const long long items = (long long)p.B * p.H * nqt;
+    // first item at or after `it` (stride gridDim.x) with a live query tile; every item in a uniform batch
+    auto next_item = [&](long long it) -> long long {
+        if (RAGGED)
+            for (; it < items; it += gridDim.x)
+                if ((int)(it % nqt) < colsum_item<true>(p, (int)(it / nqt) / p.H).nqt) break;
+        return it;
+    };
 
     if (warp == 0 && lane == 0) { tc::tma_prefetch_desc(&tmQ); tc::tma_prefetch_desc(&tmK); }
     if (warp == 1 && lane == 0) {
@@ -90,13 +116,16 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
                     for (int pl = 0; pl < 2; ++pl)
                         tc::tma_load_3d(smem + (kb * 2 + pl) * TILE, &tmQ, q_full, hh * DK + kb * 64, b * p.Nq + qt * BQ, pl);
             };
-            if ((long long)blockIdx.x < items) load_q(blockIdx.x);
-            for (long long it = blockIdx.x; it < items; it += gridDim.x, ++w) {
+            const long long first = next_item(blockIdx.x);
+            if (first < items) load_q(first);
+            for (long long it = first; it < items; it = next_item(it + gridDim.x), ++w) {
                 const int bh = (int)(it / nqt);
                 const int hh = bh % p.H, b = bh / p.H;
-                if (it + gridDim.x < items) {                   // next item's Q: staging is free once this item's Q is in TMEM
+                const int nkt = RAGGED ? colsum_item<true>(p, b).nkt : nkt_u;
+                const long long nx = next_item(it + gridDim.x);
+                if (nx < items) {                               // next item's Q: staging is free once this item's Q is in TMEM
                     tc::mbar_wait(q_empty, w & 1);
-                    load_q(it + gridDim.x);
+                    load_q(nx);
                 }
                 for (int sw = 0; sw < 2; ++sw)
                     for (int j = 0; j < nkt; ++j, ++g) {
@@ -118,7 +147,8 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         if (tc::elect_one()) {
             constexpr uint32_t idesc = tc::umma_idesc(BQ, BKV, 0);
             uint32_t g = 0, w = 0;
-            for (long long it = blockIdx.x; it < items; it += gridDim.x, ++w) {
+            for (long long it = next_item(blockIdx.x); it < items; it = next_item(it + gridDim.x), ++w) {
+                const int nkt = RAGGED ? colsum_item<true>(p, (int)(it / nqt) / p.H).nkt : nkt_u;
                 tc::mbar_wait(qt_full, w & 1);
                 tc::tc_fence_after();
                 const uint32_t q_tm = tmem_base + Q_COL0 + (w & 1) * 128;
@@ -183,12 +213,15 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
             tc::mbar_arrive(q_empty);
         };
         uint32_t g = 0, w = 0;
-        if ((long long)blockIdx.x < items) copy_q(0);
-        for (long long it = blockIdx.x; it < items; it += gridDim.x, ++w) {
+        const long long first = next_item(blockIdx.x);
+        if (first < items) copy_q(0);
+        for (long long it = first; it < items; it = next_item(it + gridDim.x), ++w) {
             const int qt = (int)(it % nqt);
             const int bh = (int)(it / nqt);
             const int hh = bh % p.H, b = bh / p.H;
-            const bool row_ok = qt * BQ + rloc < p.Nq;
+            const ItemLens li = RAGGED ? colsum_item<true>(p, b) : ItemLens{p.Nq, p.Nk, nqt, nkt_u};
+            const int nkt = li.nkt, nk = li.nk;
+            const bool row_ok = qt * BQ + rloc < li.nq;
             float m = -INFINITY, l = 0.f;        // sweep 0: running max / sum;  sweep 1: -M and 1/L
             for (int sw = 0; sw < 2; ++sw) {
                 for (int j = 0; j < nkt; ++j, ++g) {
@@ -196,7 +229,7 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
                     tc::mbar_wait(&s_full[sb], (g >> 1) & 1);
                     tc::tc_fence_after();
                     const int key0 = j * BKV + cq * 32;         // first key of this warp's 32 columns
-                    if (key0 < p.Nk) {                          // warp-uniform
+                    if (key0 < nk) {                            // warp-uniform
                         float x[32];
                         {
                             const uint32_t sa = tmem_base + sb * S_COLS + lane_adr + cq * 32;
@@ -206,10 +239,10 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
 #pragma unroll
                             for (int i = 0; i < 32; ++i) x[i] = __uint_as_float(r0[i]);   // raw scores: sc > 0 is applied in the fma below
                         }
-                        if (key0 + 32 > p.Nk) {
+                        if (key0 + 32 > nk) {
 #pragma unroll
                             for (int i = 0; i < 32; ++i)
-                                if (key0 + i >= p.Nk) x[i] = -INFINITY;
+                                if (key0 + i >= nk) x[i] = -INFINITY;
                         }
                         if (sw == 0) {
                             float c4[4] = {x[0], x[1], x[2], x[3]};             // four independent chains
@@ -238,8 +271,8 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
                                 }
                             }
                             const int key = key0 + lane;
-                            if (key < p.Nk)
-                                p.part[((size_t)b * (p.H * nqt * 4) + ((size_t)(hh * nqt + qt) * 4 + ew)) * p.Nk + key] = x[0];
+                            if (key < nk)
+                                p.part[((size_t)b * (p.H * nqt * 4) + ((size_t)(hh * li.nqt + qt) * 4 + ew)) * p.Nk + key] = x[0];
                         }
                     }
                     tc::tc_fence_before();
@@ -261,7 +294,7 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
                     l = 1.f / L;
                     asm volatile("bar.sync %0, 128;" ::"r"(1 + ew) : "memory");         // xch reusable
                     // next item's Q into the other TMEM buffer (its previous user's products retired an item ago)
-                    if (it + gridDim.x < items) copy_q(w + 1);
+                    if (next_item(it + gridDim.x) < items) copy_q(w + 1);
                 }
             }
         }
@@ -271,16 +304,29 @@ attn_colsum_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     if (warp == 2) tc::tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
-// out[b, j] = sum_s part[b, s, j] in slab order
-__global__ void colsum_reduce_kernel(const float* __restrict__ part, int slabs, int n, float* __restrict__ out) {
+// out[b, j] = sum_s part[b, s, j] in slab order.  Ragged batch (RAGGED): item b adds its first H * nqt_b * 4 slabs and
+// writes 0 past its keys.
+template <bool RAGGED>
+__global__ void colsum_reduce_kernel(const float* __restrict__ part, int slabs, int n, float* __restrict__ out,
+                                     ColsumParams p) {
     const int b = blockIdx.y;
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= n) return;
+    int ns = slabs;
+    if (RAGGED) {
+        const ItemLens li = colsum_item<true>(p, b);
+        if (j >= li.nk) { out[(size_t)b * n + j] = 0.f; return; }
+        ns = p.H * li.nqt * 4;
+    }
     const float* pb = part + (size_t)b * slabs * n + j;
     float acc = 0.f;
-    for (int s = 0; s < slabs; ++s) acc += pb[(size_t)s * n];
+    for (int s = 0; s < ns; ++s) acc += pb[(size_t)s * n];
     out[(size_t)b * n + j] = acc;
 }
+
+static int attn_colsum_launch(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                              const int* nq, const int* nk, int B, int H, int Nq, int Nk, int dk, float scale, float* out,
+                              void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
 }  // namespace
 
@@ -288,12 +334,10 @@ VCR_API size_t vcr_attn_colsum_workspace_bytes(int B, int H, int Nq, int Nk) {
     return (size_t)B * H * ((Nq + BQ - 1) / BQ) * 4 * Nk * sizeof(float);
 }
 
-// Q: operand buffer [2 planes][B*Nq][ldq] ("h3": fp16 hi, lo * 2^11), head hh in columns [hh*128, hh*128+128);
-// K: [2][B*Nk][ldk] likewise.  out [B, Nk] = column sums over heads and queries of softmax_j(q.k * scale).
-VCR_API int vcr_attn_colsum_tc(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
-                               int B, int H, int Nq, int Nk, int dk, float scale, float* out, void* workspace,
-                               size_t workspace_bytes, cudaStream_t stream) {
-    VCR_REQUIRE(Q && K && out && B > 0 && H > 0 && Nq > 0 && Nk > 0 && B <= 65535);
+namespace {
+int attn_colsum_launch(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                       const int* nq, const int* nk, int B, int H, int Nq, int Nk, int dk, float scale, float* out,
+                       void* workspace, size_t workspace_bytes, cudaStream_t stream) {
     if (dk != DK) return VCR_ERR_UNSUPPORTED;
     if (!workspace || workspace_bytes < vcr_attn_colsum_workspace_bytes(B, H, Nq, Nk)) return VCR_ERR_WORKSPACE;
     CUtensorMap tq, tk;
@@ -304,7 +348,9 @@ VCR_API int vcr_attn_colsum_tc(const void* Q, int ldq, long long q_plane, const 
     ColsumParams p;
     p.B = B; p.H = H; p.Nq = Nq; p.Nk = Nk; p.scale_log2 = scale * kLog2e;
     p.part = reinterpret_cast<float*>(workspace);
-    auto kern = attn_colsum_tc_kernel;
+    p.nq_len = nq; p.nk_len = nk;
+    const bool ragged = nq != nullptr;
+    auto kern = ragged ? attn_colsum_tc_kernel<true> : attn_colsum_tc_kernel<false>;
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM) != cudaSuccess)
         return VCR_ERR_LAUNCH;
     int dev = 0, sms = 148;
@@ -315,7 +361,30 @@ VCR_API int vcr_attn_colsum_tc(const void* Q, int ldq, long long q_plane, const 
     const int grid = (int)(items < sms ? items : sms);
     kern<<<grid, 128 + NSTAT, SMEM, stream>>>(tq, tk, p);
     VCR_CHECK_LAUNCH();
-    colsum_reduce_kernel<<<dim3(vcr_cdiv(Nk, 128), B), 128, 0, stream>>>(p.part, H * nqt * 4, Nk, out);
+    if (ragged) colsum_reduce_kernel<true><<<dim3(vcr_cdiv(Nk, 128), B), 128, 0, stream>>>(p.part, H * nqt * 4, Nk, out, p);
+    else colsum_reduce_kernel<false><<<dim3(vcr_cdiv(Nk, 128), B), 128, 0, stream>>>(p.part, H * nqt * 4, Nk, out, p);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
+}
+}  // namespace
+
+// Q: operand buffer [2 planes][B*Nq][ldq] ("h3": fp16 hi, lo * 2^11), head hh in columns [hh*128, hh*128+128);
+// K: [2][B*Nk][ldk] likewise.  out [B, Nk] = column sums over heads and queries of softmax_j(q.k * scale).
+VCR_API int vcr_attn_colsum_tc(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                               int B, int H, int Nq, int Nk, int dk, float scale, float* out, void* workspace,
+                               size_t workspace_bytes, cudaStream_t stream) {
+    VCR_REQUIRE(Q && K && out && B > 0 && H > 0 && Nq > 0 && Nk > 0 && B <= 65535);
+    return attn_colsum_launch(Q, ldq, q_plane, K, ldk, k_plane, nullptr, nullptr, B, H, Nq, Nk, dk, scale, out, workspace,
+                              workspace_bytes, stream);
+}
+
+// Ragged batch: item b has nq[b] queries and nk[b] keys (clamped to [0, Nq] / [0, Nk]) in its Nq / Nk rows.  Keys past nk[b]
+// are -inf in the row maxima and sums, key tiles past them are not loaded, query tiles past nq[b] are skipped.  out [B, Nk]:
+// columns < nk[b] equal vcr_attn_colsum_tc on the item alone, bit for bit; the rest are 0.  Workspace as vcr_attn_colsum_tc.
+VCR_API int vcr_attn_colsum_tc_ragged(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                                      const int* nq, const int* nk, int B, int H, int Nq, int Nk, int dk, float scale,
+                                      float* out, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+    VCR_REQUIRE(Q && K && nq && nk && out && B > 0 && H > 0 && Nq > 0 && Nk > 0 && B <= 65535);
+    return attn_colsum_launch(Q, ldq, q_plane, K, ldk, k_plane, nq, nk, B, H, Nq, Nk, dk, scale, out, workspace,
+                              workspace_bytes, stream);
 }

@@ -1172,16 +1172,10 @@ VCR_API int vcr_flash_attn_tc(const void* Q, int ldq, long long q_plane, const v
     return launch_attn<1, 1, 2>(tq, tk, tv, p, stream);
 }
 
-// Ragged batch: item b has nq[b] queries and nk[b] keys (each clamped to [1, Nq] / [1, Nk]) in its Nq / Nk rows.  Key tiles
-// past nk[b] are not loaded, the last one is masked as the tail of a call with Nk = nk[b], and a query tile wholly past
-// nq[b] is written as zeros after one key tile.  Rows of a real query equal vcr_flash_attn_tc on the item alone, bit for
-// bit, provided the padded V columns of the last key tile are finite (their probability is exactly 0).  Always the default
-// organisation (Q and P in tensor memory); no key mask, no lse.
-VCR_API int vcr_flash_attn_tc_ragged(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
-                                     const void* VT, int ldv, long long v_plane, const int* nq, const int* nk, int B, int H,
-                                     int Nq, int Nk, int dk, int mode, float scale, void* O, int ldo, long long o_plane,
-                                     cudaStream_t stream) {
-    VCR_REQUIRE(Q && K && VT && O && nq && nk && B > 0 && H > 0 && Nq > 0 && Nk > 0);
+static int flash_ragged_launch(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                               const void* VT, int ldv, long long v_plane, const int* nq, const int* nk, int B, int H,
+                               int Nq, int Nk, int dk, int mode, float scale, const uint8_t* keep, void* O, int ldo,
+                               long long o_plane, cudaStream_t stream) {
     if (dk != DK || mode < 0 || mode > 2) return VCR_ERR_UNSUPPORTED;
     if ((ldo & 7) || (o_plane & 7)) return VCR_ERR_INVALID;
     const int planes = mode == 0 ? 2 : 1;
@@ -1194,9 +1188,35 @@ VCR_API int vcr_flash_attn_tc_ragged(const void* Q, int ldq, long long q_plane, 
     if (rc != VCR_OK) return rc;
     AttnParams p;
     p.B = B; p.H = H; p.Nq = Nq; p.Nk = Nk;
-    p.scale_log2 = scale * kLog2e; p.keep = nullptr; p.nq_len = nq; p.nk_len = nk;
+    p.scale_log2 = scale * kLog2e; p.keep = keep; p.nq_len = nq; p.nk_len = nk;
     p.O = reinterpret_cast<__half*>(O); p.ldo = ldo; p.o_plane = o_plane; p.lse = nullptr; p.out_bf16 = mode == 2;
     if (mode == 0) return launch_attn_ts<3, 0>(tq, tk, tv, p, stream);
     if (mode == 1) return launch_attn_ts<1, 0>(tq, tk, tv, p, stream);
     return launch_attn_ts<1, 1>(tq, tk, tv, p, stream);
+}
+
+// Ragged batch: item b has nq[b] queries and nk[b] keys (each clamped to [1, Nq] / [1, Nk]) in its Nq / Nk rows.  Key tiles
+// past nk[b] are not loaded, the last one is masked as the tail of a call with Nk = nk[b], and a query tile wholly past
+// nq[b] is written as zeros after one key tile.  Rows of a real query equal vcr_flash_attn_tc on the item alone, bit for
+// bit, provided the padded V columns of the last key tile are finite (their probability is exactly 0).  Always the default
+// organisation (Q and P in tensor memory); no key mask, no lse.
+VCR_API int vcr_flash_attn_tc_ragged(const void* Q, int ldq, long long q_plane, const void* K, int ldk, long long k_plane,
+                                     const void* VT, int ldv, long long v_plane, const int* nq, const int* nk, int B, int H,
+                                     int Nq, int Nk, int dk, int mode, float scale, void* O, int ldo, long long o_plane,
+                                     cudaStream_t stream) {
+    VCR_REQUIRE(Q && K && VT && O && nq && nk && B > 0 && H > 0 && Nq > 0 && Nk > 0);
+    return flash_ragged_launch(Q, ldq, q_plane, K, ldk, k_plane, VT, ldv, v_plane, nq, nk, B, H, Nq, Nk, dk, mode, scale,
+                               nullptr, O, ldo, o_plane, stream);
+}
+
+// vcr_flash_attn_tc_ragged with the partial-overlap key mask keep [B, Nk] (uint8, row stride Nk): a key of item b with
+// keep == 0 gets -1e9 as in vcr_flash_attn_tc, a key past nk[b] gets -inf whatever keep holds.  Rows of a real query equal
+// vcr_flash_attn_tc(keep = the item's first nk[b] mask bytes) on the item alone, bit for bit.
+VCR_API int vcr_flash_attn_tc_ragged_keep(const void* Q, int ldq, long long q_plane, const void* K, int ldk,
+                                          long long k_plane, const void* VT, int ldv, long long v_plane, const int* nq,
+                                          const int* nk, const uint8_t* keep, int B, int H, int Nq, int Nk, int dk, int mode,
+                                          float scale, void* O, int ldo, long long o_plane, cudaStream_t stream) {
+    VCR_REQUIRE(Q && K && VT && O && nq && nk && keep && B > 0 && H > 0 && Nq > 0 && Nk > 0);
+    return flash_ragged_launch(Q, ldq, q_plane, K, ldk, k_plane, VT, ldv, v_plane, nq, nk, B, H, Nq, Nk, dk, mode, scale,
+                               keep, O, ldo, o_plane, stream);
 }

@@ -17,13 +17,20 @@ __device__ __forceinline__ unsigned int float_desc_key(float v) {
     return ~u;                                           // descending
 }
 
+// RAGGED: row b holds n_len[b] keys (clamped to [0, n]) of its n and selects k_len[b] of them (clamped to [0, min(K, n_b)]);
+// keys past the row are the sentinel ~0, idx_out past the row's count is 0.  Every key is unique (index in the low word), so
+// the sorted prefix does not depend on npad: the indices equal those of the row sorted alone.
+template <bool RAGGED>
 __global__ void topk_sort_kernel(const float* __restrict__ vals, int n, int npad, int K,
-                                 int* __restrict__ idx_out, uint8_t* __restrict__ mask_out) {
+                                 int* __restrict__ idx_out, uint8_t* __restrict__ mask_out,
+                                 const int* __restrict__ n_len, const int* __restrict__ k_len) {
     extern __shared__ unsigned long long keys[];
     const int b = blockIdx.x;
     const float* v = vals + (size_t)b * n;
+    const int nb = RAGGED ? min(max(__ldg(n_len + b), 0), n) : n;
+    const int kb = RAGGED ? min(max(__ldg(k_len + b), 0), min(K, nb)) : K;
     for (int i = threadIdx.x; i < npad; i += blockDim.x)
-        keys[i] = i < n ? (((unsigned long long)float_desc_key(v[i]) << 32) | (unsigned int)i) : ~0ull;
+        keys[i] = i < nb ? (((unsigned long long)float_desc_key(v[i]) << 32) | (unsigned int)i) : ~0ull;
     __syncthreads();
     for (int size = 2; size <= npad; size <<= 1) {
         for (int stride = size >> 1; stride > 0; stride >>= 1) {
@@ -41,6 +48,10 @@ __global__ void topk_sort_kernel(const float* __restrict__ vals, int n, int npad
         for (int i = threadIdx.x; i < n; i += blockDim.x) mask_out[(size_t)b * n + i] = 0;
     __syncthreads();
     for (int r = threadIdx.x; r < K; r += blockDim.x) {
+        if (RAGGED && r >= kb) {
+            if (idx_out) idx_out[(size_t)b * K + r] = 0;
+            continue;
+        }
         const int i = (int)(keys[r] & 0xffffffffu);
         if (idx_out) idx_out[(size_t)b * K + r] = i;
         if (mask_out) mask_out[(size_t)b * n + i] = 1;
@@ -50,13 +61,16 @@ __global__ void topk_sort_kernel(const float* __restrict__ vals, int n, int npad
 // npad <= 1024: one key per thread.  Compare-exchange partners closer than a warp are reached with shuffles, the 15 stages
 // with stride >= 32 go through double-buffered shared memory (one barrier each): 15 barriers instead of 55.  Same network,
 // same result as topk_sort_kernel.
+template <bool RAGGED>
 __global__ void __launch_bounds__(1024)
 topk_sort_warp_kernel(const float* __restrict__ vals, int n, int npad, int K, int* __restrict__ idx_out,
-                      uint8_t* __restrict__ mask_out) {
+                      uint8_t* __restrict__ mask_out, const int* __restrict__ n_len, const int* __restrict__ k_len) {
     __shared__ unsigned long long xch[2][1024];
     const int b = blockIdx.x, tid = threadIdx.x;
     const float* v = vals + (size_t)b * n;
-    unsigned long long key = tid < n ? (((unsigned long long)float_desc_key(v[tid]) << 32) | (unsigned int)tid) : ~0ull;
+    const int nb = RAGGED ? min(max(__ldg(n_len + b), 0), n) : n;
+    const int kb = RAGGED ? min(max(__ldg(k_len + b), 0), min(K, nb)) : K;
+    unsigned long long key = tid < nb ? (((unsigned long long)float_desc_key(v[tid]) << 32) | (unsigned int)tid) : ~0ull;
     int buf = 0;
     for (int size = 2; size <= npad; size <<= 1) {
         const bool up = (tid & size) == 0;
@@ -78,7 +92,9 @@ topk_sort_warp_kernel(const float* __restrict__ vals, int n, int npad, int K, in
     if (mask_out)
         for (int i = tid; i < n; i += blockDim.x) mask_out[(size_t)b * n + i] = 0;
     __syncthreads();
-    if (tid < K) {
+    if (RAGGED && tid >= kb && tid < K) {
+        if (idx_out) idx_out[(size_t)b * K + tid] = 0;
+    } else if (tid < K) {
         const int i = (int)(key & 0xffffffffu);
         if (idx_out) idx_out[(size_t)b * K + tid] = i;
         if (mask_out) mask_out[(size_t)b * n + i] = 1;
@@ -206,6 +222,26 @@ int topk_cluster_launch(const float* vals, int B, int n, int npad, int K, int* i
     return VCR_OK;
 }
 
+int topk_launch_cta(const float* vals, int B, int n, int npad, int K, int* idx_out, uint8_t* mask_out,
+                           const int* n_len, const int* k_len, cudaStream_t stream) {
+    const bool ragged = n_len != nullptr;
+    if (npad >= 32 && npad <= 1024) {
+        if (ragged) topk_sort_warp_kernel<true><<<B, npad, 0, stream>>>(vals, n, npad, K, idx_out, mask_out, n_len, k_len);
+        else topk_sort_warp_kernel<false><<<B, npad, 0, stream>>>(vals, n, npad, K, idx_out, mask_out, nullptr, nullptr);
+        VCR_CHECK_LAUNCH();
+        return VCR_OK;
+    }
+    const size_t smem = (size_t)npad * sizeof(unsigned long long);
+    if (smem > 224 * 1024) return VCR_ERR_UNSUPPORTED;
+    auto kern = ragged ? topk_sort_kernel<true> : topk_sort_kernel<false>;
+    if (smem > 48 * 1024 && cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        return VCR_ERR_LAUNCH;
+    const int threads = npad / 2 < 1024 ? (npad / 2 < 32 ? 32 : npad / 2) : 1024;
+    kern<<<B, threads, smem, stream>>>(vals, n, npad, K, idx_out, mask_out, n_len, k_len);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
 }  // namespace
 
 // vals [B,n] -> idx_out [B,K] (sorted, optional) and/or mask_out [B,n] uint8 (1 = selected, optional).
@@ -216,19 +252,18 @@ VCR_API int vcr_topk_select(const float* vals, int B, int n, int K, int* idx_out
     VCR_REQUIRE(vals && (idx_out || mask_out) && B > 0 && n > 0 && K > 0 && K <= n);
     int npad = 2;
     while (npad < n) npad <<= 1;
-    if (npad >= 32 && npad <= 1024) {
-        topk_sort_warp_kernel<<<B, npad, 0, stream>>>(vals, n, npad, K, idx_out, mask_out);
-        VCR_CHECK_LAUNCH();
-        return VCR_OK;
-    }
     if (npad > TOPK_SLICE) return topk_cluster_launch(vals, B, n, npad, K, idx_out, mask_out, stream);
-    const size_t smem = (size_t)npad * sizeof(unsigned long long);
-    if (smem > 224 * 1024) return VCR_ERR_UNSUPPORTED;
-    if (smem > 48 * 1024 &&
-        cudaFuncSetAttribute(topk_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-        return VCR_ERR_LAUNCH;
-    const int threads = npad / 2 < 1024 ? (npad / 2 < 32 ? 32 : npad / 2) : 1024;
-    topk_sort_kernel<<<B, threads, smem, stream>>>(vals, n, npad, K, idx_out, mask_out);
-    VCR_CHECK_LAUNCH();
-    return VCR_OK;
+    return topk_launch_cta(vals, B, n, npad, K, idx_out, mask_out, nullptr, nullptr, stream);
+}
+
+// Ragged rows: row b of vals [B, n] holds n_len[b] values (clamped to [0, n]) and selects k_len[b] of them (clamped to
+// [0, min(K, n_len[b])]).  idx_out [B, K]: the row's k_len[b] indices as vcr_topk_select on the row alone, then 0;
+// mask_out [B, n]: 1 on the selected keys, 0 elsewhere (past n_len[b] too).  n <= 16 384 (one CTA per row).
+VCR_API int vcr_topk_select_ragged(const float* vals, const int* n_len, const int* k_len, int B, int n, int K,
+                                   int* idx_out, uint8_t* mask_out, cudaStream_t stream) {
+    VCR_REQUIRE(vals && n_len && k_len && (idx_out || mask_out) && B > 0 && n > 0 && K > 0 && K <= n);
+    int npad = 2;
+    while (npad < n) npad <<= 1;
+    if (npad > TOPK_SLICE) return VCR_ERR_UNSUPPORTED;
+    return topk_launch_cta(vals, B, n, npad, K, idx_out, mask_out, n_len, k_len, stream);
 }

@@ -43,7 +43,7 @@ struct SoftcorrParams {
     const float* col_m;   // [B,Nt] per-column max        (mode 4)
     const float* col_il;  // [B,Nt] per-column 1 / sum    (mode 4)
     float* row_stat;      // [B,Ns] sum_j exp(pd_ij - col_m_j) * col_il_j   (mode 4)
-    const int* ns_len;    // ragged batch (mode 0): rows of item b, or null
+    const int* ns_len;    // ragged batch (modes 0 and 2): rows of item b, or null
     const int* nt_len;    // columns of item b, or null (a uniform batch)
 };
 
@@ -172,6 +172,13 @@ softcorr_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                     cb[row] = 0.f; cb[p.Ns + row] = 0.f; cb[2 * p.Ns + row] = 0.f;
                 }
                 if (tiles_n == 0) continue;                    // item without target tiles: nothing else to do (uniform per item)
+            }
+            if (MODE == 2 && p.ns_len != nullptr && !row_ok) { // ragged batch: best_idx = 0, best_val = 0 past the sources
+                if (chalf == 0 && row < p.Ns) {
+                    p.best_idx[(size_t)b * p.Ns + row] = 0;
+                    p.best_val[(size_t)b * p.Ns + row] = 0.f;
+                }
+                if (tiles_n == 0) continue;
             }
             const float nx = row_ok ? -p.xx[(size_t)b * p.Ns + row] : 0.f;
             const float* yb = p.yy + (size_t)b * p.Nt;
@@ -323,7 +330,8 @@ static int softcorr_run(const CUtensorMap& tmA, const CUtensorMap& tmB, const So
 // Replaces the matmul + softmax + matmul of model/vcrnet_model.py:337-345 without materialising the score matrix.
 static int softcorr_launch(int mode, const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
                            const float* xx, const float* yy, const float* tgt, int B, int Ns, int Nt, int D,
-                           float* corr, int* best_idx, float* best_val, cudaStream_t stream) {
+                           float* corr, int* best_idx, float* best_val, cudaStream_t stream, const int* ns_len = nullptr,
+                           const int* nt_len = nullptr) {
     if ((long long)B * (Ns > Nt ? Ns : Nt) > 0x7fffffffLL) return VCR_ERR_UNSUPPORTED;
     CUtensorMap tmA, tmB;
     int rc = vcr_make_operand_tmap(&tmA, S, D, (long long)B * Ns, lds, s_plane, 2, BM);
@@ -333,6 +341,7 @@ static int softcorr_launch(int mode, const void* S, int lds, long long s_plane, 
     SoftcorrParams p = {};
     p.B = B; p.Ns = Ns; p.Nt = Nt; p.D = D; p.xx = xx; p.yy = yy; p.tgt = tgt; p.corr = corr;
     p.best_idx = best_idx; p.best_val = best_val;
+    p.ns_len = ns_len; p.nt_len = nt_len;
     return mode == 0 ? softcorr_run<0, false>(tmA, tmB, p, stream) : softcorr_run<2, false>(tmA, tmB, p, stream);
 }
 
@@ -406,4 +415,15 @@ VCR_API int vcr_softcorr_tc_ragged(const void* S, int lds, long long s_plane, co
     p.B = B; p.Ns = Ns; p.Nt = Nt; p.D = D; p.xx = xx; p.yy = yy; p.tgt = tgt; p.corr = corr;
     p.ns_len = ns; p.nt_len = nt;
     return softcorr_run<0, false>(tmA, tmB, p, stream);
+}
+
+// getCopair (vcr_softcorr_best_tc) of a ragged batch: item b has ns[b] sources and nt[b] targets (each clamped to [1, Ns] /
+// [1, Nt]) in its Ns / Nt rows, with the tile walk of vcr_softcorr_tc_ragged.  Rows < ns[b] equal vcr_softcorr_best_tc on
+// the pair alone, bit for bit; rows past ns[b] get best_idx = 0 and best_val = 0.
+VCR_API int vcr_softcorr_best_tc_ragged(const void* S, int lds, long long s_plane, const void* T, int ldt, long long t_plane,
+                                        const float* xx, const float* yy, const int* ns, const int* nt, int B, int Ns, int Nt,
+                                        int D, int* best_idx, float* best_val, cudaStream_t stream) {
+    VCR_REQUIRE(S && T && xx && yy && ns && nt && best_idx && best_val && B > 0 && Ns > 0 && Nt > 0 && D > 0);
+    return softcorr_launch(2, S, lds, s_plane, T, ldt, t_plane, xx, yy, nullptr, B, Ns, Nt, D, nullptr, best_idx, best_val,
+                           stream, ns, nt);
 }

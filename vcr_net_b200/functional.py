@@ -14,7 +14,7 @@ import math
 
 import torch
 
-from . import config, ops
+from . import config, ops, ragged
 
 _F32 = torch.float32
 
@@ -583,15 +583,34 @@ def mha_project_kv(m, xkv_op, B, Nk, mode, dev, k_out=None, vt_out=None):
 def mha_attention(m, q_v, k_v, vt, B, Nq, Nk, mode, dev, max_ws_bytes=3 << 30, lens=None):
     """softmax(QK^T/sqrt(d_k)) V (+ the partial-overlap key selection, model/transformer.py:29-55) with the heads merged:
     -> operand-format [B*Nq, D].  q_v / k_v / vt: operand-format projections of B batch items.
-    lens: (query lengths, key lengths) int32 [B] of a ragged batch -- the flash kernel attends to each item's own keys."""
+    lens: (query lengths, key lengths) int32 [B] of a ragged batch -- the flash kernel attends to each item's own keys, and
+    the partial-overlap selection keeps int(nk[b] * overlap2) of them, as on the item alone."""
     D, h, dk = m.h * m.d_k, m.h, m.d_k
     scale = 1.0 / math.sqrt(dk)
     att = ops.Operand.empty(B * Nq, D, mode, dev)
     if lens is not None:
-        if m.is_src or dk != 128 or not config.flash_attention or m.__dict__.get("record_attn", False):
-            raise NotImplementedError("ragged batches: attention needs the flash kernel (d_k = 128, VCR_FLASH on), "
-                                      "no partial-overlap key selection and no record_attn")
-        return ops.flash_attn_tc_ragged(q_v, k_v, vt, att, B, h, Nq, Nk, dk, scale, lens[0], lens[1])
+        if dk != 128 or not config.flash_attention or m.__dict__.get("record_attn", False):
+            raise NotImplementedError("ragged batches: attention needs the flash kernel (d_k = 128, VCR_FLASH on) "
+                                      "and no record_attn")
+        if not m.is_src:
+            return ops.flash_attn_tc_ragged(q_v, k_v, vt, att, B, h, Nq, Nk, dk, scale, lens[0], lens[1])
+        nq, nk = lens
+        if mode == "h3" and config.fused_key_stat:
+            csum = ops.attn_colsum_tc_ragged(q_v, k_v, B, h, Nq, Nk, dk, scale, nq, nk)
+        else:
+            ldS = (Nk + 3) // 4 * 4
+            cb = max(1, min(B, min(max_ws_bytes, config.stat_chunk_bytes) // (h * Nq * ldS * 4)))
+            S = torch.empty((cb, h, Nq, ldS), dtype=_F32, device=dev)
+            csum = torch.empty((B, Nk), dtype=_F32, device=dev)
+            for b0 in range(0, B, cb):
+                nb = min(cb, B - b0)
+                ops.gemm_tc(q_v.rows_view(b0 * Nq, nb * Nq), k_v.rows_view(b0 * Nk, nb * Nk), Nq, Nk, dk, nbo=nb, nbi=h,
+                            a_off=(Nq, 0, 0, dk), b_off=(Nk, 0, 0, dk), alpha=scale, c=S,
+                            c_strides=(h * Nq * ldS, Nq * ldS))
+                csum[b0:b0 + nb] = ops.softmax_colsum_ragged(S[:nb], h, Nq, Nk, nq[b0:b0 + nb], nk[b0:b0 + nb])
+        _, keep = ops.topk_select_ragged(csum, nk, ragged.key_counts(nk, m.overlap2), int(Nk * m.overlap2),
+                                         want_idx=False, want_mask=True)
+        return ops.flash_attn_tc_ragged_keep(q_v, k_v, vt, att, B, h, Nq, Nk, dk, scale, nq, nk, keep)
     keep = None
     if m.is_src:
         # partial overlap (:35-53): column sums of the unmasked probabilities pick the surviving keys.
@@ -1002,13 +1021,38 @@ def _select_stats_materialised(src_tok, tgt_tok, pre, B, Ns, Nt):
     return row_stat, col_stat
 
 
-def vcp_select(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2, pre=None, want_tokens=True):
+def _select_stats_ragged(src_tok, tgt_tok, pre, B, Ns, Nt, ns, nt):
+    """_select_stats_materialised of a ragged batch: each pair takes the route it takes alone (fused up to 1 024 targets,
+    materialised beyond), chosen on the device.  The fused kernels read dot first; negdist_ then overwrites it in place."""
+    if pre is None:
+        src_tok, tgt_tok = src_tok.contiguous(), tgt_tok.contiguous()
+        dot, ld = pair_dots(src_tok, tgt_tok)
+        xx, yy = ops.sqnorm_rows(src_tok), ops.sqnorm_rows(tgt_tok)
+    else:
+        D = pre[0].op.cols
+        ld = (Nt + 3) // 4 * 4
+        dot = torch.empty((B, Ns, ld), dtype=_F32, device=pre[0].sq.device)
+        ops.gemm_tc(pre[0].op, pre[1].op, Ns, Nt, D, nbo=B, a_off=(Ns, 0, 0, 0), b_off=(Nt, 0, 0, 0), c=dot,
+                    c_strides=(Ns * ld, 0))
+        xx, yy = pre[0].sq, pre[1].sq
+    row_stat, col_stat = ops.select_stats_ragged(dot, ld, Ns, Nt, xx, yy, ns, nt)
+    if Nt > 1024:
+        pd = ops.negdist_(dot, ld, Ns, Nt, xx, yy)
+        ops.rowsum_colsoftmax_ragged(pd, ld, Ns, Nt, ns, nt, out=row_stat)
+        ops.softmax_rows_ragged_(pd, ld, Ns, Nt, ns, nt)
+        ops.colsum_ragged(pd, ld, Ns, Nt, ns, nt, out=col_stat)
+    return row_stat, col_stat
+
+
+def vcp_select(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2, pre=None, want_tokens=True, lengths=None):
     """selectCom (model/vcrnet_model.py:190-262) without the unused *_remain host round trips.
 
     The two selection statistics come from one fused two-read pass over the score products (vcr_select_stats), or, in
     the tensor-core modes past 16 384 points, from the operands without the score products (vcr_select_stats_tc).  With
     ``pre`` (operand copies + squared norms of both embeddings) and ``want_tokens=False`` the selected embeddings are
-    returned as ``Selected`` operand rows for vcp_copair instead of fp32 tokens (src_tok / tgt_tok may then be None)."""
+    returned as ``Selected`` operand rows for vcp_copair instead of fp32 tokens (src_tok / tgt_tok may then be None).
+    lengths: (src lengths, tgt lengths) int32 [B] of a ragged batch (up to 16 384 points, tensor-core modes): pair b keeps
+    ragged.select_counts of each cloud, and the outputs are [.., int(N_max * 0.84 * overlap2)] wide, index 0 past them."""
     if pre is not None and config.precision == "fp32":
         pre = None
     ref = pre[0].sq if pre is not None else src_tok
@@ -1016,18 +1060,25 @@ def vcp_select(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2, pre=None, want_toke
     Nt = pre[1].sq.shape[1] if pre is not None else tgt_tok.shape[1]
     srcK = int(Ns * 0.84 * overlap2)
     tgtK = int(Nt * 0.84 * overlap2)
-    if pre is not None and max(Ns, Nt) > SELECT_STATS_MATERIALISED_MAX:
-        # past 16 384 points the [Ns, Nt] score matrix is 1 GB per pair and up: statistics from the operands instead
-        row_stat, col_stat = ops.select_stats_tc(pre[0].op, pre[1].op, pre[0].sq, pre[1].sq, B, Ns, Nt, pre[0].op.cols)
+    if lengths is not None:
+        ns, nt = lengths
+        row_stat, col_stat = _select_stats_ragged(src_tok, tgt_tok, pre, B, Ns, Nt, ns, nt)
+        idx_t, _ = ops.topk_select_ragged(col_stat, nt, ragged.select_counts(nt, overlap2), tgtK)
+        idx_s, _ = ops.topk_select_ragged(row_stat, ns, ragged.select_counts(ns, overlap2), srcK)
     else:
-        row_stat, col_stat = _select_stats_materialised(src_tok, tgt_tok, pre, B, Ns, Nt)
-    both = row_stat._base
-    if srcK == tgtK and both is not None and both is col_stat._base and tuple(both.shape) == (2, B, Ns):
-        idx = ops.topk_select(both.view(2 * B, Ns), srcK)[0]           # both rankings (:222, :244) in one launch
-        idx_s, idx_t = idx[:B], idx[B:]
-    else:
-        idx_t, _ = ops.topk_select(col_stat, tgtK)
-        idx_s, _ = ops.topk_select(row_stat, srcK)
+        if pre is not None and max(Ns, Nt) > SELECT_STATS_MATERIALISED_MAX:
+            # past 16 384 points the [Ns, Nt] score matrix is 1 GB per pair and up: statistics from the operands instead
+            row_stat, col_stat = ops.select_stats_tc(pre[0].op, pre[1].op, pre[0].sq, pre[1].sq, B, Ns, Nt,
+                                                     pre[0].op.cols)
+        else:
+            row_stat, col_stat = _select_stats_materialised(src_tok, tgt_tok, pre, B, Ns, Nt)
+        both = row_stat._base
+        if srcK == tgtK and both is not None and both is col_stat._base and tuple(both.shape) == (2, B, Ns):
+            idx = ops.topk_select(both.view(2 * B, Ns), srcK)[0]       # both rankings (:222, :244) in one launch
+            idx_s, idx_t = idx[:B], idx[B:]
+        else:
+            idx_t, _ = ops.topk_select(col_stat, tgtK)
+            idx_s, _ = ops.topk_select(row_stat, srcK)
     so, to = ops.gather_cols(src_xyz, idx_s), ops.gather_cols(tgt_xyz, idx_t)
     if pre is not None and not want_tokens:
         s_sel = Selected(*ops.gather_operand_rows(pre[0].op, pre[0].sq, idx_s, B, Ns))
@@ -1036,13 +1087,32 @@ def vcp_select(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2, pre=None, want_toke
     return so, ops.gather_rows(src_tok, idx_s), to, ops.gather_rows(tgt_tok, idx_t), idx_s, idx_t
 
 
-def vcp_copair(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2):
+def vcp_copair(src_xyz, src_tok, tgt_xyz, tgt_tok, overlap2, lengths=None):
     """getCopair (model/vcrnet_model.py:264-332): hard arg-max correspondences for the
     int(Ns*0.52*overlap2) most confident sources (tgtK == 1 makes val/val_sum == 1).
-    src_tok / tgt_tok: fp32 tokens [B,N,D], or ``Selected`` operand rows from vcp_select."""
+    src_tok / tgt_tok: fp32 tokens [B,N,D], or ``Selected`` operand rows from vcp_select.
+    lengths: (selected sources, selected targets) int32 [B] of a ragged batch (vcp_select's counts): pair b keeps
+    int(sel_s[b] * 0.52 * overlap2) correspondences; src_k / corr_k columns past them are 0, keep / best_i entries 0."""
     B, _, Ns = src_xyz.shape
     Nt = tgt_xyz.shape[2]
     srcK = int(Ns * 0.52 * overlap2)
+    if lengths is not None:
+        if config.precision == "fp32" or not config.fused_softcorr:
+            raise NotImplementedError("ragged batches: getCopair needs the fused tensor-core kernel (not fp32 mode, "
+                                      "VCR_FUSED_SOFTCORR on)")
+        ns, nt = lengths
+        if isinstance(src_tok, Selected):
+            s_op, t_op, xx, yy, D = src_tok.op, tgt_tok.op, src_tok.sq, tgt_tok.sq, src_tok.op.cols
+        else:
+            D = src_tok.shape[2]
+            xx, yy = ops.sqnorm_rows(src_tok), ops.sqnorm_rows(tgt_tok)
+            s_op = ops.to_operand(src_tok.reshape(B * Ns, D), "h3")
+            t_op = ops.to_operand(tgt_tok.reshape(B * Nt, D), "h3")
+        best_i, best_v = ops.softcorr_best_tc_ragged(s_op, t_op, xx, yy, B, Ns, Nt, D, ns, nt)
+        k = ragged.copair_counts(ns, overlap2)
+        keep, _ = ops.topk_select_ragged(best_v, ns, k, srcK)
+        src_k, corr_k = ops.copair_gather(src_xyz, tgt_xyz, keep, best_i)
+        return ops.zero_padding(src_k, k), ops.zero_padding(corr_k, k), keep, best_i
     if isinstance(src_tok, Selected):
         best_i, best_v = ops.softcorr_best_tc(src_tok.op, tgt_tok.op, src_tok.sq, tgt_tok.sq, B, Ns, Nt, src_tok.op.cols)
     else:

@@ -55,19 +55,58 @@ def vcrnetIterRagged(net, src, tgt, src_len, tgt_len, iter=1):
     Transformer or Identity pointer, topK head, the tensor-core precision modes; anything else raises
     NotImplementedError.  The network's cycle estimate (R_ba, t_ba of VCRNet.forward) is never computed: vcrnetIter
     returns the inverse of the composed pose instead, so ``cycle`` does not change the outputs."""
+    _check_ragged_support(net, "vcrnetIterRagged", partial=False)
+    return _iter_ragged(net, src, tgt, src_len, tgt_len, iter, "vcrnetIterRagged")
+
+
+# the ragged partial path runs the one-CTA top-K selection and the materialised selectCom statistics (DESIGN section 8)
+RAGGED_PARTIAL_MAX_POINTS = 16384
+
+
+def vcrnetIterRaggedPartial(net, src, tgt, src_len, tgt_len, iter=1):
+    """vcrnetIterRagged for partial-to-partial registration (VCRNet(partial=True)): pairs of different sizes in one call.
+
+    Same arguments, padding contract and graph-capture property as vcrnetIterRagged, up to 16 384 points per cloud.
+    Returns (srcK, src_corrK, R_ab, t_ab, R_ba, t_ba) as vcrnetIter does, srcK / src_corrK [B,3,K_max] with
+    K_max = count(Ns_max): pair b has K_b = ragged.corr_lengths(src_len, net.head.overlap2)[b] valid columns, the rest are
+    0.  Restricted to K_b columns, every output equals vcrnetIter(net, src_b, tgt_b, iter) on the pair alone bit for bit.
+    Supported: as vcrnetIterRagged, with partial=True; the cycle estimate is not computed.  An overlap2 that leaves a
+    cloud of 21 points with no key, selected point or correspondence raises ValueError."""
+    from .. import ragged
+    _check_ragged_support(net, "vcrnetIterRaggedPartial", partial=True)
+    for name, x in (("src", src), ("tgt", tgt)):
+        if x.dim() == 3 and x.shape[2] > RAGGED_PARTIAL_MAX_POINTS:
+            raise NotImplementedError(f"vcrnetIterRaggedPartial: {x.shape[2]} points in `{name}` (at most "
+                                      f"{RAGGED_PARTIAL_MAX_POINTS} per cloud; call vcrnetIter per pair beyond)")
+    n0 = ragged.MIN_POINTS
+    counts = [int(n0 * a.overlap2) for a in _partial_attentions(net)]
+    ov = net.head.overlap2
+    sel = int(n0 * 0.84 * ov)
+    counts += [sel, int(sel * 0.52 * ov)]
+    if min(counts) <= 0:
+        raise ValueError(f"vcrnetIterRaggedPartial: overlap2 = {ov} keeps nothing of a {n0}-point cloud")
+    return _iter_ragged(net, src, tgt, src_len, tgt_len, iter, "vcrnetIterRaggedPartial")
+
+
+def _partial_attentions(net):
+    if isinstance(net.pointer, Transformer):
+        return [m for m in net.pointer.modules() if getattr(m, "is_src", False)]
+    return []
+
+
+def _iter_ragged(net, src, tgt, src_len, tgt_len, iter, fn):
     from .. import config
-    _check_ragged_support(net)
     if config.precision == "fp32":
-        raise NotImplementedError("vcrnetIterRagged: precision 'fp32' (the tensor-core modes h3 / fp16 / bf16 are supported)")
+        raise NotImplementedError(f"{fn}: precision 'fp32' (the tensor-core modes h3 / fp16 / bf16 are supported)")
     B = src.shape[0]
     for name, x in (("src", src), ("tgt", tgt)):
         ops._chk(x, name)
         if x.dim() != 3 or x.shape[0] != B or x.shape[1] != 3:
-            raise ValueError(f"vcrnetIterRagged: `{name}` must be [B,3,N], got {tuple(x.shape)}")
+            raise ValueError(f"{fn}: `{name}` must be [B,3,N], got {tuple(x.shape)}")
     for name, n in (("src_len", src_len), ("tgt_len", tgt_len)):
         ops._lengths(n, B, name)
         if n.device != src.device:
-            raise ValueError(f"vcrnetIterRagged: `{name}` must be on {src.device}")
+            raise ValueError(f"{fn}: `{name}` must be on {src.device}")
     k = net.emb_nn.k
     with torch.no_grad():
         # the padding is replaced by zeros once: every padded row the network computes is then finite (flash attention
@@ -77,39 +116,43 @@ def vcrnetIterRagged(net, src, tgt, src_len, tgt_len, iter=1):
         R_f = t_f = None
         srcK = src_corrK = None
         for _ in range(iter):
-            srcK = transformed_src
-            src_corrK, R, t = _forward_ragged(net, transformed_src, tgt_z, src_len, tgt_len)
+            srcK, src_corrK, R, t = _forward_ragged(net, transformed_src, tgt_z, src_len, tgt_len)
             transformed_src = ops.rigid_apply(transformed_src, R, t)
             if R_f is None:
                 R_f, t_f = R, t
             else:
                 ops.pose_compose_(R, t, R_f, t_f)
         R_ba, t_ba = ops.pose_inverse(R_f, t_f)
-        return ops.zero_padding(srcK, src_len, k + 1), src_corrK, R_f, t_f, R_ba, t_ba
+        if not net.head.partial:
+            srcK = ops.zero_padding(srcK, src_len, k + 1)
+        return srcK, src_corrK, R_f, t_f, R_ba, t_ba
 
 
-def _check_ragged_support(net):
+def _check_ragged_support(net, fn, partial):
     if isinstance(net, nn.DataParallel):
-        raise NotImplementedError("vcrnetIterRagged: nn.DataParallel (pass the module on one device)")
+        raise NotImplementedError(f"{fn}: nn.DataParallel (pass the module on one device)")
     if not isinstance(net, VCRNet):
-        raise NotImplementedError(f"vcrnetIterRagged: {type(net).__name__} (a VCRNet is required)")
+        raise NotImplementedError(f"{fn}: {type(net).__name__} (a VCRNet is required)")
     if net.training:
-        raise NotImplementedError("vcrnetIterRagged: training mode (call .eval())")
+        raise NotImplementedError(f"{fn}: training mode (call .eval())")
     if not isinstance(net.emb_nn, LPDNet):
-        raise NotImplementedError(f"vcrnetIterRagged: emb_nn {type(net.emb_nn).__name__} (only lpdnet)")
+        raise NotImplementedError(f"{fn}: emb_nn {type(net.emb_nn).__name__} (only lpdnet)")
     if net.emb_nn.t3d or net.emb_nn.tfea:
-        raise NotImplementedError("vcrnetIterRagged: LPDNet with t3d / tfea")
+        raise NotImplementedError(f"{fn}: LPDNet with t3d / tfea")
     if not isinstance(net.pointer, (Transformer, Identity)):
-        raise NotImplementedError(f"vcrnetIterRagged: pointer {type(net.pointer).__name__} (transformer or identity)")
+        raise NotImplementedError(f"{fn}: pointer {type(net.pointer).__name__} (transformer or identity)")
     if not isinstance(net.head, VcpTopK):
-        raise NotImplementedError(f"vcrnetIterRagged: vcp_nn {type(net.head).__name__} (only topK)")
-    if net.head.partial:
-        raise NotImplementedError("vcrnetIterRagged: partial=True (only whole-to-whole registration)")
+        raise NotImplementedError(f"{fn}: vcp_nn {type(net.head).__name__} (only topK)")
+    if net.head.partial and not partial:
+        raise NotImplementedError(f"{fn}: partial=True (only whole-to-whole registration; vcrnetIterRaggedPartial "
+                                  "registers partial pairs)")
+    if partial and not net.head.partial:
+        raise NotImplementedError(f"{fn}: partial=False (vcrnetIterRagged registers whole-to-whole pairs)")
 
 
 def _forward_ragged(net, src, tgt, src_len, tgt_len):
-    """VCRNet.forward's (src_corrK, R_ab, t_ab) for a ragged batch (model/vcrnet_model.py:495-516, whole-to-whole)."""
-    from .. import config
+    """VCRNet.forward's (srcK, src_corrK, R_ab, t_ab) for a ragged batch (model/vcrnet_model.py:495-516)."""
+    from .. import config, ragged
     src_tok = Fn.lpdnet_tokens(net.emb_nn, src, lengths=src_len)
     tgt_tok = Fn.lpdnet_tokens(net.emb_nn, tgt, lengths=tgt_len)
     pre = None
@@ -125,9 +168,18 @@ def _forward_ragged(net, src, tgt, src_len, tgt_len):
                                               lens=(tgt_len, src_len))
         pre = (Fn.HeadPre(op_s, sq_s), Fn.HeadPre(op_t, sq_t))
         src_tok = tgt_tok = None
-    corr = Fn.vcp_whole(src_tok, tgt_tok, tgt, pre=pre, lengths=(src_len, tgt_len))            # :507
-    R, t, _, _ = ops.svd_head_ragged(src, corr, src_len)                                       # :509-516
-    return corr, R, t
+    if net.head.partial:                                                                       # :507 (selectCom, getCopair)
+        ov = net.head.overlap2
+        so, seo, to, teo, _, _ = Fn.vcp_select(src, src_tok, tgt, tgt_tok, ov, pre=pre, want_tokens=False,
+                                               lengths=(src_len, tgt_len))
+        sel = (ragged.select_counts(src_len, ov), ragged.select_counts(tgt_len, ov))
+        srcK, corr, _, _ = Fn.vcp_copair(so, seo, to, teo, ov, lengths=sel)
+        m = ragged.copair_counts(sel[0], ov)
+    else:
+        srcK, corr = src, Fn.vcp_whole(src_tok, tgt_tok, tgt, pre=pre, lengths=(src_len, tgt_len))
+        m = src_len
+    R, t, _, _ = ops.svd_head_ragged(srcK, corr, m)                                            # :509-516
+    return srcK, corr, R, t
 
 
 class _IterLoop(nn.Module):

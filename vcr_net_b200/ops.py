@@ -380,6 +380,22 @@ def flash_attn_tc_ragged(q: Operand, k: Operand, vt: Operand, out: Operand, B, H
     return out
 
 
+def flash_attn_tc_ragged_keep(q: Operand, k: Operand, vt: Operand, out: Operand, B, H, Nq, Nk, dk, scale, nq, nk,
+                              keep: torch.Tensor):
+    """flash_attn_tc_ragged with the partial-overlap key mask keep uint8 [B, Nk] (keys past nk[b] stay excluded)."""
+    L = lib()
+    nq, nk = _lengths(nq, B, "nq"), _lengths(nk, B, "nk")
+    _chk(keep, "keep", torch.uint8)
+    if tuple(keep.shape) != (B, Nk):
+        raise RuntimeError(f"vcr_net_b200: `keep` must have shape ({B}, {Nk}), got {tuple(keep.shape)}")
+    keep = keep.contiguous()
+    L.check(L.vcr_flash_attn_tc_ragged_keep(q.ptr, q.ld, q.plane_stride, k.ptr, k.ld, k.plane_stride, vt.ptr, vt.ld,
+                                            vt.plane_stride, nq.data_ptr(), nk.data_ptr(), keep.data_ptr(), B, H, Nq, Nk,
+                                            dk, TC_MODES[q.mode], float(scale), out.ptr, out.ld, out.plane_stride,
+                                            _stream(q.buf)), "vcr_flash_attn_tc_ragged_keep")
+    return out
+
+
 def attn_colsum_tc(q: Operand, k: Operand, B, H, Nq, Nk, dk, scale):
     """Column sums over heads and queries of softmax(Q K^T * scale) -> [B, Nk]; scores never reach HBM."""
     assert q.mode == "h3" and k.mode == "h3"
@@ -390,6 +406,37 @@ def attn_colsum_tc(q: Operand, k: Operand, B, H, Nq, Nk, dk, scale):
     out = torch.empty((B, Nk), dtype=_F32, device=dev)
     L.check(L.vcr_attn_colsum_tc(q.ptr, q.ld, q.plane_stride, k.ptr, k.ld, k.plane_stride, B, H, Nq, Nk, dk,
                                  float(scale), out.data_ptr(), ws.data_ptr(), wsb, _stream(q.buf)), "vcr_attn_colsum_tc")
+    return out
+
+
+def attn_colsum_tc_ragged(q: Operand, k: Operand, B, H, Nq, Nk, dk, scale, nq, nk):
+    """attn_colsum_tc of a ragged batch (item b: nq[b] queries, nk[b] keys) -> [B, Nk], 0 past nk[b]."""
+    assert q.mode == "h3" and k.mode == "h3"
+    dev = q.buf.device
+    nq, nk = _lengths(nq, B, "nq"), _lengths(nk, B, "nk")
+    L = lib()
+    wsb = L.vcr_attn_colsum_workspace_bytes(B, H, Nq, Nk)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+    out = torch.empty((B, Nk), dtype=_F32, device=dev)
+    L.check(L.vcr_attn_colsum_tc_ragged(q.ptr, q.ld, q.plane_stride, k.ptr, k.ld, k.plane_stride, nq.data_ptr(),
+                                        nk.data_ptr(), B, H, Nq, Nk, dk, float(scale), out.data_ptr(), ws.data_ptr(), wsb,
+                                        _stream(q.buf)), "vcr_attn_colsum_tc_ragged")
+    return out
+
+
+def softmax_colsum_ragged(S: torch.Tensor, H: int, Nq: int, Nk: int, nq, nk):
+    """Key statistic of a ragged batch over scaled scores S fp32 [B, H, Nq, ld] -> [B, Nk] (0 past nk[b]); each item's
+    columns equal colsum_softmax on the item alone."""
+    _chk(S, "S")
+    B, ld = S.shape[0], S.shape[-1]
+    assert tuple(S.shape) == (B, H, Nq, ld) and S.is_contiguous()
+    nq, nk = _lengths(nq, B, "nq"), _lengths(nk, B, "nk")
+    L = lib()
+    wsb = L.vcr_softmax_colsum_ragged_workspace_bytes(B, H, Nq, Nk)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=S.device)
+    out = torch.empty((B, Nk), dtype=_F32, device=S.device)
+    L.check(L.vcr_softmax_colsum_ragged(S.data_ptr(), ld, nq.data_ptr(), nk.data_ptr(), B, H, Nq, Nk, out.data_ptr(),
+                                        ws.data_ptr(), wsb, _stream(S)), "vcr_softmax_colsum_ragged")
     return out
 
 
@@ -707,6 +754,25 @@ def colsum(P: torch.Tensor, B: int, out=None):
 TOPK_MAX_N = 16 * 16384
 
 
+def topk_select_ragged(vals: torch.Tensor, n: torch.Tensor, k: torch.Tensor, K: int, want_idx=True, want_mask=False):
+    """topk_select of ragged rows: row b of vals [B, N] holds n[b] values and selects k[b] <= K of them (int32 [B] device
+    tensors).  -> (idx int32 [B, K], 0 past k[b]; mask uint8 [B, N]), either None when not wanted."""
+    _chk(vals, "vals")
+    vals = vals.contiguous()
+    B, N = vals.shape
+    n, k = _lengths(n, B, "n"), _lengths(k, B, "k")
+    if N > 16384:
+        raise RuntimeError(f"vcr_net_b200: ragged top-K selection takes up to 16384 values a row, got {N}")
+    idx = torch.empty((B, K), dtype=torch.int32, device=vals.device) if want_idx else None
+    mask = torch.empty((B, N), dtype=torch.uint8, device=vals.device) if want_mask else None
+    L = lib()
+    L.check(L.vcr_topk_select_ragged(vals.data_ptr(), n.data_ptr(), k.data_ptr(), B, N, K,
+                                     idx.data_ptr() if idx is not None else None,
+                                     mask.data_ptr() if mask is not None else None, _stream(vals)),
+            "vcr_topk_select_ragged")
+    return idx, mask
+
+
 def topk_select(vals: torch.Tensor, K: int, want_idx=True, want_mask=False):
     _chk(vals, "vals")
     vals = vals.contiguous()
@@ -840,6 +906,71 @@ def softcorr_best_tc(s_op: "Operand", t_op: "Operand", xx, yy, B: int, Ns: int, 
                                    xx.data_ptr(), yy.data_ptr(), B, Ns, Nt, D, best_i.data_ptr(), best_v.data_ptr(),
                                    _stream(xx)), "vcr_softcorr_best_tc")
     return best_i, best_v
+
+
+def softcorr_best_tc_ragged(s_op: "Operand", t_op: "Operand", xx, yy, B: int, Ns: int, Nt: int, D: int, ns, nt):
+    """softcorr_best_tc of a ragged batch (pair b: ns[b] sources, nt[b] targets); rows past ns[b] are (0, 0)."""
+    assert s_op.mode == "h3" and t_op.mode == "h3" and s_op.rows == B * Ns and t_op.rows == B * Nt
+    dev = xx.device
+    ns, nt = _lengths(ns, B, "ns"), _lengths(nt, B, "nt")
+    best_i = torch.empty((B, Ns), dtype=torch.int32, device=dev)
+    best_v = torch.empty((B, Ns), dtype=_F32, device=dev)
+    L = lib()
+    L.check(L.vcr_softcorr_best_tc_ragged(s_op.ptr, s_op.ld, s_op.plane_stride, t_op.ptr, t_op.ld, t_op.plane_stride,
+                                          xx.data_ptr(), yy.data_ptr(), ns.data_ptr(), nt.data_ptr(), B, Ns, Nt, D,
+                                          best_i.data_ptr(), best_v.data_ptr(), _stream(xx)), "vcr_softcorr_best_tc_ragged")
+    return best_i, best_v
+
+
+def select_stats_ragged(dot: torch.Tensor, ld: int, Ns: int, Nt: int, xx, yy, ns, nt, row_stat=None, col_stat=None):
+    """select_stats of a ragged batch for the pairs with nt[b] <= 1024 (the others are left untouched):
+    -> (row_stat [B, Ns], col_stat [B, Nt]), 0 past each pair's lengths."""
+    B = dot.shape[0]
+    dev = dot.device
+    ns, nt = _lengths(ns, B, "ns"), _lengths(nt, B, "nt")
+    row_stat = torch.empty((B, Ns), dtype=_F32, device=dev) if row_stat is None else row_stat
+    col_stat = torch.empty((B, Nt), dtype=_F32, device=dev) if col_stat is None else col_stat
+    L = lib()
+    wsb = L.vcr_select_stats_workspace_bytes(B, Ns, Nt)
+    ws = torch.empty(wsb // 4, dtype=_F32, device=dev)
+    L.check(L.vcr_select_stats_ragged(dot.data_ptr(), ld, ns.data_ptr(), nt.data_ptr(), B, Ns, Nt, xx.data_ptr(),
+                                      yy.data_ptr(), row_stat.data_ptr(), col_stat.data_ptr(), ws.data_ptr(), wsb,
+                                      _stream(dot)), "vcr_select_stats_ragged")
+    return row_stat, col_stat
+
+
+def rowsum_colsoftmax_ragged(pd, ld, Ns, Nt, ns, nt, out):
+    """rowsum_colsoftmax of a ragged batch into out [B, Ns], for the pairs with nt[b] > 1024."""
+    B = pd.shape[0]
+    ns, nt = _lengths(ns, B, "ns"), _lengths(nt, B, "nt")
+    L = lib()
+    ws = torch.empty(L.vcr_rowsum_colsoftmax_workspace_bytes(B, Nt) // 4, dtype=_F32, device=pd.device)
+    L.check(L.vcr_rowsum_colsoftmax_ragged(pd.data_ptr(), ld, ns.data_ptr(), nt.data_ptr(), B, Ns, Nt, out.data_ptr(),
+                                           ws.data_ptr(), ws.numel() * 4, _stream(pd)), "vcr_rowsum_colsoftmax_ragged")
+    return out
+
+
+def softmax_rows_ragged_(S, ld, Ns, Nt, ns, nt):
+    """In-place row softmax of a ragged batch S [B, Ns, ld] over each pair's rows and columns, for the pairs with
+    nt[b] > 1024."""
+    B = S.shape[0]
+    ns, nt = _lengths(ns, B, "ns"), _lengths(nt, B, "nt")
+    L = lib()
+    L.check(L.vcr_softmax_rows_ragged(S.data_ptr(), ld, ns.data_ptr(), nt.data_ptr(), B, Ns, Nt, _stream(S)),
+            "vcr_softmax_rows_ragged")
+    return S
+
+
+def colsum_ragged(P, ld, Ns, Nt, ns, nt, out):
+    """colsum of a ragged batch P [B, Ns, ld] into out [B, Nt], for the pairs with nt[b] > 1024."""
+    B = P.shape[0]
+    ns, nt = _lengths(ns, B, "ns"), _lengths(nt, B, "nt")
+    L = lib()
+    wsb = L.vcr_colsum_workspace_bytes(B, Nt)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=P.device)
+    L.check(L.vcr_colsum_ragged(P.data_ptr(), ld, ns.data_ptr(), nt.data_ptr(), B, Ns, Nt, out.data_ptr(), ws.data_ptr(),
+                                wsb, _stream(P)), "vcr_colsum_ragged")
+    return out
 
 
 def negdist_(dot, ld, Ns, Nt, xx, yy):

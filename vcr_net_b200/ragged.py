@@ -38,3 +38,31 @@ def pad_clouds(clouds, n_max: int | None = None, device=None):
     for b, c in enumerate(clouds):
         out[b, :, :lengths[b]].copy_(c)
     return out, torch.tensor(lengths, dtype=torch.int32, device=device)
+
+
+# Per-pair counts of the partial path (model/transformer.py:41, model/vcrnet_model.py:200-201, :283), evaluated on the
+# device with Python's arithmetic: fp64 products left to right, truncated toward zero.  Each is non-decreasing in n, so
+# buffers sized from N_max hold every pair.
+def _trunc(x: torch.Tensor) -> torch.Tensor:
+    return x.to(torch.int32)
+
+
+def key_counts(nk: torch.Tensor, overlap2: float) -> torch.Tensor:
+    """int(nk * overlap2): the keys the partial cross attention keeps."""
+    return _trunc(nk.double() * float(overlap2))
+
+
+def select_counts(n: torch.Tensor, overlap2: float) -> torch.Tensor:
+    """int(n * 0.84 * overlap2): the points selectCom keeps of a cloud."""
+    return _trunc(n.double() * 0.84 * float(overlap2))
+
+
+def copair_counts(sel: torch.Tensor, overlap2: float) -> torch.Tensor:
+    """int(sel * 0.52 * overlap2): the correspondences getCopair keeps of sel selected sources."""
+    return _trunc(sel.double() * 0.52 * float(overlap2))
+
+
+def corr_lengths(src_len: torch.Tensor, overlap2: float) -> torch.Tensor:
+    """int(int(ns * 0.84 * overlap2) * 0.52 * overlap2): the correspondences getCopair keeps of pair b, the valid columns
+    of vcrnetIterRaggedPartial's srcK / src_corrK (int32 [B] on the lengths' device)."""
+    return copair_counts(select_counts(src_len, overlap2), overlap2)
