@@ -386,6 +386,32 @@ int vcr_crop_nearest_sort(const double* pc64, int P, int N, int keep, float* out
 int vcr_eval_metrics(const float* src, const float* tgt, int N, const float* srcK, const float* corrK, int M,
                      const float* R_gt, const float* t_gt, const float* R_ab, const float* t_ab,
                      const float* R_ba, const float* t_ba, int B, double* acc, cudaStream_t stream);
+/* Ragged batches of the data step (int32 per-item lengths on the device, read there only and clamped into range; no host
+ * sync, no allocation, so each call can be captured in a CUDA graph and replayed with new lengths):
+ * vcr_make_pairs_ragged: vcr_make_pairs with item p at n[p] points (clamped to [0, N_max]) of N_max columns; idx_src /
+ *   idx_tgt are [P, N_max] and are read below n[p] only.  Columns at or past n[p] are written as 0 in every output given.
+ *   P in [1, 65535], Nb >= 1, N_max >= 1, else -2.
+ * vcr_crop_nearest_ragged: the one-CTA crop of cloud p's first n[p] points (clamped to [1, N_max]) to the keep[p] (clamped
+ *   to [0, min(keep_max, n[p])]) nearest to its point n[p] - 1 -> out [P,3,keep_max], columns past keep[p] written as 0.
+ *   1 <= keep_max <= N_max <= 25 600 and P >= 1, else -2.
+ * vcr_crop_nearest_sort_ragged: the same by the radix sort for any N_max (limits and -2 as vcr_crop_nearest_sort); the
+ *   workspace is vcr_crop_nearest_workspace_bytes(P, N_max) bytes (-4 if smaller).  Keys past n[p] sort after every
+ *   point of the cloud, NaN distances included.  Where both apply and no distance is NaN, the two ragged crops, and the
+ *   uniform crop of each cloud alone, give the same bits.
+ * vcr_eval_metrics_ragged: vcr_eval_metrics with pair b over its n[b] points of src / tgt [B,3,N_max] and its m[b]
+ *   columns of srcK / corrK [B,3,M_max] (both clamped to [1, *]): each pair's sums are divided by its own denominators,
+ *   and pair b adds what vcr_eval_metrics on it alone adds (up to the order of the fp64 sums).  B in [1, 65535]. */
+int vcr_make_pairs_ragged(const float* base, int P, int Nb, const int* idx_src, const int* idx_tgt, const double* pose,
+                          const int* n, int N_max, double* src64, double* tgt64, float* src, float* tgt,
+                          cudaStream_t stream);
+int vcr_crop_nearest_ragged(const double* pc64, const int* n, const int* keep, int P, int N_max, int keep_max,
+                            float* out, cudaStream_t stream);
+int vcr_crop_nearest_sort_ragged(const double* pc64, const int* n, const int* keep, int P, int N_max, int keep_max,
+                                 float* out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+int vcr_eval_metrics_ragged(const float* src, const float* tgt, const int* n, int N_max, const float* srcK,
+                            const float* corrK, const int* m, int M_max, const float* R_gt, const float* t_gt,
+                            const float* R_ab, const float* t_ab, const float* R_ba, const float* t_ba, int B,
+                            double* acc, cudaStream_t stream);
 
 /* ---- ICP refinement (--iter=0): model/icp_model.py:26-108 ICP.forward, model/vcrnet_model.py:46-62 -----------
  * vcr_icp_nearest = nearest_neighbor (:52-75): corr [B,3,Ns] = nearest dst point per src point under

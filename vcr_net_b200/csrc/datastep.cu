@@ -13,6 +13,8 @@
 //   vcr_eval_metrics   model/vcrnet_model.py:583-630: pose loss, cycle loss, mse/mae of the a->b and b->a transformed
 //                      clouds, accumulated into a device-resident double[8] (the reference does 6+ .item() host
 //                      syncs per batch).
+// Each has a _ragged entry point for batches of clouds of different sizes (per-item lengths read on the device and
+// clamped into range); the ragged code is a template parameter compiled out of the uniform kernels.
 // Roofline: HBM / latency bound helpers (a few bytes per point); they exist to keep the 8 GPUs fed without host work.
 #include "common.cuh"
 
@@ -20,13 +22,23 @@ namespace {
 
 // base [P, Nb, 3] fp32; idx_src / idx_tgt [P, N] int32 (indices into the item's base cloud, permutations composed on
 // the host); pose [P, 12] fp64 = row-major R (9) then t (3).  src[p,:,n] = base[idx_src[n]], tgt[p,:,n] = R base[idx_tgt[n]] + t.
+// RAGGED: item p has n_len[p] points (clamped to [0, N]) of its N columns; the columns past them are written as 0.
+template <bool RAGGED>
 __global__ void make_pairs_kernel(const float* __restrict__ base, int Nb, const int* __restrict__ idx_src,
                                   const int* __restrict__ idx_tgt, const double* __restrict__ pose, int N,
                                   double* __restrict__ src64, double* __restrict__ tgt64,
-                                  float* __restrict__ src, float* __restrict__ tgt) {
+                                  float* __restrict__ src, float* __restrict__ tgt, const int* __restrict__ n_len) {
     const int p = blockIdx.y;
     const int n = blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= N) return;
+    if (RAGGED && n >= min(max(__ldg(n_len + p), 0), N)) {
+        const size_t o0 = (size_t)p * 3 * N + n;
+        if (src64) { src64[o0] = 0.0; src64[o0 + N] = 0.0; src64[o0 + 2 * N] = 0.0; }
+        if (tgt64) { tgt64[o0] = 0.0; tgt64[o0 + N] = 0.0; tgt64[o0 + 2 * N] = 0.0; }
+        if (src) { src[o0] = 0.f; src[o0 + N] = 0.f; src[o0 + 2 * N] = 0.f; }
+        if (tgt) { tgt[o0] = 0.f; tgt[o0 + N] = 0.f; tgt[o0 + 2 * N] = 0.f; }
+        return;
+    }
     const float* bp = base + (size_t)p * Nb * 3;
     const double* ps = pose + (size_t)p * 12;
     const int is = idx_src[(size_t)p * N + n], it = idx_tgt[(size_t)p * N + n];
@@ -51,27 +63,42 @@ __device__ __forceinline__ double sqdist_to_anchor(double x, double y, double z,
     return __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
 }
 
-// pc64 [P,3,N] fp64 -> out [P,3,keep] fp32: the keep points nearest to point N-1, nearest first
-__global__ void crop_nearest_kernel(const double* __restrict__ pc64, int N, int keep, float* __restrict__ out) {
+// Ragged crop lengths: cloud p has nb = n_len[p] points (clamped to [1, N]: the anchor is its point nb - 1) and keeps
+// keep_len[p] of them (clamped to [0, min(keep, nb)]).
+__device__ __forceinline__ int crop_len(const int* n_len, int p, int N) { return min(max(__ldg(n_len + p), 1), N); }
+__device__ __forceinline__ int crop_keep(const int* keep_len, int p, int keep, int nb) {
+    return min(max(__ldg(keep_len + p), 0), min(keep, nb));
+}
+
+// pc64 [P,3,N] fp64 -> out [P,3,keep] fp32: the keep points nearest to point N-1, nearest first.
+// RAGGED: the kb points of cloud p's first nb nearest to its point nb - 1 (crop_len / crop_keep), columns kb.. of its keep
+// written as 0.
+template <bool RAGGED>
+__global__ void crop_nearest_kernel(const double* __restrict__ pc64, int N, int keep, float* __restrict__ out,
+                                    const int* __restrict__ n_len, const int* __restrict__ keep_len) {
     extern __shared__ double d2[];
     const int p = blockIdx.x;
+    const int nb = RAGGED ? crop_len(n_len, p, N) : N;
+    const int kb = RAGGED ? crop_keep(keep_len, p, keep, nb) : keep;
     const double* pc = pc64 + (size_t)p * 3 * N;
-    const double lx = pc[N - 1], ly = pc[2 * N - 1], lz = pc[3 * N - 1];
-    for (int i = threadIdx.x; i < N; i += blockDim.x)
+    const double lx = pc[nb - 1], ly = pc[N + nb - 1], lz = pc[2 * N + nb - 1];
+    for (int i = threadIdx.x; i < nb; i += blockDim.x)
         d2[i] = sqdist_to_anchor(pc[i], pc[N + i], pc[2 * N + i], lx, ly, lz);
     __syncthreads();
-    for (int i = threadIdx.x; i < N; i += blockDim.x) {
+    float* o = out + (size_t)p * 3 * keep;
+    for (int i = threadIdx.x; i < nb; i += blockDim.x) {
         const double di = d2[i];
         int rank = 0;
-        for (int j = 0; j < N; ++j) {
+        for (int j = 0; j < nb; ++j) {
             const double dj = d2[j];
             rank += (dj < di) || (dj == di && j < i);
         }
-        if (rank < keep) {
-            float* o = out + (size_t)p * 3 * keep;
+        if (rank < kb) {
             o[rank] = (float)pc[i]; o[keep + rank] = (float)pc[N + i]; o[2 * keep + rank] = (float)pc[2 * N + i];
         }
     }
+    if (RAGGED)
+        for (int j = kb + threadIdx.x; j < keep; j += blockDim.x) o[j] = o[keep + j] = o[2 * keep + j] = 0.f;
 }
 
 // ---- the same crop for any N: a stable LSD radix sort of (d2 bits, index) pairs, segmented per cloud ------------------
@@ -116,15 +143,25 @@ __device__ __forceinline__ unsigned block_exclusive_scan(unsigned v, unsigned* w
     return x - v + (w ? warp_tot[w - 1] : 0u);
 }
 
-// keys[p*N + i] = crop_key(d2 of point i of cloud p to its point N-1), idx[p*N + i] = i
+// keys[p*N + i] = crop_key(d2 of point i of cloud p to its point N-1), idx[p*N + i] = i.
+// RAGGED: the anchor is point nb - 1 (crop_len), and points at or past nb get the key ~0, above the NaN key: they sort
+// after every point of the cloud and the stable sort of the cloud's own keys is unchanged.
+template <bool RAGGED>
 __global__ void crop_keys_kernel(const double* __restrict__ pc64, int N, size_t total,
-                                 unsigned long long* __restrict__ keys, unsigned* __restrict__ idx) {
+                                 unsigned long long* __restrict__ keys, unsigned* __restrict__ idx,
+                                 const int* __restrict__ n_len) {
     const size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= total) return;
     const size_t p = g / N, i = g - p * N;
     const double* pc = pc64 + p * 3 * N;
-    keys[g] = crop_key(sqdist_to_anchor(pc[i], pc[N + i], pc[2 * (size_t)N + i], pc[N - 1], pc[2 * (size_t)N - 1],
-                                        pc[3 * (size_t)N - 1]));
+    if (RAGGED) {
+        const size_t a = crop_len(n_len, (int)p, N) - 1;
+        keys[g] = i > a ? ~0ull : crop_key(sqdist_to_anchor(pc[i], pc[N + i], pc[2 * (size_t)N + i], pc[a], pc[N + a],
+                                                            pc[2 * (size_t)N + a]));
+    } else {
+        keys[g] = crop_key(sqdist_to_anchor(pc[i], pc[N + i], pc[2 * (size_t)N + i], pc[N - 1], pc[2 * (size_t)N - 1],
+                                            pc[3 * (size_t)N - 1]));
+    }
     idx[g] = (unsigned)i;
 }
 
@@ -259,15 +296,23 @@ __global__ void __launch_bounds__(kSortThreads, 4) radix_scatter_kernel(
     }
 }
 
-// out[p, :, j] = (float)pc64[p, :, order[p*N + j]] for j < keep
+// out[p, :, j] = (float)pc64[p, :, order[p*N + j]] for j < keep.  RAGGED: columns at or past kb (crop_keep) are 0.
+template <bool RAGGED>
 __global__ void crop_gather_kernel(const double* __restrict__ pc64, int N, int keep, size_t total,
-                                   const unsigned* __restrict__ order, float* __restrict__ out) {
+                                   const unsigned* __restrict__ order, float* __restrict__ out,
+                                   const int* __restrict__ n_len, const int* __restrict__ keep_len) {
     const size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= total) return;
     const size_t p = g / keep, j = g - p * keep;
+    float* o = out + p * 3 * keep;
+    if (RAGGED && j >= (size_t)crop_keep(keep_len, (int)p, keep, crop_len(n_len, (int)p, N))) {
+        o[j] = 0.f;
+        o[keep + j] = 0.f;
+        o[2 * (size_t)keep + j] = 0.f;
+        return;
+    }
     const double* pc = pc64 + p * 3 * N;
     const size_t i = order[p * N + j];
-    float* o = out + p * 3 * keep;
     o[j] = (float)pc[i];
     o[keep + j] = (float)pc[N + i];
     o[2 * (size_t)keep + j] = (float)pc[2 * (size_t)N + i];
@@ -285,17 +330,30 @@ __device__ __forceinline__ void rigid(const float* R, const float* t, float x, f
 
 // acc[0] pose loss, [1] cycle loss, [2] mse_ab, [3] mae_ab, [4] mse_ba, [5] mae_ba, [6] number of examples (each already
 // multiplied by the batch size as the reference accumulates `.item() * batch_size`)
+// RAGGED: blockIdx.y is pair b0, which has nb = n_len[b0] cloud points of N and mb = m_len[b0] correspondences of M (each
+// clamped to [1, *]); the block's loops cover that pair alone (Bp = 1), so its sums are divided by the pair's own means'
+// denominators before they are accumulated, and the pair adds what a call on it alone adds.
+template <bool RAGGED>
 __global__ void eval_metrics_kernel(const float* __restrict__ src, const float* __restrict__ tgt, int N,
                                     const float* __restrict__ srcK, const float* __restrict__ corrK, int M,
                                     const float* __restrict__ R_gt, const float* __restrict__ t_gt,
                                     const float* __restrict__ R_ab, const float* __restrict__ t_ab,
                                     const float* __restrict__ R_ba, const float* __restrict__ t_ba, int B,
-                                    double* __restrict__ acc) {
+                                    double* __restrict__ acc, const int* __restrict__ n_len,
+                                    const int* __restrict__ m_len) {
     __shared__ double red[4][8];
+    const int b0 = RAGGED ? blockIdx.y : 0;
+    const int Bp = RAGGED ? 1 : B;
+    const int nb = RAGGED ? min(max(__ldg(n_len + b0), 1), N) : N;
+    const int mb = RAGGED ? min(max(__ldg(m_len + b0), 1), M) : M;
+    if (RAGGED) {
+        src += (size_t)b0 * 3 * N; tgt += (size_t)b0 * 3 * N; srcK += (size_t)b0 * 3 * M; corrK += (size_t)b0 * 3 * M;
+        R_gt += b0 * 9; t_gt += b0 * 3; R_ab += b0 * 9; t_ab += b0 * 3; R_ba += b0 * 9; t_ba += b0 * 3;
+    }
     double s_ab2 = 0.0, s_ab1 = 0.0, s_ba2 = 0.0, s_ba1 = 0.0;
     const int stride = gridDim.x * blockDim.x, g = blockIdx.x * blockDim.x + threadIdx.x;
-    for (long long e = g; e < (long long)B * M; e += stride) {             // transformed_srcK vs src_corrK (:591,623-624)
-        const int b = (int)(e / M), m = (int)(e - (long long)b * M);
+    for (long long e = g; e < (long long)Bp * mb; e += stride) {           // transformed_srcK vs src_corrK (:591,623-624)
+        const int b = (int)(e / mb), m = (int)(e - (long long)b * mb);
         const float* s = srcK + (size_t)b * 3 * M;
         const float* c = corrK + (size_t)b * 3 * M;
         float o[3];
@@ -303,8 +361,8 @@ __global__ void eval_metrics_kernel(const float* __restrict__ src, const float* 
 #pragma unroll
         for (int i = 0; i < 3; ++i) { const double d = (double)(o[i] - c[i * M + m]); s_ab2 += d * d; s_ab1 += fabs(d); }
     }
-    for (long long e = g; e < (long long)B * N; e += stride) {             // transformed_target vs src (:589,626-627)
-        const int b = (int)(e / N), n = (int)(e - (long long)b * N);
+    for (long long e = g; e < (long long)Bp * nb; e += stride) {           // transformed_target vs src (:589,626-627)
+        const int b = (int)(e / nb), n = (int)(e - (long long)b * nb);
         const float* t = tgt + (size_t)b * 3 * N;
         const float* s = src + (size_t)b * 3 * N;
         float o[3];
@@ -322,12 +380,12 @@ __global__ void eval_metrics_kernel(const float* __restrict__ src, const float* 
     if (threadIdx.x < 4) {
         double s = 0.0;
         for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += red[threadIdx.x][w];
-        const double denom = threadIdx.x < 2 ? 3.0 * M : 3.0 * N;          // mean over [B,3,*] times batch size
+        const double denom = threadIdx.x < 2 ? 3.0 * mb : 3.0 * nb;        // mean over [B,3,*] times batch size
         atomicAdd(acc + 2 + threadIdx.x, s / denom);
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) {                              // pose / cycle losses (:598-617), tiny
         double lr = 0.0, lt = 0.0, cr = 0.0, ct = 0.0;
-        for (int b = 0; b < B; ++b) {
+        for (int b = 0; b < Bp; ++b) {
             const float* Rp = R_ab + b * 9; const float* Rg = R_gt + b * 9; const float* Rb = R_ba + b * 9;
             for (int i = 0; i < 3; ++i)
                 for (int j = 0; j < 3; ++j) {
@@ -345,11 +403,11 @@ __global__ void eval_metrics_kernel(const float* __restrict__ src, const float* 
                 ct += c * c;
             }
         }
-        const double pose = lr / (9.0 * B) + lt / (3.0 * B);
-        const double cyc = cr / (9.0 * B) + ct / (3.0 * B);
-        atomicAdd(acc + 0, pose * B);
-        atomicAdd(acc + 1, cyc * B);
-        atomicAdd(acc + 6, (double)B);
+        const double pose = lr / (9.0 * Bp) + lt / (3.0 * Bp);
+        const double cyc = cr / (9.0 * Bp) + ct / (3.0 * Bp);
+        atomicAdd(acc + 0, pose * Bp);
+        atomicAdd(acc + 1, cyc * Bp);
+        atomicAdd(acc + 6, (double)Bp);
     }
 }
 
@@ -359,7 +417,18 @@ VCR_API int vcr_make_pairs(const float* base, int P, int Nb, const int* idx_src,
                            int N, double* src64, double* tgt64, float* src, float* tgt, cudaStream_t stream) {
     VCR_REQUIRE(base && idx_src && idx_tgt && pose && P > 0 && Nb > 0 && N > 0 && P <= 65535 && (src64 || src) && (tgt64 || tgt));
     dim3 g(vcr_cdiv(N, 256), P);
-    make_pairs_kernel<<<g, 256, 0, stream>>>(base, Nb, idx_src, idx_tgt, pose, N, src64, tgt64, src, tgt);
+    make_pairs_kernel<false><<<g, 256, 0, stream>>>(base, Nb, idx_src, idx_tgt, pose, N, src64, tgt64, src, tgt, nullptr);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
+VCR_API int vcr_make_pairs_ragged(const float* base, int P, int Nb, const int* idx_src, const int* idx_tgt,
+                                  const double* pose, const int* n, int N_max, double* src64, double* tgt64, float* src,
+                                  float* tgt, cudaStream_t stream) {
+    VCR_REQUIRE(base && idx_src && idx_tgt && pose && n && (src64 || src) && (tgt64 || tgt));
+    if (P < 1 || P > 65535 || Nb < 1 || N_max < 1) return VCR_ERR_UNSUPPORTED;
+    dim3 g(vcr_cdiv(N_max, 256), P);
+    make_pairs_kernel<true><<<g, 256, 0, stream>>>(base, Nb, idx_src, idx_tgt, pose, N_max, src64, tgt64, src, tgt, n);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
 }
@@ -369,8 +438,20 @@ VCR_API int vcr_crop_nearest(const double* pc64, int P, int N, int keep, float* 
     if ((size_t)N * sizeof(double) > 200 * 1024) return VCR_ERR_UNSUPPORTED;
     const size_t smem = (size_t)N * sizeof(double);
     // set on every launch: the attribute is per device, and one process may drive several (nn.DataParallel)
-    if (cudaFuncSetAttribute(crop_nearest_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) return VCR_ERR_LAUNCH;
-    crop_nearest_kernel<<<P, 256, smem, stream>>>(pc64, N, keep, out);
+    if (cudaFuncSetAttribute(crop_nearest_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) return VCR_ERR_LAUNCH;
+    crop_nearest_kernel<false><<<P, 256, smem, stream>>>(pc64, N, keep, out, nullptr, nullptr);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
+VCR_API int vcr_crop_nearest_ragged(const double* pc64, const int* n, const int* keep, int P, int N_max, int keep_max,
+                                    float* out, cudaStream_t stream) {
+    VCR_REQUIRE(pc64 && n && keep && out);
+    if (P < 1 || N_max < 1 || keep_max < 1 || keep_max > N_max || (size_t)N_max * sizeof(double) > 200 * 1024)
+        return VCR_ERR_UNSUPPORTED;
+    const size_t smem = (size_t)N_max * sizeof(double);
+    if (cudaFuncSetAttribute(crop_nearest_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) return VCR_ERR_LAUNCH;
+    crop_nearest_kernel<true><<<P, 256, smem, stream>>>(pc64, N_max, keep_max, out, n, keep);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
 }
@@ -401,8 +482,10 @@ VCR_API size_t vcr_crop_nearest_workspace_bytes(int P, int N) {
     return crop_sort_shape_ok(P, N) ? crop_sort_layout(P, N).bytes : 0;
 }
 
-VCR_API int vcr_crop_nearest_sort(const double* pc64, int P, int N, int keep, float* out, void* workspace,
-                                  size_t workspace_bytes, cudaStream_t stream) {
+namespace {
+// n == nullptr: the uniform crop; otherwise the ragged one with per-cloud n / keep (device)
+int crop_nearest_sort_launch(const double* pc64, const int* n_len, const int* keep_len, int P, int N, int keep,
+                             float* out, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
     VCR_REQUIRE(pc64 && out && workspace && ((uintptr_t)workspace & 7) == 0);
     if (!crop_sort_shape_ok(P, N) || keep < 1 || keep > N) return VCR_ERR_UNSUPPORTED;
     const CropSortLayout l = crop_sort_layout(P, N);
@@ -413,7 +496,8 @@ VCR_API int vcr_crop_nearest_sort(const double* pc64, int P, int N, int keep, fl
     unsigned* idx[2] = {reinterpret_cast<unsigned*>(ws + l.idx0), reinterpret_cast<unsigned*>(ws + l.idx1)};
     unsigned* counts = reinterpret_cast<unsigned*>(ws + l.counts);
     const size_t n = (size_t)P * N;
-    crop_keys_kernel<<<vcr_cdiv(n, 256), 256, 0, stream>>>(pc64, N, n, keys[0], idx[0]);
+    if (n_len) crop_keys_kernel<true><<<vcr_cdiv(n, 256), 256, 0, stream>>>(pc64, N, n, keys[0], idx[0], n_len);
+    else crop_keys_kernel<false><<<vcr_cdiv(n, 256), 256, 0, stream>>>(pc64, N, n, keys[0], idx[0], nullptr);
     VCR_CHECK_LAUNCH();
     const int tiles_total = P * l.tiles;                  // <= P * N
     for (int pass = 0; pass < 8; ++pass) {                // even, so the sorted pairs end in buffer 0
@@ -427,9 +511,27 @@ VCR_API int vcr_crop_nearest_sort(const double* pc64, int P, int N, int keep, fl
         VCR_CHECK_LAUNCH();
     }
     const size_t total = (size_t)P * keep;
-    crop_gather_kernel<<<vcr_cdiv(total, 256), 256, 0, stream>>>(pc64, N, keep, total, idx[0], out);
+    if (n_len)
+        crop_gather_kernel<true><<<vcr_cdiv(total, 256), 256, 0, stream>>>(pc64, N, keep, total, idx[0], out, n_len,
+                                                                            keep_len);
+    else
+        crop_gather_kernel<false><<<vcr_cdiv(total, 256), 256, 0, stream>>>(pc64, N, keep, total, idx[0], out, nullptr,
+                                                                             nullptr);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
+}
+}  // namespace
+
+VCR_API int vcr_crop_nearest_sort(const double* pc64, int P, int N, int keep, float* out, void* workspace,
+                                  size_t workspace_bytes, cudaStream_t stream) {
+    return crop_nearest_sort_launch(pc64, nullptr, nullptr, P, N, keep, out, workspace, workspace_bytes, stream);
+}
+
+VCR_API int vcr_crop_nearest_sort_ragged(const double* pc64, const int* n, const int* keep, int P, int N_max,
+                                         int keep_max, float* out, void* workspace, size_t workspace_bytes,
+                                         cudaStream_t stream) {
+    VCR_REQUIRE(n && keep);
+    return crop_nearest_sort_launch(pc64, n, keep, P, N_max, keep_max, out, workspace, workspace_bytes, stream);
 }
 
 // acc: device double[8], zero-initialised once per evaluation run; src/tgt [B,3,N], srcK/corrK [B,3,M].
@@ -440,7 +542,24 @@ VCR_API int vcr_eval_metrics(const float* src, const float* tgt, int N, const fl
     const long long work = (long long)B * (N > M ? N : M);
     int blocks = vcr_cdiv(work, 256);
     if (blocks > 592) blocks = 592;
-    eval_metrics_kernel<<<blocks, 256, 0, stream>>>(src, tgt, N, srcK, corrK, M, R_gt, t_gt, R_ab, t_ab, R_ba, t_ba, B, acc);
+    eval_metrics_kernel<false><<<blocks, 256, 0, stream>>>(src, tgt, N, srcK, corrK, M, R_gt, t_gt, R_ab, t_ab, R_ba, t_ba,
+                                                           B, acc, nullptr, nullptr);
+    VCR_CHECK_LAUNCH();
+    return VCR_OK;
+}
+
+// src/tgt [B,3,N_max] with n[b] points, srcK/corrK [B,3,M_max] with m[b] columns; one grid row of blocks per pair.
+VCR_API int vcr_eval_metrics_ragged(const float* src, const float* tgt, const int* n, int N_max, const float* srcK,
+                                    const float* corrK, const int* m, int M_max, const float* R_gt, const float* t_gt,
+                                    const float* R_ab, const float* t_ab, const float* R_ba, const float* t_ba, int B,
+                                    double* acc, cudaStream_t stream) {
+    VCR_REQUIRE(src && tgt && n && srcK && corrK && m && R_gt && t_gt && R_ab && t_ab && R_ba && t_ba && acc);
+    if (B < 1 || B > 65535 || N_max < 1 || M_max < 1) return VCR_ERR_UNSUPPORTED;
+    const int per_pair = 592 / B > 1 ? 592 / B : 1;
+    int bx = vcr_cdiv(N_max > M_max ? N_max : M_max, 256);
+    if (bx > per_pair) bx = per_pair;
+    eval_metrics_kernel<true><<<dim3(bx, B), 256, 0, stream>>>(src, tgt, N_max, srcK, corrK, M_max, R_gt, t_gt, R_ab,
+                                                               t_ab, R_ba, t_ba, B, acc, n, m);
     VCR_CHECK_LAUNCH();
     return VCR_OK;
 }

@@ -231,6 +231,72 @@ def crop_nearest_sort(pc64: torch.Tensor, keep: int):
     return out
 
 
+def make_pairs_ragged(base: torch.Tensor, idx_src: torch.Tensor, idx_tgt: torch.Tensor, pose: torch.Tensor,
+                      n: torch.Tensor, fp64: bool = False):
+    """vcr_make_pairs_ragged: base fp32 [P,Nb,3], idx_src / idx_tgt int32 [P,N_max], pose fp64 [P,12], n int32 [P] ->
+    (src, tgt) [P,3,N_max] (fp64 when ``fp64``, the crop's input, else fp32); columns past n[p] are 0."""
+    _chk(base, "base"); _chk(idx_src, "idx_src", torch.int32); _chk(idx_tgt, "idx_tgt", torch.int32)
+    _chk(pose, "pose", torch.float64)
+    P, Nb, _ = base.shape
+    N = idx_src.shape[1]
+    if tuple(idx_tgt.shape) != (P, N) or tuple(idx_src.shape) != (P, N) or tuple(pose.shape) != (P, 12):
+        raise RuntimeError("vcr_net_b200: make_pairs_ragged: idx_src / idx_tgt must be [P, N_max] and pose [P, 12]")
+    n = _lengths(n, P, "n")
+    base, idx_src, idx_tgt, pose = base.contiguous(), idx_src.contiguous(), idx_tgt.contiguous(), pose.contiguous()
+    dt = torch.float64 if fp64 else _F32
+    src = torch.empty((P, 3, N), dtype=dt, device=base.device)
+    tgt = torch.empty((P, 3, N), dtype=dt, device=base.device)
+    p64 = (src.data_ptr(), tgt.data_ptr()) if fp64 else (None, None)
+    p32 = (None, None) if fp64 else (src.data_ptr(), tgt.data_ptr())
+    L = lib()
+    L.check(L.vcr_make_pairs_ragged(base.data_ptr(), P, Nb, idx_src.data_ptr(), idx_tgt.data_ptr(), pose.data_ptr(),
+                                    n.data_ptr(), N, p64[0], p64[1], p32[0], p32[1], _stream(base)),
+            "vcr_make_pairs_ragged")
+    return src, tgt
+
+
+def crop_nearest_ragged(pc64: torch.Tensor, n: torch.Tensor, keep: torch.Tensor, keep_max: int):
+    """crop_nearest of a ragged batch: pc64 fp64 [P,3,N_max], cloud p is its first n[p] points; -> fp32 [P,3,keep_max]
+    holding the keep[p] points nearest to point n[p] - 1, nearest first, then zeros.  Routed as crop_nearest, by N_max;
+    both routes give the same bits (NaN distances aside, which only the sort orders)."""
+    _chk(pc64, "pc64", torch.float64)
+    P, C, N = pc64.shape
+    assert C == 3
+    n, keep = _lengths(n, P, "n"), _lengths(keep, P, "keep")
+    pc64 = pc64.contiguous()
+    out = torch.empty((P, 3, keep_max), dtype=_F32, device=pc64.device)
+    L = lib()
+    if N <= CROP_ONE_CTA_MAX_POINTS:
+        L.check(L.vcr_crop_nearest_ragged(pc64.data_ptr(), n.data_ptr(), keep.data_ptr(), P, N, keep_max,
+                                          out.data_ptr(), _stream(pc64)), "vcr_crop_nearest_ragged")
+        return out
+    if P * N > CROP_MAX_TOTAL_POINTS:
+        raise RuntimeError(f"vcr_crop_nearest_sort_ragged: the crop takes at most {CROP_MAX_TOTAL_POINTS} points per "
+                           f"call (clouds x points), got {P} x {N}")
+    wsb = L.vcr_crop_nearest_workspace_bytes(P, N)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=pc64.device)
+    L.check(L.vcr_crop_nearest_sort_ragged(pc64.data_ptr(), n.data_ptr(), keep.data_ptr(), P, N, keep_max,
+                                           out.data_ptr(), ws.data_ptr(), wsb, _stream(pc64)),
+            "vcr_crop_nearest_sort_ragged")
+    return out
+
+
+def eval_metrics_ragged(acc: torch.Tensor, src, tgt, n, srcK, corrK, m, R_gt, t_gt, R_ab, t_ab, R_ba, t_ba):
+    """vcr_eval_metrics_ragged into the device double[8] ``acc``: src / tgt [B,3,N_max] with n[b] points, srcK / corrK
+    [B,3,M_max] with m[b] columns, poses [B,3,3] / [B,3] fp32."""
+    _chk(acc, "acc", torch.float64)
+    ts = [_chk(x, name).contiguous() for x, name in zip((src, tgt, srcK, corrK, R_gt, t_gt, R_ab, t_ab, R_ba, t_ba),
+                                                       ("src", "tgt", "srcK", "corrK", "R_gt", "t_gt", "R_ab", "t_ab",
+                                                        "R_ba", "t_ba"))]
+    B, N, M = src.shape[0], src.shape[2], srcK.shape[2]
+    n, m = _lengths(n, B, "n"), _lengths(m, B, "m")
+    L = lib()
+    L.check(L.vcr_eval_metrics_ragged(ts[0].data_ptr(), ts[1].data_ptr(), n.data_ptr(), N, ts[2].data_ptr(),
+                                      ts[3].data_ptr(), m.data_ptr(), M, ts[4].data_ptr(), ts[5].data_ptr(),
+                                      ts[6].data_ptr(), ts[7].data_ptr(), ts[8].data_ptr(), ts[9].data_ptr(), B,
+                                      acc.data_ptr(), _stream(src)), "vcr_eval_metrics_ragged")
+
+
 # --------------------------------------------------------------------------------------------------
 # GEMM
 # --------------------------------------------------------------------------------------------------

@@ -106,3 +106,8 @@ class PairSource:
     def batch(self, first, count):
         assert first + count <= self.n_items
         return self.gen.batch(range(first, first + count))
+
+    def batch_ragged(self, first, count, num_points, n_max=None):
+        """batch() as a ragged batch, item first + i at num_points[i] points (PairGenerator.batch_ragged)."""
+        assert first + count <= self.n_items
+        return self.gen.batch_ragged(range(first, first + count), num_points, n_max)
